@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: batched witness generation for circuit9_authV2 (BASELINE.json config 4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -41,6 +41,8 @@ sys.path.insert(0, ROOT)
 CIRCUIT_DEFAULT = "circuit9_authV2"
 M = 21888242871839275222246405745257275088548364400416034343698204186575808495617
 UNIT = "witnesses/s"
+DUMP_BUDGET_BYTES = 60 << 20         # witness.npy of --dump-outputs (float64 limbs); the index array and headers fit beside it
+DUMP_SEED = 20241
 
 
 def shard_range(n_units: int, rank: int, world: int):
@@ -262,7 +264,17 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed, seeded sample of the witnesses the last timed step computed (rank 0's shard) to DIR: "
+                         "witness.npy float64 [R, W, 8] = the 32-bit little-endian limbs of each canonical witness value, "
+                         "input_set.npy float64 [R] = the index of each sampled input set in the batch; at most 64 MB.  "
+                         "The row copies run in the last timed step; their event-measured time is left out of the timing "
+                         "(extra.dump_copy_ms_excluded)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -356,9 +368,31 @@ def main():
     d_out = torch.empty((chunk, W * 32), dtype=torch.uint8, device=dev)
     stream = torch.cuda.current_stream()
 
-    def step():
-        for lo, hi in launches:
+    # --dump-outputs: the sampled rows are chosen by their index in the shard, not by launch, so that two builds whose
+    # launch plans differ still dump the same input sets.  d_out only holds the current launch, so in the last timed step
+    # the sampled rows are copied into d_dump after each launch, on the same stream (one cudaMemcpyAsync per row, no
+    # kernel).  CUDA events bracket each group of copies, and their time is taken out of the timed total.
+    d_dump, dump_rows, dump_at, dump_events = None, None, [[] for _ in launches], []
+    if a.dump_outputs and rank == 0:
+        n_dump = min(B, DUMP_BUDGET_BYTES // (W * 8 * 8))
+        if n_dump < 1:
+            raise SystemExit(f"--dump-outputs: one witness of {W} values exceeds {DUMP_BUDGET_BYTES} bytes as float64 limbs")
+        dump_rows = np.sort(np.random.default_rng(DUMP_SEED).choice(B, n_dump, replace=False))
+        d_dump = torch.empty((n_dump, W * 32), dtype=torch.uint8, device=dev)
+        for k, r in enumerate(dump_rows):
+            i = next(i for i, (lo, hi) in enumerate(launches) if lo <= r < hi)
+            dump_at[i].append((k, int(r) - launches[i][0]))
+
+    def step(dump=False):
+        for (lo, hi), dumps in zip(launches, dump_at):
             g.calc_witness_batch_device(local_rank, d_in[lo:hi].data_ptr(), hi - lo, d_out.data_ptr(), None, stream.cuda_stream)
+            if dump and dumps:
+                c0, c1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                c0.record(stream)
+                for k, r in dumps:
+                    d_dump[k].copy_(d_out[r])
+                c1.record(stream)
+                dump_events.append((c0, c1))
 
     for _ in range(a.warmup):
         step()
@@ -366,11 +400,12 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
-    for _ in range(a.steps):
-        step()
+    for s in range(a.steps):
+        step(dump=d_dump is not None and s == a.steps - 1)
     e1.record(stream)
     barrier()
-    ms_total = e0.elapsed_time(e1)
+    dump_copy_ms = sum(c0.elapsed_time(c1) for c0, c1 in dump_events)
+    ms_total = e0.elapsed_time(e1) - dump_copy_ms
     clocks = sampler.stop() if sampler else None
     ms_step = max_over_ranks(ms_total) / a.steps
     value = B_total / (ms_step * 1e-3)
@@ -386,6 +421,12 @@ def main():
         rows = sorted({int(x) for x in np.linspace(0, hi - lo - 1, 64)})
         got = d_out[rows].cpu().numpy().reshape(len(rows), W, 32)
         verified = bool((cg.evaluate_batch(host_in[[lo + r for r in rows]], min(len(rows), os.cpu_count() or 1)) == got).all())
+    if d_dump is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        limbs = d_dump.cpu().numpy().reshape(len(dump_rows), W, 32).view("<u4")
+        np.save(os.path.join(a.dump_outputs, "witness.npy"), limbs.astype(np.float64))
+        np.save(os.path.join(a.dump_outputs, "input_set.npy"), (lo_set + dump_rows).astype(np.float64))
+        del d_dump
     del d_out
     torch.cuda.empty_cache()
 
@@ -532,6 +573,8 @@ def main():
         "roofline": roofline, "roofline_hbm": roofline_hbm, "cpu_baseline": cpu, "e2e": e2e,
         "gpu_launches": n_launches, "clocks": clocks, "configs": configs,
     }
+    if a.dump_outputs:
+        line["extra"]["dump_copy_ms_excluded"] = dump_copy_ms
     if world > 1:
         dist.destroy_process_group()
     emit(line)

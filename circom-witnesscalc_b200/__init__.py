@@ -18,7 +18,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GW_LIB_PATH") or os.path.join(_HERE, "lib", "libcircom_witnesscalc.so")   # GW_LIB_PATH: kernel-variant experiments (tools/)
 CLI_PATH = os.path.join(_HERE, "bin", "calc-witness")
 CLI_BATCH_PATH = os.path.join(_HERE, "bin", "calc-witness-batch")
-REF_EXAMPLE_PATH = os.path.join(_HERE, "bin", "ref-example-calc-witness")   # reference examples/calc_witness.c, built unchanged
+EXAMPLE_PATH = os.path.join(_HERE, "bin", "example-calc-witness")   # examples/calc_witness.c, the plain-C embedding example
 
 if not os.path.exists(LIB_PATH):
     raise ImportError(

@@ -2,10 +2,11 @@
 
   python circom-witnesscalc_b200/build.py [--force] [--verbose]
 
-Outputs (git-ignored, shipped to the GPU box by gpurun):
+Outputs (git-ignored):
   circom-witnesscalc_b200/lib/libcircom_witnesscalc.so   the C-ABI library of include/graph_witness.h
   circom-witnesscalc_b200/bin/calc-witness               CLI with the reference's argv contract
   circom-witnesscalc_b200/bin/calc-witness-batch         batch companion: <graph.bin> <inputs.jsonl> <out_dir> [n_gpus]
+  circom-witnesscalc_b200/bin/example-calc-witness       examples/calc_witness.c: <inputs.json> <graph.bin> <out.wtns>
 """
 import os
 import subprocess
@@ -19,11 +20,9 @@ LIB = os.path.join(HERE, "lib", "libcircom_witnesscalc.so")
 LIB_PROF = os.path.join(HERE, "lib_variants", "libcwc_prof.so")
 BIN = os.path.join(HERE, "bin", "calc-witness")
 BIN_BATCH = os.path.join(HERE, "bin", "calc-witness-batch")
-# the reference's own C embedding example (examples/calc_witness.c), compiled UNCHANGED from where it lies against this
-# library's header: the acceptance test of the drop-in C ABI.  Only built where /root/reference exists (here, not on the
-# GPU box, which uses the prebuilt binary); no reference source is copied into the repo.
-REF_EXAMPLE_SRC = "/root/reference/examples/calc_witness.c"
-BIN_REF_EXAMPLE = os.path.join(HERE, "bin", "ref-example-calc-witness")
+# the plain-C embedding example of the drop-in ABI (examples/calc_witness.c): the acceptance test of the C ABI runs it
+EXAMPLE_SRC = os.path.join(HERE, "..", "examples", "calc_witness.c")
+BIN_EXAMPLE = os.path.join(HERE, "bin", "example-calc-witness")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 SOURCES = ["engine.cu", "graph.cpp", "plan.cpp", "bitplan.cpp", "inputs.cpp", "wtns.cpp", "capi.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
@@ -60,15 +59,9 @@ def build(force=False, verbose=False):
                "-L" + os.path.dirname(LIB), "-lcircom_witnesscalc", "-Wl,-rpath,$ORIGIN/../lib"]
         subprocess.check_call(cmd)
     header = os.path.join(HERE, "..", "include", "graph_witness.h")
-    if os.path.exists(REF_EXAMPLE_SRC) and (force or _newer(BIN_REF_EXAMPLE, [LIB, REF_EXAMPLE_SRC, header])):
-        import tempfile
-        with tempfile.TemporaryDirectory() as tmp:
-            # the example includes "../include/graph_witness.h": give it OUR header at that relative path
-            os.makedirs(os.path.join(tmp, "examples")); os.makedirs(os.path.join(tmp, "include"))
-            os.symlink(REF_EXAMPLE_SRC, os.path.join(tmp, "examples", "calc_witness.c"))
-            os.symlink(os.path.abspath(header), os.path.join(tmp, "include", "graph_witness.h"))
-            subprocess.check_call(["gcc", "-w", "-o", BIN_REF_EXAMPLE, os.path.join(tmp, "examples", "calc_witness.c"),
-                                   "-L" + os.path.dirname(LIB), "-lcircom_witnesscalc", "-Wl,-rpath,$ORIGIN/../lib"])
+    if force or _newer(BIN_EXAMPLE, [LIB, EXAMPLE_SRC, header]):
+        subprocess.check_call(["gcc", "-std=c99", "-O2", "-Wall", "-Wextra", "-o", BIN_EXAMPLE, EXAMPLE_SRC,
+                               "-L" + os.path.dirname(LIB), "-lcircom_witnesscalc", "-Wl,-rpath,$ORIGIN/../lib"])
     return LIB
 
 

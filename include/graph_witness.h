@@ -2,7 +2,7 @@
  *
  * Part 1 is the reference's header verbatim in meaning: /root/reference/include/graph_witness.h:7-28
  * (GW_ERROR_CODE, gw_status_t, gw_calc_witness, gw_free_status), implemented by the reference in
- * src/lib.rs:28-111.  examples/calc_witness.c of the reference compiles against this file unchanged.
+ * src/lib.rs:28-111.  tests/csrc/reference_abi_part1.c checks it against the reference's declarations.
  * Part 2 is the batch extension (SURVEY.md section 8b): load a graph once, evaluate many input sets.
  *
  * Every entry point is backed by CUDA kernels; there is no CPU fallback: without a usable GPU the

@@ -1,6 +1,7 @@
 """The C-ABI shared library: loads without a GPU, exports every symbol include/graph_witness.h
-declares, graph-level entry points that need no device work behave, and the reference's own C
-example compiles and links against it unchanged.  No compute calls here (no GPU in this suite)."""
+declares, graph-level entry points that need no device work behave, part 1 of the header matches the
+reference's declarations, and the plain-C example compiles and links against it.  No compute calls here
+(no GPU in this suite)."""
 import ctypes
 import importlib
 import os
@@ -76,18 +77,40 @@ def test_product_does_not_link_or_import_the_oracle(cwc):
                 assert "oracle/" not in txt and "import oracle" not in txt and "from oracle" not in txt, f
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/examples/calc_witness.c"), reason="reference tree not present")
-def test_reference_c_example_links_unchanged(cwc, tmp_path):
-    """examples/calc_witness.c includes "../include/graph_witness.h": give it our header at that relative path"""
-    ex = tmp_path / "examples"
-    inc = tmp_path / "include"
-    ex.mkdir(); inc.mkdir()
-    os.symlink("/root/reference/examples/calc_witness.c", ex / "calc_witness.c")
-    os.symlink(HEADER, inc / "graph_witness.h")
+def test_header_part1_is_the_reference_abi(tmp_path):
+    """tests/csrc/reference_abi_part1.c restates the reference header's drop-in declarations (SURVEY.md 8(b)) and compiles
+    only if include/graph_witness.h matches them; a header with a changed constant or parameter type must not compile"""
+    src = os.path.join(util.ROOT, "tests", "csrc", "reference_abi_part1.c")
+
+    def compiles(root):
+        r = subprocess.run(["gcc", "-std=c11", "-Wall", "-Wextra", "-Werror", "-fsyntax-only",
+                            os.path.join(root, "tests", "csrc", "reference_abi_part1.c")], capture_output=True, text=True)
+        return r.returncode == 0, r.stderr
+    ok, err = compiles(util.ROOT)
+    assert ok, err
+    hdr = open(HEADER).read()
+    for k, (old, new) in enumerate((("ERROR = 1", "ERROR = 2"), ("char *error_msg;", "const char *error_msg;"),
+                                    ("size_t *wtns_len,\n                const", "uint32_t *wtns_len,\n                const"),
+                                    ("const gw_status_t *status);", "gw_status_t *status);"))):
+        assert hdr.count(old) == 1, old
+        root = tmp_path / str(k)
+        (root / "include").mkdir(parents=True)
+        (root / "tests" / "csrc").mkdir(parents=True)
+        (root / "include" / "graph_witness.h").write_text(hdr.replace(old, new))
+        (root / "tests" / "csrc" / "reference_abi_part1.c").write_text(open(src).read())
+        assert not compiles(str(root))[0], new
+
+
+def test_c_example_compiles_as_c99_and_links(cwc, tmp_path):
+    """examples/calc_witness.c (plain C, includes "../include/graph_witness.h" like the reference's example) compiles
+    without a warning as C99 and links against the library; wrong argc -> usage on stderr, exit 1"""
     exe = tmp_path / "calc_witness_example"
-    subprocess.check_call(["gcc", "-o", str(exe), str(ex / "calc_witness.c"), "-L" + os.path.dirname(cwc.LIB_PATH),
+    subprocess.check_call(["gcc", "-std=c99", "-Wall", "-Wextra", "-Werror", "-o", str(exe),
+                           os.path.join(util.ROOT, "examples", "calc_witness.c"), "-L" + os.path.dirname(cwc.LIB_PATH),
                            "-lcircom_witnesscalc", "-Wl,-rpath," + os.path.dirname(cwc.LIB_PATH)])
-    assert exe.exists()
+    r = subprocess.run([str(exe)], capture_output=True, text=True)
+    assert r.returncode == 1 and "<inputs.json> <graph.bin> <witness.wtns>" in r.stderr
+    assert os.path.exists(cwc.EXAMPLE_PATH)
     # CLI contract of the reference binary (calc-witness.rs:13-19): wrong argc -> usage on stderr, exit 1
     r = subprocess.run([cwc.CLI_PATH], capture_output=True, text=True)
     assert r.returncode == 1 and "Usage:" in r.stderr and "<graph.bin> <inputs.json> <witness.wtns>" in r.stderr

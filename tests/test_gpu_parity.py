@@ -35,8 +35,8 @@ def test_golden_wtns_drop_in(cwc, name):
 @pytest.mark.parametrize("name", ["circuit5_poseidon", "circuit2", "circuit6_num2bits", "circuit9_authV2"])
 def test_drop_in_binaries_run_and_cmp(cwc, name, tmp_path):
     """The equivalent of test_circuits.sh:64,81: RUN `calc-witness <graph.bin> <inputs.json> <out.wtns>` and the
-    reference's own embedding example (examples/calc_witness.c, compiled unchanged against this library; argv order
-    <inputs> <graph> <witness>) and `cmp` what they write with the golden .wtns."""
+    plain-C embedding example (examples/calc_witness.c, argv order <inputs> <graph> <witness> as in the reference's
+    example) and `cmp` what they write with the golden .wtns."""
     import os
     import subprocess
     gp, ip = tmp_path / "graph.bin", tmp_path / "inputs.json"
@@ -48,9 +48,9 @@ def test_drop_in_binaries_run_and_cmp(cwc, name, tmp_path):
     assert r.returncode == 0, r.stderr
     assert "Witness generated in:" in r.stdout and f"witness saved to {out1}" in r.stdout      # calc-witness.rs:41,48
     assert out1.read_bytes() == want
-    assert os.path.exists(cwc.REF_EXAMPLE_PATH), "bin/ref-example-calc-witness missing: run build() where /root/reference exists"
+    assert os.path.exists(cwc.EXAMPLE_PATH), "bin/example-calc-witness missing: run circom-witnesscalc_b200/build.py"
     out2 = tmp_path / "example.wtns"
-    r = subprocess.run([cwc.REF_EXAMPLE_PATH, str(ip), str(gp), str(out2)], capture_output=True, text=True, timeout=300)
+    r = subprocess.run([cwc.EXAMPLE_PATH, str(ip), str(gp), str(out2)], capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, r.stderr + r.stdout
     assert out2.read_bytes() == want
     # error path of the CLI: a corrupt graph is an error message and a non-zero exit, not a crash
