@@ -46,6 +46,15 @@ class gw_graph_info_t(ctypes.Structure):
                 ("bit_wide", ctypes.c_uint32)]
 
 
+class gw_r1cs_info_t(ctypes.Structure):
+    _fields_ = [("n_wires", ctypes.c_uint32), ("n_pub_out", ctypes.c_uint32), ("n_pub_in", ctypes.c_uint32),
+                ("n_prv_in", ctypes.c_uint32), ("n_constraints", ctypes.c_uint32), ("n_consts", ctypes.c_uint32),
+                ("n_labels", ctypes.c_uint64), ("n_terms", ctypes.c_uint64), ("n_mac_terms", ctypes.c_uint64),
+                ("n_chunks", ctypes.c_uint64)]
+
+
+R1CS_OK = 0xFFFFFFFF    # GW_R1CS_OK: every constraint holds
+
 _libc = ctypes.CDLL(None)
 _libc.free.argtypes = [ctypes.c_void_p]
 
@@ -68,6 +77,12 @@ _L.gw_calc_witness_batch_wtns.argtypes = [_vp, _vp, _sz, _vp, _sz, _vp, ctypes.c
 _L.gw_graph_select.argtypes = [_vp, _vp, _sz, ctypes.POINTER(_vp), ctypes.POINTER(gw_status_t)]
 CHUNK_FN = ctypes.CFUNCTYPE(ctypes.c_int, _vp, ctypes.c_int, _sz, _sz, _vp, _sz, _vp)
 _L.gw_calc_witness_batch_stream.argtypes = [_vp, ctypes.c_int, ctypes.c_int, _vp, _sz, _sz, CHUNK_FN, _vp, ctypes.POINTER(gw_status_t)]
+_L.gw_r1cs_load.argtypes = [_vp, _sz, ctypes.POINTER(_vp), ctypes.POINTER(gw_status_t)]
+_L.gw_r1cs_free.argtypes = [_vp]
+_L.gw_r1cs_info.argtypes = [_vp, ctypes.POINTER(gw_r1cs_info_t)]
+_L.gw_r1cs_check_batch.argtypes = [_vp, _vp, _sz, _sz, _vp, ctypes.c_int, ctypes.POINTER(gw_status_t)]
+_L.gw_r1cs_check_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _sz, _vp, _vp, ctypes.POINTER(gw_status_t)]
+_L.gw_calc_witness_batch_check.argtypes = [_vp, _vp, ctypes.c_int, ctypes.c_int, _vp, _sz, _vp, _vp, _vp, ctypes.POINTER(gw_status_t)]
 _L.gw_set_device.argtypes = [ctypes.c_int]
 _L.gw_device_count.restype = ctypes.c_int
 _L.gw_microbench_imad.restype = ctypes.c_double
@@ -76,7 +91,8 @@ _L.gw_microbench_imad.argtypes = [ctypes.c_int, ctypes.c_int]
 EXPORTS = ["gw_calc_witness", "gw_graph_load", "gw_graph_free", "gw_graph_info", "gw_graph_input_signal",
            "gw_graph_calc_witness", "gw_calc_witness_batch", "gw_calc_witness_batch_on", "gw_calc_witness_batch_device", "gw_calc_witness_latency", "gw_wtns_header",
            "gw_device_count", "gw_microbench_imad", "gw_inputs_parse_batch", "gw_wtns_file_size", "gw_calc_witness_batch_wtns",
-           "gw_graph_select", "gw_calc_witness_batch_stream", "gw_set_device"]
+           "gw_graph_select", "gw_calc_witness_batch_stream", "gw_set_device", "gw_r1cs_load", "gw_r1cs_free", "gw_r1cs_info",
+           "gw_r1cs_check_batch", "gw_r1cs_check_batch_device", "gw_calc_witness_batch_check"]
 
 
 class WitnessCalcError(RuntimeError):
@@ -279,9 +295,75 @@ class Graph:
         rc = _L.gw_calc_witness_batch_stream(self._h, first_device, n_gpus, inputs_ptr, n_sets, chunk_sets, cb, None, ctypes.byref(st))
         _check(rc, st)
 
+    def calc_witness_batch_check(self, r1cs: "R1cs", inputs: np.ndarray, n_gpus=1, want_witness=True, first_device=0):
+        """HOST buffers: evaluate and check against `r1cs` on the device in one pass (gw_calc_witness_batch_check).
+        Returns (witness uint8 [B, W, 32] or None, flags uint32 [B], first_failed uint32 [B]); first_failed[b] is the
+        lowest violated constraint of set b or R1CS_OK.  want_witness=False keeps the witnesses on the device."""
+        inputs = np.ascontiguousarray(inputs, dtype=np.uint8)
+        B = inputs.shape[0]
+        assert inputs.shape[1:] == (self.n_inputs, 32), inputs.shape
+        out = np.empty((B, self.n_witness, 32), dtype=np.uint8) if want_witness else None
+        flags = np.zeros(B, dtype=np.uint32)
+        first = np.zeros(B, dtype=np.uint32)
+        st = gw_status_t()
+        rc = _L.gw_calc_witness_batch_check(self._h, r1cs._h, first_device, n_gpus, inputs.ctypes.data, B,
+                                            out.ctypes.data if want_witness else None, flags.ctypes.data, first.ctypes.data,
+                                            ctypes.byref(st))
+        _check(rc, st)
+        return out, flags, first
+
     def calc_witness_batch_device(self, device, d_inputs_ptr, n_sets, d_witness_ptr, d_flags_ptr=None, stream=None):
         """DEVICE pointers; asynchronous on `stream` (a cudaStream_t as int, None = default stream)."""
         st = gw_status_t()
         rc = _L.gw_calc_witness_batch_device(self._h, device, d_inputs_ptr, n_sets, d_witness_ptr, d_flags_ptr,
                                              stream, ctypes.byref(st))
+        _check(rc, st)
+
+
+class R1cs:
+    """A circuit's .r1cs file parsed and compiled once: gw_r1cs_load.  Checks witness rows against its constraints."""
+
+    def __init__(self, data: bytes):
+        self._h = _vp()
+        st = gw_status_t()
+        rc = _L.gw_r1cs_load(data, len(data), ctypes.byref(self._h), ctypes.byref(st))
+        _check(rc, st)
+
+    def info(self) -> dict:
+        info = gw_r1cs_info_t()
+        _L.gw_r1cs_info(self._h, ctypes.byref(info))
+        return {k: int(getattr(info, k)) for k, _ in gw_r1cs_info_t._fields_}
+
+    def close(self):
+        if self._h:
+            _L.gw_r1cs_free(self._h)
+            self._h = _vp()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def check_batch(self, rows, row_pitch=0, n_gpus=1, n_sets=None) -> np.ndarray:
+        """HOST rows: a uint8 array whose row r starts at byte r * row_pitch (row_pitch 0: dense rows of n_wires x 32 B,
+        e.g. a [B, W, 32] witness array) -> uint32 [B]: lowest violated constraint per row, or R1CS_OK
+        (gw_r1cs_check_batch).  n_sets defaults to what the array holds."""
+        rows = np.ascontiguousarray(rows, dtype=np.uint8)
+        pitch = row_pitch or self.info()["n_wires"] * 32
+        if n_sets is None:
+            n_sets = rows.shape[0] if rows.ndim > 1 and not row_pitch else (rows.size // pitch if pitch else 0)
+        assert n_sets == 0 or (n_sets - 1) * pitch + self.info()["n_wires"] * 32 <= rows.size, "rows too short"
+        first = np.zeros(n_sets, dtype=np.uint32)
+        st = gw_status_t()
+        rc = _L.gw_r1cs_check_batch(self._h, rows.ctypes.data, n_sets, pitch, first.ctypes.data, n_gpus, ctypes.byref(st))
+        _check(rc, st)
+        return first
+
+    def check_batch_device(self, device, d_witness_ptr, n_sets, d_first_failed_ptr, row_pitch=0, stream=None):
+        """DEVICE pointers; asynchronous on `stream` (a cudaStream_t as int, None = default stream)
+        (gw_r1cs_check_batch_device)."""
+        st = gw_status_t()
+        rc = _L.gw_r1cs_check_batch_device(self._h, device, d_witness_ptr, n_sets, row_pitch, d_first_failed_ptr, stream,
+                                           ctypes.byref(st))
         _check(rc, st)

@@ -7,6 +7,7 @@ Outputs (git-ignored):
   circom-witnesscalc_b200/bin/calc-witness               CLI with the reference's argv contract
   circom-witnesscalc_b200/bin/calc-witness-batch         batch companion: <graph.bin> <inputs.jsonl> <out_dir> [n_gpus]
   circom-witnesscalc_b200/bin/example-calc-witness       examples/calc_witness.c: <inputs.json> <graph.bin> <out.wtns>
+  circom-witnesscalc_b200/bin/wtns-check                 <circuit.r1cs> <witness.wtns> [more.wtns ...] (snarkjs wtns check)
 """
 import os
 import subprocess
@@ -20,11 +21,12 @@ LIB = os.path.join(HERE, "lib", "libcircom_witnesscalc.so")
 LIB_PROF = os.path.join(HERE, "lib_variants", "libcwc_prof.so")
 BIN = os.path.join(HERE, "bin", "calc-witness")
 BIN_BATCH = os.path.join(HERE, "bin", "calc-witness-batch")
+BIN_WTNS_CHECK = os.path.join(HERE, "bin", "wtns-check")
 # the plain-C embedding example of the drop-in ABI (examples/calc_witness.c): the acceptance test of the C ABI runs it
 EXAMPLE_SRC = os.path.join(HERE, "..", "examples", "calc_witness.c")
 BIN_EXAMPLE = os.path.join(HERE, "bin", "example-calc-witness")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-SOURCES = ["engine.cu", "graph.cpp", "plan.cpp", "bitplan.cpp", "inputs.cpp", "wtns.cpp", "capi.cpp"]
+SOURCES = ["engine.cu", "r1cs.cu", "graph.cpp", "plan.cpp", "bitplan.cpp", "inputs.cpp", "wtns.cpp", "r1cs.cpp", "capi.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
 
@@ -56,6 +58,10 @@ def build(force=False, verbose=False):
         subprocess.check_call(cmd)
     if force or _newer(BIN_BATCH, [LIB, os.path.join(CSRC, "calc_witness_batch_main.cpp")]):
         cmd = ["g++", "-O2", "-std=c++17", "-o", BIN_BATCH, os.path.join(CSRC, "calc_witness_batch_main.cpp"),
+               "-L" + os.path.dirname(LIB), "-lcircom_witnesscalc", "-Wl,-rpath,$ORIGIN/../lib"]
+        subprocess.check_call(cmd)
+    if force or _newer(BIN_WTNS_CHECK, [LIB, os.path.join(CSRC, "wtns_check_main.cpp")]):
+        cmd = ["g++", "-O2", "-std=c++17", "-o", BIN_WTNS_CHECK, os.path.join(CSRC, "wtns_check_main.cpp"),
                "-L" + os.path.dirname(LIB), "-lcircom_witnesscalc", "-Wl,-rpath,$ORIGIN/../lib"]
         subprocess.check_call(cmd)
     header = os.path.join(HERE, "..", "include", "graph_witness.h")

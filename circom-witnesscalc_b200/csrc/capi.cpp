@@ -21,6 +21,10 @@ struct gw_graph {
   std::vector<std::string> input_names;
 };
 
+struct gw_r1cs {
+  std::unique_ptr<R1cs> r1cs;
+};
+
 static void set_status(const gw_status_t* status_c, GW_ERROR_CODE code, const char* msg) {   // lib.rs:28-38
   gw_status_t* status = const_cast<gw_status_t*>(status_c);
   if (!status) return;
@@ -250,6 +254,63 @@ int gw_calc_witness_batch_stream(gw_graph_t* graph, int first_device, int n_gpus
                               [&](int device, size_t first, size_t n, const uint8_t* rows, size_t row_bytes, const uint32_t* flags) {
                                 return fn(user, device, first, n, rows, row_bytes, flags);
                               });
+  });
+}
+
+int gw_r1cs_load(const void* data, size_t len, gw_r1cs_t** r1cs, gw_status_t* status) {
+  if (!data || !r1cs) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    std::unique_ptr<gw_r1cs> r(new gw_r1cs());
+    r->r1cs.reset(new R1cs((const uint8_t*)data, len));
+    *r1cs = r.release();
+  });
+}
+
+void gw_r1cs_free(gw_r1cs_t* r1cs) { delete r1cs; }
+
+int gw_r1cs_info(const gw_r1cs_t* r1cs, gw_r1cs_info_t* info) {
+  if (!r1cs || !info) return 1;
+  const R1cs& r = *r1cs->r1cs;
+  memset(info, 0, sizeof *info);
+  info->n_wires = r.hdr.n_wires; info->n_pub_out = r.hdr.n_pub_out; info->n_pub_in = r.hdr.n_pub_in; info->n_prv_in = r.hdr.n_prv_in;
+  info->n_constraints = r.hdr.n_constraints; info->n_consts = (uint32_t)r.prog.consts.size(); info->n_labels = r.hdr.n_labels;
+  info->n_terms = r.prog.n_terms; info->n_mac_terms = r.prog.n_mac_terms; info->n_chunks = r.prog.n_chunks;
+  return 0;
+}
+
+int gw_r1cs_check_batch(gw_r1cs_t* r1cs, const uint8_t* witness, size_t n_sets, size_t row_pitch, uint32_t* first_failed,
+                        int n_gpus, gw_status_t* status) {
+  if (!r1cs || (n_sets && (!witness || !first_failed))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    int ndev = cuda_device_count();
+    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
+    if (n_gpus < 1) n_gpus = 1;
+    if (n_gpus > ndev) throw Error("n_gpus exceeds the number of visible CUDA devices");
+    r1cs->r1cs->check_host(witness, n_sets, row_pitch ? row_pitch : (size_t)r1cs->r1cs->hdr.n_wires * 32, first_failed, n_gpus, 0);
+  });
+}
+
+int gw_r1cs_check_batch_device(gw_r1cs_t* r1cs, int device, const void* d_witness, size_t n_sets, size_t row_pitch,
+                               uint32_t* d_first_failed, void* cuda_stream, gw_status_t* status) {
+  if (!r1cs || (n_sets && (!d_witness || !d_first_failed))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    r1cs->r1cs->check_device(device, d_witness, n_sets, row_pitch ? row_pitch : (size_t)r1cs->r1cs->hdr.n_wires * 32, d_first_failed,
+                             cuda_stream);
+  });
+}
+
+int gw_calc_witness_batch_check(gw_graph_t* graph, gw_r1cs_t* r1cs, int first_device, int n_gpus, const uint8_t* inputs,
+                                size_t n_sets, uint8_t* witness, uint32_t* flags, uint32_t* first_failed, gw_status_t* status) {
+  if (!graph || !r1cs || (n_sets && (!inputs || !first_failed))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    const uint32_t W = graph->engine->plan.n_witness, n_wires = r1cs->r1cs->hdr.n_wires;
+    if (W != n_wires)
+      throw Error("the graph's witness has " + std::to_string(W) + " values but the R1CS has " + std::to_string(n_wires) + " wires");
+    int ndev = cuda_device_count();
+    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
+    if (n_gpus < 1) n_gpus = 1;
+    if (first_device < 0 || first_device + n_gpus > ndev) throw Error("device range exceeds the visible CUDA devices");
+    graph->engine->run_host(inputs, n_sets, witness, flags, n_gpus, first_device, 0, r1cs->r1cs.get(), first_failed);
   });
 }
 

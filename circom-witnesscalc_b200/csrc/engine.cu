@@ -24,6 +24,7 @@
 
 #include "engine.hpp"
 #include "alu.cuh"
+#include "cuda_util.hpp"
 
 namespace gw {
 
@@ -936,21 +937,6 @@ __global__ void imad_bench_kernel(uint32_t* out, int iters, uint32_t y) {
   if (acc == 0x12345678u) out[0] = acc;
 }
 
-// The library works on the device it is told to, and leaves the calling thread's current device as it found it
-// (a caller that mixes this library with its own CUDA code must not find itself on another GPU after a call).
-struct DeviceGuard {
-  int prev = -1;
-  explicit DeviceGuard(int device) {
-    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-    cudaError_t e = cudaSetDevice(device);
-    if (e != cudaSuccess) throw Error(std::string("CUDA error: ") + cudaGetErrorString(e) + " at cudaSetDevice");
-  }
-  ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
-  DeviceGuard(const DeviceGuard&) = delete;
-};
-
-#define CUDA_CHECK(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) throw Error(std::string("CUDA error: ") + cudaGetErrorString(e_) + " at " #x); } while (0)
-
 double imad_microbench(int device, int which) {
   DeviceGuard on(device);
   cudaDeviceProp prop; CUDA_CHECK(cudaGetDeviceProperties(&prop, device));
@@ -993,6 +979,7 @@ struct Engine::Dev {
   cudaStream_t stream[2] = {nullptr, nullptr};
   uint4* d_in[2] = {nullptr, nullptr}; uint4* d_out[2] = {nullptr, nullptr};
   uint32_t* d_status[2] = {nullptr, nullptr};
+  uint32_t* d_ff[2] = {nullptr, nullptr};     // lowest violated constraint per set (gw_calc_witness_batch_check only)
   size_t chunk = 0;
   // pinned host ring of the streaming API (three chunks: one in the consumer's hands, one landing, one enqueued)
   uint8_t* h_ring[3] = {nullptr, nullptr, nullptr}; uint32_t* h_flags[3] = {nullptr, nullptr, nullptr};
@@ -1017,7 +1004,7 @@ static int env_int(const char* name, int dflt) { const char* s = getenv(name); r
 // Pins the CALLING thread to the CPUs of the NUMA node the GPU hangs off (sysfs: numa_node of its PCI function,
 // cpulist of that node), so that the thread's pinned allocations are node-local and its copies do not cross the
 // socket interconnect.  Only ever called on threads this library created.  GW_NUMA=0 turns it off.
-static void bind_thread_near_device(int device) {
+void bind_thread_near_device(int device) {
   if (env_int("GW_NUMA", 1) == 0) return;
   char bus[32] = {0};
   if (cudaDeviceGetPCIBusId(bus, (int)sizeof bus, device) != cudaSuccess) return;
@@ -1101,7 +1088,7 @@ Engine::~Engine() {
     cudaFreeHost(d->bit_nbad_host); if (d->bit_nbad_ev) cudaEventDestroy(d->bit_nbad_ev);
     cudaFree(d->lat_soff); cudaFree(d->lat_schunks);
     cudaFree(d->lat_code); cudaFree(d->lat_first); cudaFree(d->lat_jobs); cudaFree(d->lat_njobs); cudaFree(d->lat_waits); cudaFree(d->lat_clock); cudaFree(d->lat_in); cudaFree(d->lat_out); cudaFree(d->lat_status);
-    for (int i = 0; i < 2; i++) { cudaFree(d->d_in[i]); cudaFree(d->d_out[i]); cudaFree(d->d_status[i]); if (d->stream[i]) cudaStreamDestroy(d->stream[i]); }
+    for (int i = 0; i < 2; i++) { cudaFree(d->d_in[i]); cudaFree(d->d_out[i]); cudaFree(d->d_status[i]); cudaFree(d->d_ff[i]); if (d->stream[i]) cudaStreamDestroy(d->stream[i]); }
     for (int i = 0; i < 3; i++) { cudaFreeHost(d->h_ring[i]); cudaFreeHost(d->h_flags[i]); }
     if (d->last_kernel) cudaEventDestroy(d->last_kernel);
     delete d;
@@ -1309,6 +1296,7 @@ void Engine::ensure_staging(Dev* d, size_t chunk) {
     cudaFree(d->d_in[i]); d->d_in[i] = nullptr;
     cudaFree(d->d_out[i]); d->d_out[i] = nullptr;
     cudaFree(d->d_status[i]); d->d_status[i] = nullptr;
+    cudaFree(d->d_ff[i]); d->d_ff[i] = nullptr;
   }
   for (int i = 0; i < 2; i++) {
     CUDA_CHECK(cudaMalloc(&d->d_in[i], std::max<size_t>(chunk * in_b, 32)));
@@ -1341,7 +1329,8 @@ struct StreamDrain {
 }  // namespace
 
 // host buffers: chunked, double-buffered H2D -> kernel -> D2H on two streams
-void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, size_t out_pitch) {
+void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, size_t out_pitch,
+                         R1cs* check, uint32_t* first_failed) {
   Dev* d = dev(device);
   DeviceGuard on(device);
   std::lock_guard<std::mutex> lk(d->mu);
@@ -1359,6 +1348,8 @@ void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* w
   if (B >= 4 * 2048) chunk = std::min(chunk, (B + 3) / 4);
   chunk = std::max<size_t>(std::min(chunk, B), 1);
   ensure_staging(d, chunk);
+  if (check)                                   // verdict buffers of the staging chunk size, allocated on the first check
+    for (int i = 0; i < 2; i++) if (!d->d_ff[i]) CUDA_CHECK(cudaMalloc(&d->d_ff[i], d->chunk * 4));
   // The kernels of consecutive chunks run back to back (launch() chains them: one spill area) while the copies
   // of the two streams overlap with them.
   HostTrace tr;
@@ -1371,8 +1362,14 @@ void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* w
     CUDA_CHECK(cudaMemcpyAsync(d->d_in[k], inputs + off * in_b, nb * in_b, cudaMemcpyHostToDevice, s));
     tr.mark(s);
     launch(d, d->d_in[k], nb, d->d_out[k], status ? d->d_status[k] : nullptr, s);
+    if (check) {
+      // the chunk's witness rows are checked where they are; only the verdicts have to cross PCIe
+      check->check_device(device, d->d_out[k], nb, out_b, d->d_ff[k], s);
+      CUDA_CHECK(cudaMemcpyAsync(first_failed + off, d->d_ff[k], nb * 4, cudaMemcpyDeviceToHost, s));
+    }
     tr.mark(s);
-    if (out_pitch == out_b) CUDA_CHECK(cudaMemcpyAsync(witness + off * out_b, d->d_out[k], nb * out_b, cudaMemcpyDeviceToHost, s));
+    if (!witness) {}      // gw_calc_witness_batch_check without witness: the rows stay on the device
+    else if (out_pitch == out_b) CUDA_CHECK(cudaMemcpyAsync(witness + off * out_b, d->d_out[k], nb * out_b, cudaMemcpyDeviceToHost, s));
     else if (out_b) CUDA_CHECK(cudaMemcpy2DAsync(witness + off * out_pitch, out_pitch, d->d_out[k], out_b, out_b, nb, cudaMemcpyDeviceToHost, s));
     if (status) CUDA_CHECK(cudaMemcpyAsync(status + off, d->d_status[k], nb * 4, cudaMemcpyDeviceToHost, s));
     tr.mark(s);
@@ -1382,10 +1379,11 @@ void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* w
   tr.print(device, B, chunk);
 }
 
-void Engine::run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, int n_gpus, int first_device, size_t out_pitch) {
+void Engine::run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, int n_gpus, int first_device, size_t out_pitch,
+                      R1cs* check, uint32_t* first_failed) {
   if (B == 0) return;
   if (out_pitch == 0) out_pitch = (size_t)plan.n_witness * 32;
-  if (n_gpus <= 1) { run_host_on(first_device, inputs, B, witness, status, out_pitch); return; }
+  if (n_gpus <= 1) { run_host_on(first_device, inputs, B, witness, status, out_pitch, check, first_failed); return; }
   // independent input sets: contiguous shards, one host thread per GPU (pinned to the GPU's NUMA node), no collective
   const size_t in_b = (size_t)plan.n_inputs * 32;
   std::vector<std::thread> th;
@@ -1396,7 +1394,8 @@ void Engine::run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_
     th.emplace_back([=, &errs]() {
       try {
         bind_thread_near_device(first_device + g);
-        run_host_on(first_device + g, inputs + lo * in_b, hi - lo, witness + lo * out_pitch, status ? status + lo : nullptr, out_pitch);
+        run_host_on(first_device + g, inputs + lo * in_b, hi - lo, witness ? witness + lo * out_pitch : nullptr, status ? status + lo : nullptr,
+                    out_pitch, check, check ? first_failed + lo : nullptr);
       } catch (const std::exception& e) { errs[g] = e.what(); }
     });
   }

@@ -11,6 +11,7 @@
 #include "bitplan.hpp"
 #include "graph.hpp"
 #include "plan.hpp"
+#include "r1cs.hpp"
 
 namespace gw {
 
@@ -35,7 +36,10 @@ class Engine {
   // witness row r is written at witness + r * out_pitch (out_pitch >= W * 32 bytes; 0 = dense rows): with a pitch of
   // wtns_size(W) rounded up and witness pointing WTNS_HEADER_BYTES into the first row, every row becomes a complete
   // .wtns file image once the caller has written the 76-byte headers (the DMA engine does the framing).
-  void run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, int n_gpus, int first_device, size_t out_pitch = 0);
+  // With `check`, every chunk's rows are also checked against that R1CS on the device (first_failed[r] = lowest violated
+  // constraint of set r, or R1CS_OK), and witness may be null: then no witness row is copied to the host.
+  void run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, int n_gpus, int first_device, size_t out_pitch = 0,
+                R1cs* check = nullptr, uint32_t* first_failed = nullptr);
   // Streaming output path: chunks of witness rows are handed to `fn` from a pinned ring as they land (one worker
   // thread per GPU; fn(device, first_set, n_sets, rows, row_bytes, flags) returns nonzero to stop).  The memory
   // is only valid during the call.  chunk_sets = 0 picks the chunk size.
@@ -57,7 +61,8 @@ class Engine {
   void launch_bit(Dev* d, const void* d_inputs, size_t B, void* d_witness, uint32_t* d_status, void* stream);
   void ensure_staging(Dev* d, size_t chunk);
   void stream_on(int device, const uint8_t* inputs, size_t B, size_t first_set, size_t chunk_req, const ChunkFn& fn);
-  void run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, size_t out_pitch);
+  void run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, size_t out_pitch, R1cs* check,
+                   uint32_t* first_failed);
   void init_plan();
   std::map<int, Dev*> devs;
   std::mutex mu;

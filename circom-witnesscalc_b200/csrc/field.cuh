@@ -20,7 +20,7 @@
 
 #if defined(__CUDACC__)
 #define GW_HD __host__ __device__ __forceinline__
-#define GW_HD_NOINLINE __host__ __device__ __noinline__
+#define GW_HD_NOINLINE inline __host__ __device__ __noinline__   // inline: one definition however many .cu files include this
 #else
 #define GW_HD inline
 #define GW_HD_NOINLINE inline __attribute__((noinline))

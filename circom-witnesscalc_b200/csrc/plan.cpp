@@ -35,13 +35,17 @@ inline bool op_has_b_host(uint32_t op) { return op < 32 || op == OP_TERN || op =
 
 fe to_fe(const U256& v) { fe r; memcpy(r.l, v.l, 32); return r; }
 U256 to_u256(const fe& v) { U256 r; memcpy(r.l, v.l, 32); return r; }
-// c * 2^256 mod M (or (M - c) * 2^256 mod M): the form OP_DOT constants are stored in
+
+}  // namespace
+
 U256 prescale(const U256& c, bool neg) {
   fe r1; for (int i = 0; i < 8; i++) r1.l[i] = R1_L(i);
   fe v = to_fe(c);
   if (neg) v = fe_neg(v);
   return to_u256(fe_mul(v, r1));
 }
+
+namespace {
 
 // ---- Div batching -----------------------------------------------------------------------------------
 // dl(n) = number of Div nodes on the longest operand path ending at n (n itself excluded).  Div nodes with

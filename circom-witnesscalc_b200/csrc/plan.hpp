@@ -56,6 +56,9 @@ struct Plan {
 
 Plan compile_plan(const Graph& g, const PlanOptions& opt);
 
+// c * 2^256 mod M (or (M - c) * 2^256 mod M): the form OP_DOT constants are stored in (c canonical)
+U256 prescale(const U256& c, bool neg);
+
 // Single-witness ("latency") mode.  The macro ops (fused linear combinations included) are scheduled level by
 // level: all instructions of a level are independent.  A level's instructions are spread over `n_warps` MAIN
 // warps of one CTA -- instructions of the same class share a warp (SIMT lanes), different classes go to different

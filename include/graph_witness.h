@@ -169,6 +169,52 @@ typedef int (*gw_witness_chunk_fn)(void *user, int device, size_t first_set, siz
 int gw_calc_witness_batch_stream(gw_graph_t *graph, int first_device, int n_gpus, const uint8_t *inputs, size_t n_sets,
                                  size_t chunk_sets, gw_witness_chunk_fn fn, void *user, gw_status_t *status);
 
+/* ---- R1CS check (the `snarkjs wtns check` step) ----
+ * A graph has no constraints: an input set that violates the circuit (a bad signature, a stale Merkle root) still gets a
+ * witness.  These calls check witnesses against the circuit's iden3 .r1cs file (version 1, as circom writes it) on the
+ * GPU.  Wire i of the R1CS is witness position i, so n_wires == gw_graph_info_t.n_witness for the graph of the same
+ * circuit.  A row passes when <A_k,w> * <B_k,w> == <C_k,w> (mod M) for every constraint k; a witness value >= M fails
+ * the first constraint that reads it.  first_failed[r] receives the lowest violated constraint of row r, or GW_R1CS_OK. */
+typedef struct gw_r1cs gw_r1cs_t;
+
+typedef struct {
+  uint32_t n_wires;       /* wires = witness length */
+  uint32_t n_pub_out;     /* public outputs (wires 1 .. n_pub_out) */
+  uint32_t n_pub_in;      /* public inputs (after the outputs) */
+  uint32_t n_prv_in;      /* private inputs */
+  uint32_t n_constraints;
+  uint32_t n_consts;      /* distinct coefficients other than 1 and M - 1 (the device's constant table) */
+  uint64_t n_labels;
+  uint64_t n_terms;       /* compiled terms (zero coefficients dropped): 32-byte witness reads per row */
+  uint64_t n_mac_terms;   /* terms with a coefficient other than 1 and M - 1: one 256 x 256-bit product each */
+  uint64_t n_chunks;      /* Montgomery reductions: linear combinations are cut into chunks the accumulator can hold */
+} gw_r1cs_info_t;
+
+#define GW_R1CS_OK 0xFFFFFFFFu
+
+/* parses and compiles an .r1cs file (no GPU needed).  Rejected with a message: bad magic, version != 1, missing header
+ * or constraints section, truncated file or section, a section longer than its content, n8 != 32, a prime other than
+ * BN254's, wire ids >= n_wires, custom-gate sections (4, 5).  Coefficients >= M are reduced mod M. */
+int gw_r1cs_load(const void *data, size_t len, gw_r1cs_t **r1cs, gw_status_t *status);
+void gw_r1cs_free(gw_r1cs_t *r1cs);
+int gw_r1cs_info(const gw_r1cs_t *r1cs, gw_r1cs_info_t *info);
+/* HOST rows: row r (n_wires x 32 B, canonical little-endian) at witness + r * row_pitch (row_pitch >= n_wires x 32;
+ * 0 = dense).  With row_pitch = gw_wtns_file_size(graph) and witness = files + 76, the .wtns images of
+ * gw_calc_witness_batch_wtns are checked in place.  The rows are split into n_gpus contiguous shards, one per device. */
+int gw_r1cs_check_batch(gw_r1cs_t *r1cs, const uint8_t *witness, size_t n_sets, size_t row_pitch, uint32_t *first_failed,
+                        int n_gpus, gw_status_t *status);
+/* DEVICE rows on CUDA device `device` (d_witness and row_pitch 16-byte aligned; row_pitch 0 = dense), d_first_failed on
+ * the same device; enqueued on `cuda_stream` (NULL = default stream) and asynchronous with respect to the host: what a
+ * GPU prover pipeline calls after gw_calc_witness_batch_device on the same stream. */
+int gw_r1cs_check_batch_device(gw_r1cs_t *r1cs, int device, const void *d_witness, size_t n_sets, size_t row_pitch,
+                               uint32_t *d_first_failed, void *cuda_stream, gw_status_t *status);
+/* gw_calc_witness_batch_on and the check in one pass: every chunk's witness rows are checked on the device right after
+ * they are computed.  witness may be NULL: then only flags (optional) and first_failed cross PCIe.  Fails when
+ * graph.n_witness != r1cs.n_wires. */
+int gw_calc_witness_batch_check(gw_graph_t *graph, gw_r1cs_t *r1cs, int first_device, int n_gpus, const uint8_t *inputs,
+                                size_t n_sets, uint8_t *witness, uint32_t *flags, uint32_t *first_failed,
+                                gw_status_t *status);
+
 /* CUDA device used by the single-witness entry points gw_calc_witness / gw_graph_calc_witness (default: the GW_DEVICE
  * environment variable, else device 0 of CUDA_VISIBLE_DEVICES).  Returns 1 if the device does not exist. */
 int gw_set_device(int device);

@@ -45,6 +45,28 @@ pub struct gw_graph_info_t {
     pub bit_wide: u32,
 }
 
+#[repr(C)]
+pub struct gw_r1cs_t {
+    _private: [u8; 0],
+}
+
+#[repr(C)]
+#[derive(Default, Clone, Copy)]
+pub struct gw_r1cs_info_t {
+    pub n_wires: u32,
+    pub n_pub_out: u32,
+    pub n_pub_in: u32,
+    pub n_prv_in: u32,
+    pub n_constraints: u32,
+    pub n_consts: u32,
+    pub n_labels: u64,
+    pub n_terms: u64,
+    pub n_mac_terms: u64,
+    pub n_chunks: u64,
+}
+
+pub const GW_R1CS_OK: u32 = 0xFFFF_FFFF;
+
 pub type gw_witness_chunk_fn = unsafe extern "C" fn(
     user: *mut c_void, device: c_int, first_set: usize, n_sets: usize, rows: *const u8, row_bytes: usize, flags: *const u32,
 ) -> c_int;
@@ -64,4 +86,15 @@ extern "C" {
                                         n_sets: usize, chunk_sets: usize, f: gw_witness_chunk_fn, user: *mut c_void,
                                         status: *mut gw_status_t) -> c_int;
     pub fn gw_wtns_header(n_witness: u32, dst76: *mut u8);
+    pub fn gw_r1cs_load(data: *const c_void, len: usize, r1cs: *mut *mut gw_r1cs_t, status: *mut gw_status_t) -> c_int;
+    pub fn gw_r1cs_free(r1cs: *mut gw_r1cs_t);
+    pub fn gw_r1cs_info(r1cs: *const gw_r1cs_t, info: *mut gw_r1cs_info_t) -> c_int;
+    pub fn gw_r1cs_check_batch(r1cs: *mut gw_r1cs_t, witness: *const u8, n_sets: usize, row_pitch: usize,
+                               first_failed: *mut u32, n_gpus: c_int, status: *mut gw_status_t) -> c_int;
+    pub fn gw_r1cs_check_batch_device(r1cs: *mut gw_r1cs_t, device: c_int, d_witness: *const c_void, n_sets: usize,
+                                      row_pitch: usize, d_first_failed: *mut u32, cuda_stream: *mut c_void,
+                                      status: *mut gw_status_t) -> c_int;
+    pub fn gw_calc_witness_batch_check(graph: *mut gw_graph_t, r1cs: *mut gw_r1cs_t, first_device: c_int, n_gpus: c_int,
+                                       inputs: *const u8, n_sets: usize, witness: *mut u8, flags: *mut u32,
+                                       first_failed: *mut u32, status: *mut gw_status_t) -> c_int;
 }
