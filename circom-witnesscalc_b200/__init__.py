@@ -54,6 +54,7 @@ class gw_r1cs_info_t(ctypes.Structure):
 
 
 R1CS_OK = 0xFFFFFFFF    # GW_R1CS_OK: every constraint holds
+R1CS_ABC_GROTH16 = 1    # GW_R1CS_ABC_GROTH16: ABC vectors in the Groth16 domain layout
 
 _libc = ctypes.CDLL(None)
 _libc.free.argtypes = [ctypes.c_void_p]
@@ -82,6 +83,11 @@ _L.gw_r1cs_free.argtypes = [_vp]
 _L.gw_r1cs_info.argtypes = [_vp, ctypes.POINTER(gw_r1cs_info_t)]
 _L.gw_r1cs_check_batch.argtypes = [_vp, _vp, _sz, _sz, _vp, ctypes.c_int, ctypes.POINTER(gw_status_t)]
 _L.gw_r1cs_check_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _sz, _vp, _vp, ctypes.POINTER(gw_status_t)]
+_L.gw_r1cs_abc_len.restype = ctypes.c_uint64
+_L.gw_r1cs_abc_len.argtypes = [_vp, ctypes.c_uint32]
+_L.gw_r1cs_abc_batch.argtypes = [_vp, _vp, _sz, _sz, _vp, _sz, ctypes.c_uint32, _vp, ctypes.c_int, ctypes.POINTER(gw_status_t)]
+_L.gw_r1cs_abc_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _sz, _vp, _sz, ctypes.c_uint32, _vp, _vp,
+                                        ctypes.POINTER(gw_status_t)]
 _L.gw_calc_witness_batch_check.argtypes = [_vp, _vp, ctypes.c_int, ctypes.c_int, _vp, _sz, _vp, _vp, _vp, ctypes.POINTER(gw_status_t)]
 _L.gw_set_device.argtypes = [ctypes.c_int]
 _L.gw_device_count.restype = ctypes.c_int
@@ -92,7 +98,8 @@ EXPORTS = ["gw_calc_witness", "gw_graph_load", "gw_graph_free", "gw_graph_info",
            "gw_graph_calc_witness", "gw_calc_witness_batch", "gw_calc_witness_batch_on", "gw_calc_witness_batch_device", "gw_calc_witness_latency", "gw_wtns_header",
            "gw_device_count", "gw_microbench_imad", "gw_inputs_parse_batch", "gw_wtns_file_size", "gw_calc_witness_batch_wtns",
            "gw_graph_select", "gw_calc_witness_batch_stream", "gw_set_device", "gw_r1cs_load", "gw_r1cs_free", "gw_r1cs_info",
-           "gw_r1cs_check_batch", "gw_r1cs_check_batch_device", "gw_calc_witness_batch_check"]
+           "gw_r1cs_check_batch", "gw_r1cs_check_batch_device", "gw_calc_witness_batch_check", "gw_r1cs_abc_len",
+           "gw_r1cs_abc_batch", "gw_r1cs_abc_batch_device"]
 
 
 class WitnessCalcError(RuntimeError):
@@ -366,4 +373,36 @@ class R1cs:
         st = gw_status_t()
         rc = _L.gw_r1cs_check_batch_device(self._h, device, d_witness_ptr, n_sets, row_pitch, d_first_failed_ptr, stream,
                                            ctypes.byref(st))
+        _check(rc, st)
+
+    def abc_len(self, groth16=False) -> int:
+        """entries per vector of one ABC row (gw_r1cs_abc_len): n_constraints, or the Groth16 domain size"""
+        return int(_L.gw_r1cs_abc_len(self._h, R1CS_ABC_GROTH16 if groth16 else 0))
+
+    def abc_batch(self, rows, groth16=False, row_pitch=0, n_gpus=1, n_sets=None, want_verdict=False):
+        """HOST rows as for check_batch -> uint8 [B, 3, n, 32]: <A_k,w>, <B_k,w>, <C_k,w> of every row (gw_r1cs_abc_batch);
+        with want_verdict also the uint32 [B] verdicts of check_batch, from the same pass."""
+        rows = np.ascontiguousarray(rows, dtype=np.uint8)
+        n_wires = self.info()["n_wires"]
+        pitch = row_pitch or n_wires * 32
+        if n_sets is None:
+            n_sets = rows.shape[0] if rows.ndim > 1 and not row_pitch else (rows.size // pitch if pitch else 0)
+        assert n_sets == 0 or (n_sets - 1) * pitch + n_wires * 32 <= rows.size, "rows too short"
+        n = self.abc_len(groth16)
+        out = np.empty((n_sets, 3, n, 32), dtype=np.uint8)
+        first = np.zeros(n_sets, dtype=np.uint32) if want_verdict else None
+        st = gw_status_t()
+        rc = _L.gw_r1cs_abc_batch(self._h, rows.ctypes.data, n_sets, pitch, out.ctypes.data, 0,
+                                  R1CS_ABC_GROTH16 if groth16 else 0, first.ctypes.data if want_verdict else None, n_gpus,
+                                  ctypes.byref(st))
+        _check(rc, st)
+        return (out, first) if want_verdict else out
+
+    def abc_batch_device(self, device, d_witness_ptr, n_sets, d_abc_ptr, row_pitch=0, abc_pitch=0, groth16=False,
+                         d_first_failed_ptr=None, stream=None):
+        """DEVICE pointers; asynchronous on `stream` (a cudaStream_t as int, None = default stream)
+        (gw_r1cs_abc_batch_device)."""
+        st = gw_status_t()
+        rc = _L.gw_r1cs_abc_batch_device(self._h, device, d_witness_ptr, n_sets, row_pitch, d_abc_ptr, abc_pitch,
+                                         R1CS_ABC_GROTH16 if groth16 else 0, d_first_failed_ptr, stream, ctypes.byref(st))
         _check(rc, st)

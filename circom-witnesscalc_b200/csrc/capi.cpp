@@ -299,6 +299,39 @@ int gw_r1cs_check_batch_device(gw_r1cs_t* r1cs, int device, const void* d_witnes
   });
 }
 
+uint64_t gw_r1cs_abc_len(const gw_r1cs_t* r1cs, uint32_t options) {
+  if (!r1cs) return 0;
+  try { return r1cs->r1cs->abc_len(options); } catch (...) { return 0; }
+}
+
+int gw_r1cs_abc_batch(gw_r1cs_t* r1cs, const uint8_t* witness, size_t n_sets, size_t row_pitch, uint8_t* abc, size_t abc_pitch,
+                      uint32_t options, uint32_t* first_failed, int n_gpus, gw_status_t* status) {
+  if (!r1cs || (n_sets && (!witness || !abc))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    R1cs& r = *r1cs->r1cs;
+    if (!row_pitch) row_pitch = (size_t)r.hdr.n_wires * 32;
+    if (!abc_pitch) abc_pitch = 3 * 32 * (size_t)r.abc_len(options);
+    r.abc_row_bytes(row_pitch, abc_pitch, options, false);          // the arguments first: no device is touched
+    if (!n_sets) return;
+    int ndev = cuda_device_count();
+    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
+    if (n_gpus < 1) n_gpus = 1;
+    if (n_gpus > ndev) throw Error("n_gpus exceeds the number of visible CUDA devices");
+    r.abc_host(witness, n_sets, row_pitch, abc, abc_pitch, options, first_failed, n_gpus, 0);
+  });
+}
+
+int gw_r1cs_abc_batch_device(gw_r1cs_t* r1cs, int device, const void* d_witness, size_t n_sets, size_t row_pitch, void* d_abc,
+                             size_t abc_pitch, uint32_t options, uint32_t* d_first_failed, void* cuda_stream, gw_status_t* status) {
+  if (!r1cs || (n_sets && (!d_witness || !d_abc))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    R1cs& r = *r1cs->r1cs;
+    if (!row_pitch) row_pitch = (size_t)r.hdr.n_wires * 32;
+    if (!abc_pitch) abc_pitch = 3 * 32 * (size_t)r.abc_len(options);
+    r.abc_device(device, d_witness, n_sets, row_pitch, d_abc, abc_pitch, options, d_first_failed, cuda_stream);
+  });
+}
+
 int gw_calc_witness_batch_check(gw_graph_t* graph, gw_r1cs_t* r1cs, int first_device, int n_gpus, const uint8_t* inputs,
                                 size_t n_sets, uint8_t* witness, uint32_t* flags, uint32_t* first_failed, gw_status_t* status) {
   if (!graph || !r1cs || (n_sets && (!inputs || !first_failed))) { set_status(status, ERROR, "null argument"); return 1; }

@@ -21,6 +21,7 @@
 namespace gw {
 
 static const uint32_t R1CS_OK = 0xFFFFFFFFu;        // GW_R1CS_OK: every constraint holds
+static const uint32_t R1CS_ABC_GROTH16 = 1u;        // GW_R1CS_ABC_GROTH16: the ABC vectors in the Groth16 domain layout
 
 struct R1csHeader {
   uint32_t n8 = 0, n_wires = 0, n_pub_out = 0, n_pub_in = 0, n_prv_in = 0, n_constraints = 0;
@@ -56,10 +57,26 @@ class R1cs {
   // host rows (row r at witness + r * row_pitch), sharded over n_gpus devices starting at first_device
   void check_host(const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, int n_gpus, int first_device);
 
+  // <A_k,w>, <B_k,w>, <C_k,w> per row (gw_r1cs_abc_batch): row r of the output at abc + r * abc_pitch is A | B | C, each
+  // abc_len(options) entries of 32 bytes.  first_failed (optional) receives the check's verdicts.
+  // entries per vector: n_constraints, or with R1CS_ABC_GROTH16 the smallest power of two >= n_constraints + n_pub + 1
+  uint64_t abc_len(uint32_t options) const;
+  // checks the layout arguments (device: 16-byte multiples too) without touching a device; returns 3 x n x 32
+  size_t abc_row_bytes(size_t row_pitch, size_t abc_pitch, uint32_t options, bool device) const;
+  void abc_device(int device, const void* d_witness, size_t B, size_t row_pitch, void* d_abc, size_t abc_pitch, uint32_t options,
+                  uint32_t* d_first_failed, void* stream);
+  void abc_host(const uint8_t* witness, size_t B, size_t row_pitch, uint8_t* abc, size_t abc_pitch, uint32_t options,
+                uint32_t* first_failed, int n_gpus, int first_device);
+
  private:
   struct Dev;
+  struct Launch;
+  struct AbcOut { uint8_t* abc; size_t pitch; uint32_t options; };
   Dev* dev(int device);
-  void check_host_on(int device, const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed);
+  Launch launch(Dev* d, const void* d_witness, size_t B, size_t row_pitch, uint32_t* d_first_failed) const;
+  void host_rows_on(int device, const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, const AbcOut* out);
+  void host_rows(const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, const AbcOut* out, int n_gpus,
+                 int first_device);
   std::map<int, Dev*> devs;
   std::mutex mu;
 };

@@ -44,4 +44,30 @@ GW_HD bool r1cs_holds(const fe& a, const fe& b, const fe& c) {
   return u256_eq(ab.l, c.l);
 }
 
+// A witness value as the ABC evaluation reads it: reduced mod M (like Fr::new on graph inputs), so that <A_k,w>,
+// <B_k,w> and <C_k,w> are defined for every row.  *reduced is set when x was >= M: the check's verdict still fails the
+// constraint that reads it.
+GW_HD fe r1cs_wire_reduce(fe x, bool* reduced) {
+  if (x.l[7] >= MOD_L(7) && fe_geq_m(x)) {
+    *reduced = true;
+    x = fe_reduce256(x);
+  }
+  return x;
+}
+
+// <A_k,w>, <B_k,w>, <C_k,w> of one constraint (its header and terms come from next): emit(which, value) receives each
+// value, canonical, as soon as it is reduced (which = 0, 1, 2 for A, B, C).  Wire values >= M are reduced
+// (r1cs_wire_reduce) and set *reduced.
+template <class Next, class WireVal, class ConstVal, class Emit>
+GW_HD void r1cs_abc(Next&& next, WireVal&& wire_val, ConstVal&& const_val, bool* reduced, Emit&& emit) {
+  uint32_t na, nb, nc, unused;
+  next(na, nb);
+  next(nc, unused);
+  auto wire = [&](uint32_t i) { return r1cs_wire_reduce(wire_val(i), reduced); };
+  bool never = false;                          // reduced values are < M: r1cs_lc never sets it
+#pragma unroll 1
+  for (int which = 0; which < 3; which++)      // one copy of the term loop for A, B and C
+    emit(which, r1cs_lc(which == 0 ? na : which == 1 ? nb : nc, next, wire, const_val, &never));
+}
+
 }  // namespace gw

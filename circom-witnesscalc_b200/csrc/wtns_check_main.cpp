@@ -1,15 +1,20 @@
-// wtns-check <circuit.r1cs> <witness.wtns> [more.wtns ...]
+// wtns-check [--all] <circuit.r1cs> <witness.wtns> [more.wtns ...]
 // Drop-in for `snarkjs wtns check circuit.r1cs witness.wtns`: checks that each witness satisfies the circuit's
 // constraints.  The .wtns headers are checked on the host (version 2, n8 = 32, BN254's prime, one value per wire);
 // the payloads of all files are checked on the GPU in one gw_r1cs_check_batch call.  Prints one line per file
 // ("OK" or "constraint k not satisfied") and exits 0 only if every file passes.
+// --all: the payloads go through one gw_r1cs_abc_batch call instead (plain layout, with the verdicts), and every failing
+// file gets one more line per violated constraint, "  constraint k: a * b != c" (decimal values of <A_k,w>, <B_k,w>,
+// <C_k,w>, with witness values reduced mod M), then one line per wire that holds a value >= M.
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
 #include "../../include/graph_witness.h"
+#include "r1cs_eval.cuh"
 
 static bool read_file(const char* path, std::vector<uint8_t>& out) {
   FILE* f = fopen(path, "rb");
@@ -63,9 +68,31 @@ static std::string parse_wtns(const std::vector<uint8_t>& b, uint32_t n_wires, s
   return "";
 }
 
+static std::string decimal(const uint8_t* v32) {
+  uint32_t l[8];
+  memcpy(l, v32, 32);
+  std::string s;
+  do {
+    uint64_t rem = 0;
+    for (int i = 7; i >= 0; i--) {
+      const uint64_t cur = (rem << 32) | l[i];
+      l[i] = (uint32_t)(cur / 10);
+      rem = cur % 10;
+    }
+    s.push_back((char)('0' + rem));
+  } while (std::any_of(l, l + 8, [](uint32_t x) { return x != 0; }));
+  std::reverse(s.begin(), s.end());
+  return s;
+}
+
+static gw::fe to_fe(const uint8_t* v32) { gw::fe r; memcpy(r.l, v32, 32); return r; }
+
 int main(int argc, char** argv) {
+  const char* prog = argv[0];
+  const bool all = argc > 1 && strcmp(argv[1], "--all") == 0;
+  if (all) { argv++; argc--; }
   if (argc < 3) {
-    fprintf(stderr, "Usage: %s <circuit.r1cs> <witness.wtns> [more.wtns ...]\n", argv[0]);
+    fprintf(stderr, "Usage: %s [--all] <circuit.r1cs> <witness.wtns> [more.wtns ...]\n", prog);
     return 1;
   }
   std::vector<uint8_t> r1cs_bytes;
@@ -94,7 +121,10 @@ int main(int argc, char** argv) {
     slot[i] = (int)n_rows++;
   }
   std::vector<uint32_t> first_failed(n_rows);
-  if (n_rows && gw_r1cs_check_batch(r, rows.data(), n_rows, row_b, first_failed.data(), 1, &st)) {
+  const size_t n_con = info.n_constraints, abc_b = 3 * 32 * n_con;
+  std::vector<uint8_t> abc(all ? n_rows * abc_b : 0);
+  if (n_rows && (all ? gw_r1cs_abc_batch(r, rows.data(), n_rows, row_b, abc.data(), abc_b, 0, first_failed.data(), 1, &st)
+                     : gw_r1cs_check_batch(r, rows.data(), n_rows, row_b, first_failed.data(), 1, &st))) {
     fprintf(stderr, "Error: %s\n", st.error_msg ? st.error_msg : "unknown");
     gw_free_status(&st);
     gw_r1cs_free(r);
@@ -105,6 +135,16 @@ int main(int argc, char** argv) {
     if (slot[i] >= 0) verdict[i] = first_failed[slot[i]] == GW_R1CS_OK ? "OK" : "constraint " + std::to_string(first_failed[slot[i]]) + " not satisfied";
     bad += verdict[i] != "OK";
     printf("%s: %s\n", argv[2 + i], verdict[i].c_str());
+    if (!all || slot[i] < 0 || first_failed[slot[i]] == GW_R1CS_OK) continue;
+    const uint8_t* a = abc.data() + slot[i] * abc_b;
+    for (size_t k = 0; k < n_con; k++) {
+      const uint8_t *ak = a + 32 * k, *bk = ak + 32 * n_con, *ck = bk + 32 * n_con;
+      if (!gw::r1cs_holds(to_fe(ak), to_fe(bk), to_fe(ck)))
+        printf("  constraint %zu: %s * %s != %s\n", k, decimal(ak).c_str(), decimal(bk).c_str(), decimal(ck).c_str());
+    }
+    const uint8_t* w = rows.data() + slot[i] * row_b;
+    for (uint32_t j = 0; j < info.n_wires; j++)
+      if (gw::fe_geq_m(to_fe(w + 32 * (size_t)j))) printf("  wire %u: %s >= M\n", j, decimal(w + 32 * (size_t)j).c_str());
   }
   gw_r1cs_free(r);
   return bad ? 1 : 0;

@@ -215,6 +215,30 @@ int gw_calc_witness_batch_check(gw_graph_t *graph, gw_r1cs_t *r1cs, int first_de
                                 size_t n_sets, uint8_t *witness, uint32_t *flags, uint32_t *first_failed,
                                 gw_status_t *status);
 
+/* ---- A, B and C of witness rows (the witness-dependent product of a prover, snarkjs / rapidsnark `buildABC`) ----
+ * For every constraint k of row w: a_k = <A_k,w>, b_k = <B_k,w>, c_k = <C_k,w> (mod M), 32 bytes each, canonical
+ * little-endian.  Output row = A[0..n) | B[0..n) | C[0..n).  A witness value >= M is reduced mod M before it enters a
+ * linear combination.  first_failed (optional, may be NULL) receives the verdicts of gw_r1cs_check_batch, computed in
+ * the same pass.
+ *   options = 0                   n = n_constraints.
+ *   options = GW_R1CS_ABC_GROTH16 the domain of a Groth16 prover (snarkjs zkey setup, read by rapidsnark): n = the
+ *                                 smallest power of two >= n_constraints + n_pub + 1 (n_pub = n_pub_out + n_pub_in);
+ *                                 entry n_constraints + s, s = 0 .. n_pub, has A = w_s and B = C = 0; the rest is 0. */
+#define GW_R1CS_ABC_GROTH16 1u
+/* entries per vector of one row: n_constraints, or with GW_R1CS_ABC_GROTH16 the power of two above; 0 for unknown
+ * options or when the public signals do not fit the wires */
+uint64_t gw_r1cs_abc_len(const gw_r1cs_t *r1cs, uint32_t options);
+/* HOST rows (as gw_r1cs_check_batch: row_pitch 0 = dense, .wtns images in place with witness = files + 76);
+ * abc: row r at abc + r * abc_pitch, abc_pitch >= 3 * n * 32 (0 = dense); bytes past 3 * n * 32 are not written;
+ * first_failed optional; sharded over n_gpus devices.  n_sets = 0 does nothing. */
+int gw_r1cs_abc_batch(gw_r1cs_t *r1cs, const uint8_t *witness, size_t n_sets, size_t row_pitch, uint8_t *abc,
+                      size_t abc_pitch, uint32_t options, uint32_t *first_failed, int n_gpus, gw_status_t *status);
+/* DEVICE buffers on `device` (16-byte aligned, pitches multiples of 16), asynchronous on cuda_stream (NULL = default
+ * stream): composes with gw_calc_witness_batch_device on the same stream */
+int gw_r1cs_abc_batch_device(gw_r1cs_t *r1cs, int device, const void *d_witness, size_t n_sets, size_t row_pitch,
+                             void *d_abc, size_t abc_pitch, uint32_t options, uint32_t *d_first_failed,
+                             void *cuda_stream, gw_status_t *status);
+
 /* CUDA device used by the single-witness entry points gw_calc_witness / gw_graph_calc_witness (default: the GW_DEVICE
  * environment variable, else device 0 of CUDA_VISIBLE_DEVICES).  Returns 1 if the device does not exist. */
 int gw_set_device(int device);

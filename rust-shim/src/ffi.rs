@@ -66,6 +66,7 @@ pub struct gw_r1cs_info_t {
 }
 
 pub const GW_R1CS_OK: u32 = 0xFFFF_FFFF;
+pub const GW_R1CS_ABC_GROTH16: u32 = 1;
 
 pub type gw_witness_chunk_fn = unsafe extern "C" fn(
     user: *mut c_void, device: c_int, first_set: usize, n_sets: usize, rows: *const u8, row_bytes: usize, flags: *const u32,
@@ -97,4 +98,12 @@ extern "C" {
     pub fn gw_calc_witness_batch_check(graph: *mut gw_graph_t, r1cs: *mut gw_r1cs_t, first_device: c_int, n_gpus: c_int,
                                        inputs: *const u8, n_sets: usize, witness: *mut u8, flags: *mut u32,
                                        first_failed: *mut u32, status: *mut gw_status_t) -> c_int;
+    pub fn gw_r1cs_abc_len(r1cs: *const gw_r1cs_t, options: u32) -> u64;
+    pub fn gw_r1cs_abc_batch(r1cs: *mut gw_r1cs_t, witness: *const u8, n_sets: usize, row_pitch: usize, abc: *mut u8,
+                             abc_pitch: usize, options: u32, first_failed: *mut u32, n_gpus: c_int,
+                             status: *mut gw_status_t) -> c_int;
+    pub fn gw_r1cs_abc_batch_device(r1cs: *mut gw_r1cs_t, device: c_int, d_witness: *const c_void, n_sets: usize,
+                                    row_pitch: usize, d_abc: *mut c_void, abc_pitch: usize, options: u32,
+                                    d_first_failed: *mut u32, cuda_stream: *mut c_void,
+                                    status: *mut gw_status_t) -> c_int;
 }
