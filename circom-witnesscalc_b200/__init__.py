@@ -55,6 +55,8 @@ class gw_r1cs_info_t(ctypes.Structure):
 
 R1CS_OK = 0xFFFFFFFF    # GW_R1CS_OK: every constraint holds
 R1CS_ABC_GROTH16 = 1    # GW_R1CS_ABC_GROTH16: ABC vectors in the Groth16 domain layout
+NTT_INVERSE = 1         # GW_NTT_INVERSE
+NTT_COSET = 2           # GW_NTT_COSET
 
 _libc = ctypes.CDLL(None)
 _libc.free.argtypes = [ctypes.c_void_p]
@@ -88,6 +90,9 @@ _L.gw_r1cs_abc_len.argtypes = [_vp, ctypes.c_uint32]
 _L.gw_r1cs_abc_batch.argtypes = [_vp, _vp, _sz, _sz, _vp, _sz, ctypes.c_uint32, _vp, ctypes.c_int, ctypes.POINTER(gw_status_t)]
 _L.gw_r1cs_abc_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _sz, _vp, _sz, ctypes.c_uint32, _vp, _vp,
                                         ctypes.POINTER(gw_status_t)]
+_L.gw_fr_ntt_batch_device.argtypes = [ctypes.c_int, _vp, _sz, ctypes.c_uint32, _sz, ctypes.c_uint32, _vp, ctypes.POINTER(gw_status_t)]
+_L.gw_r1cs_quotient_batch.argtypes = [_vp, _vp, _sz, _sz, _vp, _sz, _vp, ctypes.c_int, ctypes.POINTER(gw_status_t)]
+_L.gw_r1cs_quotient_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _sz, _vp, _sz, _vp, _vp, ctypes.POINTER(gw_status_t)]
 _L.gw_calc_witness_batch_check.argtypes = [_vp, _vp, ctypes.c_int, ctypes.c_int, _vp, _sz, _vp, _vp, _vp, ctypes.POINTER(gw_status_t)]
 _L.gw_set_device.argtypes = [ctypes.c_int]
 _L.gw_device_count.restype = ctypes.c_int
@@ -99,7 +104,8 @@ EXPORTS = ["gw_calc_witness", "gw_graph_load", "gw_graph_free", "gw_graph_info",
            "gw_device_count", "gw_microbench_imad", "gw_inputs_parse_batch", "gw_wtns_file_size", "gw_calc_witness_batch_wtns",
            "gw_graph_select", "gw_calc_witness_batch_stream", "gw_set_device", "gw_r1cs_load", "gw_r1cs_free", "gw_r1cs_info",
            "gw_r1cs_check_batch", "gw_r1cs_check_batch_device", "gw_calc_witness_batch_check", "gw_r1cs_abc_len",
-           "gw_r1cs_abc_batch", "gw_r1cs_abc_batch_device"]
+           "gw_r1cs_abc_batch", "gw_r1cs_abc_batch_device", "gw_fr_ntt_batch_device", "gw_r1cs_quotient_batch",
+           "gw_r1cs_quotient_batch_device"]
 
 
 class WitnessCalcError(RuntimeError):
@@ -153,6 +159,14 @@ def set_device(device: int):
 
 def device_count() -> int:
     return _L.gw_device_count()
+
+
+def ntt_batch_device(device, d_data_ptr, n_vectors, log_n, pitch=0, flags=0, stream=None):
+    """DEVICE pointer: n_vectors transforms of 2^log_n 32-byte entries in place, vector v at d_data_ptr + v * pitch
+    (pitch 0 = dense); flags NTT_INVERSE | NTT_COSET; asynchronous on `stream` (gw_fr_ntt_batch_device)."""
+    st = gw_status_t()
+    rc = _L.gw_fr_ntt_batch_device(device, d_data_ptr, n_vectors, log_n, pitch, flags, stream, ctypes.byref(st))
+    _check(rc, st)
 
 
 def microbench_imad(device=0, which=0) -> float:
@@ -405,4 +419,31 @@ class R1cs:
         st = gw_status_t()
         rc = _L.gw_r1cs_abc_batch_device(self._h, device, d_witness_ptr, n_sets, row_pitch, d_abc_ptr, abc_pitch,
                                          R1CS_ABC_GROTH16 if groth16 else 0, d_first_failed_ptr, stream, ctypes.byref(st))
+        _check(rc, st)
+
+    def quotient_batch(self, rows, row_pitch=0, n_gpus=1, n_sets=None, want_verdict=False):
+        """HOST rows as for check_batch -> uint8 [B, n, 32] (n = abc_len(groth16=True)): the Groth16 quotient evaluations
+        h = A_odd * B_odd - C_odd of every row (gw_r1cs_quotient_batch); with want_verdict also the uint32 [B] verdicts
+        of check_batch, from the same pass."""
+        rows = np.ascontiguousarray(rows, dtype=np.uint8)
+        n_wires = self.info()["n_wires"]
+        pitch = row_pitch or n_wires * 32
+        if n_sets is None:
+            n_sets = rows.shape[0] if rows.ndim > 1 and not row_pitch else (rows.size // pitch if pitch else 0)
+        assert n_sets == 0 or (n_sets - 1) * pitch + n_wires * 32 <= rows.size, "rows too short"
+        out = np.empty((n_sets, self.abc_len(groth16=True), 32), dtype=np.uint8)
+        first = np.zeros(n_sets, dtype=np.uint32) if want_verdict else None
+        st = gw_status_t()
+        rc = _L.gw_r1cs_quotient_batch(self._h, rows.ctypes.data, n_sets, pitch, out.ctypes.data, 0,
+                                       first.ctypes.data if want_verdict else None, n_gpus, ctypes.byref(st))
+        _check(rc, st)
+        return (out, first) if want_verdict else out
+
+    def quotient_batch_device(self, device, d_witness_ptr, n_sets, d_work_ptr, row_pitch=0, work_pitch=0,
+                              d_first_failed_ptr=None, stream=None):
+        """DEVICE pointers; work rows of at least 3 x n x 32 bytes, h left in the first n x 32 bytes of each;
+        asynchronous on `stream` (gw_r1cs_quotient_batch_device)."""
+        st = gw_status_t()
+        rc = _L.gw_r1cs_quotient_batch_device(self._h, device, d_witness_ptr, n_sets, row_pitch, d_work_ptr, work_pitch,
+                                              d_first_failed_ptr, stream, ctypes.byref(st))
         _check(rc, st)

@@ -12,6 +12,7 @@
 
 #include "engine.hpp"
 #include "inputs.hpp"
+#include "ntt.hpp"
 #include "wtns.hpp"
 
 using namespace gw;
@@ -329,6 +330,40 @@ int gw_r1cs_abc_batch_device(gw_r1cs_t* r1cs, int device, const void* d_witness,
     if (!row_pitch) row_pitch = (size_t)r.hdr.n_wires * 32;
     if (!abc_pitch) abc_pitch = 3 * 32 * (size_t)r.abc_len(options);
     r.abc_device(device, d_witness, n_sets, row_pitch, d_abc, abc_pitch, options, d_first_failed, cuda_stream);
+  });
+}
+
+int gw_fr_ntt_batch_device(int device, void* d_data, size_t n_vectors, uint32_t log_n, size_t pitch, uint32_t flags,
+                           void* cuda_stream, gw_status_t* status) {
+  if (n_vectors && !d_data) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() { ntt_batch_device(device, d_data, n_vectors, log_n, pitch, flags, cuda_stream); });
+}
+
+int gw_r1cs_quotient_batch(gw_r1cs_t* r1cs, const uint8_t* witness, size_t n_sets, size_t row_pitch, uint8_t* h, size_t h_pitch,
+                           uint32_t* first_failed, int n_gpus, gw_status_t* status) {
+  if (!r1cs || (n_sets && (!witness || !h))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    R1cs& r = *r1cs->r1cs;
+    if (!row_pitch) row_pitch = (size_t)r.hdr.n_wires * 32;
+    if (!h_pitch) h_pitch = 32 * (size_t)r.abc_len(GW_R1CS_ABC_GROTH16);
+    r.quotient_log_n(row_pitch, h_pitch, false);                    // the arguments first: no device is touched
+    if (!n_sets) return;
+    int ndev = cuda_device_count();
+    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
+    if (n_gpus < 1) n_gpus = 1;
+    if (n_gpus > ndev) throw Error("n_gpus exceeds the number of visible CUDA devices");
+    r.quotient_host(witness, n_sets, row_pitch, h, h_pitch, first_failed, n_gpus, 0);
+  });
+}
+
+int gw_r1cs_quotient_batch_device(gw_r1cs_t* r1cs, int device, const void* d_witness, size_t n_sets, size_t row_pitch, void* d_work,
+                                  size_t work_pitch, uint32_t* d_first_failed, void* cuda_stream, gw_status_t* status) {
+  if (!r1cs || (n_sets && (!d_witness || !d_work))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    R1cs& r = *r1cs->r1cs;
+    if (!row_pitch) row_pitch = (size_t)r.hdr.n_wires * 32;
+    if (!work_pitch) work_pitch = 3 * 32 * (size_t)r.abc_len(GW_R1CS_ABC_GROTH16);
+    r.quotient_device(device, d_witness, n_sets, row_pitch, d_work, work_pitch, d_first_failed, cuda_stream);
   });
 }
 

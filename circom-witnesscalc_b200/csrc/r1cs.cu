@@ -17,6 +17,7 @@
 #include <vector>
 
 #include "cuda_util.hpp"
+#include "ntt.hpp"
 #include "r1cs.hpp"
 #include "r1cs_eval.cuh"
 
@@ -338,14 +339,16 @@ struct Drain {
 };
 }  // namespace
 
-// host rows: chunked, double-buffered H2D (pitched) -> check or ABC -> D2H of the results on two streams.  out == NULL:
-// the check; else the ABC vectors (and the verdicts when first_failed is not NULL).
+// host rows: chunked, double-buffered H2D (pitched) -> check, ABC or quotient -> D2H of the results on two streams.
+// out == NULL: the check; else the ABC vectors or h (and the verdicts when first_failed is not NULL).  The chunk size
+// counts the 3 x n x 32 device bytes of a row in both output modes; only h (n x 32 bytes) of a quotient row is copied.
 void R1cs::host_rows_on(int device, const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, const AbcOut* out) {
   Dev* d = dev(device);
   DeviceGuard on(device);
   std::lock_guard<std::mutex> lk(d->mu);
   const size_t row_b = (size_t)hdr.n_wires * 32, dev_row = std::max<size_t>(row_b, 16);
   const size_t out_row = out ? 3 * 32 * (size_t)abc_len(out->options) : 0;
+  const size_t copy_b = out && out->quotient ? out_row / 3 : out_row;       // bytes of a result row copied back
   size_t free_b = 0, total_b = 0;
   CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
   // two staging buffers of at most 8 GiB each, and together at most 2/5 of what is free
@@ -377,10 +380,11 @@ void R1cs::host_rows_on(int device, const uint8_t* witness, size_t B, size_t row
     else CUDA_CHECK(cudaMemcpy2DAsync(d->d_rows[k], dev_row, witness + off * row_pitch, row_pitch, row_b, nb, cudaMemcpyHostToDevice, s));
     if (!out) check_device(device, d->d_rows[k], nb, dev_row, d->d_ff[k], s);
     else {
-      abc_device(device, d->d_rows[k], nb, dev_row, d->d_out[k], out_row, out->options, first_failed ? d->d_ff[k] : nullptr, s);
+      if (out->quotient) quotient_device(device, d->d_rows[k], nb, dev_row, d->d_out[k], out_row, first_failed ? d->d_ff[k] : nullptr, s);
+      else abc_device(device, d->d_rows[k], nb, dev_row, d->d_out[k], out_row, out->options, first_failed ? d->d_ff[k] : nullptr, s);
       if (out_row == 0) {}
-      else if (out->pitch == out_row) CUDA_CHECK(cudaMemcpyAsync(out->abc + off * out_row, d->d_out[k], nb * out_row, cudaMemcpyDeviceToHost, s));
-      else CUDA_CHECK(cudaMemcpy2DAsync(out->abc + off * out->pitch, out->pitch, d->d_out[k], out_row, out_row, nb, cudaMemcpyDeviceToHost, s));
+      else if (out->pitch == out_row && copy_b == out_row) CUDA_CHECK(cudaMemcpyAsync(out->abc + off * out_row, d->d_out[k], nb * out_row, cudaMemcpyDeviceToHost, s));
+      else CUDA_CHECK(cudaMemcpy2DAsync(out->abc + off * out->pitch, out->pitch, d->d_out[k], out_row, copy_b, nb, cudaMemcpyDeviceToHost, s));
     }
     if (first_failed) CUDA_CHECK(cudaMemcpyAsync(first_failed + off, d->d_ff[k], nb * 4, cudaMemcpyDeviceToHost, s));
   }
@@ -402,7 +406,7 @@ void R1cs::host_rows(const uint8_t* witness, size_t B, size_t row_pitch, uint32_
       try {
         bind_thread_near_device(first_device + g);
         AbcOut shard;
-        if (out) shard = AbcOut{out->abc + lo * out->pitch, out->pitch, out->options};
+        if (out) shard = AbcOut{out->abc + lo * out->pitch, out->pitch, out->options, out->quotient};
         host_rows_on(first_device + g, witness + lo * row_pitch, hi - lo, row_pitch, first_failed ? first_failed + lo : nullptr,
                      out ? &shard : nullptr);
       } catch (const std::exception& e) { errs[g] = e.what(); }
@@ -420,7 +424,36 @@ void R1cs::check_host(const uint8_t* witness, size_t B, size_t row_pitch, uint32
 void R1cs::abc_host(const uint8_t* witness, size_t B, size_t row_pitch, uint8_t* abc, size_t abc_pitch, uint32_t options,
                     uint32_t* first_failed, int n_gpus, int first_device) {
   abc_row_bytes(row_pitch, abc_pitch, options, false);
-  const AbcOut out{abc, abc_pitch, options};
+  const AbcOut out{abc, abc_pitch, options, false};
+  host_rows(witness, B, row_pitch, first_failed, &out, n_gpus, first_device);
+}
+
+uint32_t R1cs::quotient_log_n(size_t row_pitch, size_t out_pitch, bool device) const {
+  const uint64_t n = abc_len(R1CS_ABC_GROTH16);
+  uint32_t log_n = 0;
+  while ((1ull << log_n) < n) log_n++;
+  if (log_n > NTT_MAX_LOG)
+    throw Error("r1cs: the Groth16 domain 2^" + std::to_string(log_n) + " is larger than 2^24: domains above 2^24 are not supported");
+  if (row_pitch < (size_t)hdr.n_wires * 32) throw Error("row_pitch is smaller than n_wires x 32 bytes");
+  if (device && out_pitch < 3 * 32 * n) throw Error("work_pitch is smaller than 3 x n x 32 bytes (n = gw_r1cs_abc_len)");
+  if (!device && out_pitch < 32 * n) throw Error("h_pitch is smaller than n x 32 bytes (n = gw_r1cs_abc_len)");
+  if (device && (row_pitch % 16 || out_pitch % 16)) throw Error("device rows must be 16-byte aligned (row_pitch and work_pitch multiples of 16)");
+  return log_n;
+}
+
+void R1cs::quotient_device(int device, const void* d_witness, size_t B, size_t row_pitch, void* d_work, size_t work_pitch,
+                           uint32_t* d_first_failed, void* stream) {
+  const uint32_t log_n = quotient_log_n(row_pitch, work_pitch, true);
+  if (((uintptr_t)d_witness & 15) || ((uintptr_t)d_work & 15)) throw Error("device buffers must be 16-byte aligned");
+  if (B == 0) return;
+  abc_device(device, d_witness, B, row_pitch, d_work, work_pitch, R1CS_ABC_GROTH16, d_first_failed, stream);
+  ntt_quotient_device(device, d_work, B, log_n, work_pitch, stream);
+}
+
+void R1cs::quotient_host(const uint8_t* witness, size_t B, size_t row_pitch, uint8_t* h, size_t h_pitch, uint32_t* first_failed,
+                         int n_gpus, int first_device) {
+  quotient_log_n(row_pitch, h_pitch, false);
+  const AbcOut out{h, h_pitch, R1CS_ABC_GROTH16, true};
   host_rows(witness, B, row_pitch, first_failed, &out, n_gpus, first_device);
 }
 

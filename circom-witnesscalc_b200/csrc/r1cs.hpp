@@ -68,10 +68,21 @@ class R1cs {
   void abc_host(const uint8_t* witness, size_t B, size_t row_pitch, uint8_t* abc, size_t abc_pitch, uint32_t options,
                 uint32_t* first_failed, int n_gpus, int first_device);
 
+  // Groth16 quotient evaluations per row (gw_r1cs_quotient_batch): with n = abc_len(R1CS_ABC_GROTH16) and X_odd the
+  // coset forward transform of the inverse transform of X (ntt.hpp), h_i = A_odd[i] * B_odd[i] - C_odd[i].
+  // Device: abc_device into the work rows (d_work + r * work_pitch, work_pitch >= 3 x n x 32), then the transforms in
+  // place, all on `stream`; h is left in the first n x 32 bytes of each work row.  Host: h row r at h + r * h_pitch.
+  // checks the layout arguments without touching a device; returns log2(n)
+  uint32_t quotient_log_n(size_t row_pitch, size_t out_pitch, bool device) const;
+  void quotient_device(int device, const void* d_witness, size_t B, size_t row_pitch, void* d_work, size_t work_pitch,
+                       uint32_t* d_first_failed, void* stream);
+  void quotient_host(const uint8_t* witness, size_t B, size_t row_pitch, uint8_t* h, size_t h_pitch, uint32_t* first_failed,
+                     int n_gpus, int first_device);
+
  private:
   struct Dev;
   struct Launch;
-  struct AbcOut { uint8_t* abc; size_t pitch; uint32_t options; };
+  struct AbcOut { uint8_t* abc; size_t pitch; uint32_t options; bool quotient; };   // quotient: h only (n x 32 bytes per row)
   Dev* dev(int device);
   Launch launch(Dev* d, const void* d_witness, size_t B, size_t row_pitch, uint32_t* d_first_failed) const;
   void host_rows_on(int device, const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, const AbcOut* out);

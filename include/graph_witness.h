@@ -239,6 +239,36 @@ int gw_r1cs_abc_batch_device(gw_r1cs_t *r1cs, int device, const void *d_witness,
                              void *d_abc, size_t abc_pitch, uint32_t options, uint32_t *d_first_failed,
                              void *cuda_stream, gw_status_t *status);
 
+/* ---- Groth16 quotient evaluations and batched NTTs over the BN254 scalar field (M - 1 = 2^28 t) ----
+ * w_28 = 5^t mod M (ffjavascript Fr.w[28], rapidsnark FFT); for n = 2^k: w_n = w_28^(2^(28 - k)), g = w_2n.
+ * gw_fr_ntt_batch_device: in place, natural order in and out; vector v at d_data + v * pitch (pitch 0 = dense, else
+ * >= n * 32 and a multiple of 16; d_data 16-byte aligned); inputs are any 256-bit values (reduced mod M), outputs
+ * canonical 32-byte little-endian.  0 <= log_n <= 24.  Asynchronous on cuda_stream (NULL = default stream).
+ *   flags 0                              y_j = sum_i x_i w_n^(ij)
+ *   GW_NTT_INVERSE                       x_i = n^-1 sum_j y_j w_n^(-ij)
+ *   GW_NTT_COSET                         y_j = sum_i x_i (g w_n^j)^i   (the input is multiplied by g^i first)
+ *   GW_NTT_COSET | GW_NTT_INVERSE        the exact inverse of the coset transform (output i multiplied by g^-i)
+ * n_vectors = 0 does nothing. */
+#define GW_NTT_INVERSE 1u
+#define GW_NTT_COSET 2u
+int gw_fr_ntt_batch_device(int device, void *d_data, size_t n_vectors, uint32_t log_n, size_t pitch, uint32_t flags,
+                           void *cuda_stream, gw_status_t *status);
+/* h of every witness row (snarkjs groth16_prove joinABC, rapidsnark's vector before the H multi-scalar
+ * multiplication): with n = gw_r1cs_abc_len(r1cs, GW_R1CS_ABC_GROTH16) and A, B, C the Groth16-layout vectors of
+ * gw_r1cs_abc_batch, X_odd = the coset transform (GW_NTT_COSET) of the inverse transform (GW_NTT_INVERSE) of X and
+ * h_i = A_odd[i] * B_odd[i] - C_odd[i] (mod M), i = 0 .. n - 1, 32 bytes each, canonical.  n > 2^24 is rejected.
+ * first_failed (optional) receives the verdicts of gw_r1cs_check_batch from the same pass.
+ * HOST rows as gw_r1cs_abc_batch (row_pitch 0 = dense, .wtns images in place with witness = files + 76); h row r at
+ * h + r * h_pitch, h_pitch >= n * 32 (0 = dense); sharded over n_gpus devices.  n_sets = 0 does nothing. */
+int gw_r1cs_quotient_batch(gw_r1cs_t *r1cs, const uint8_t *witness, size_t n_sets, size_t row_pitch, uint8_t *h,
+                           size_t h_pitch, uint32_t *first_failed, int n_gpus, gw_status_t *status);
+/* DEVICE buffers on `device` (16-byte aligned, pitches multiples of 16), asynchronous on cuda_stream: work row r at
+ * d_work + r * work_pitch, work_pitch >= 3 * n * 32 (0 = dense); h is left in the first n * 32 bytes of each work row,
+ * the rest of the row is scratch.  Composes with gw_calc_witness_batch_device on the same stream. */
+int gw_r1cs_quotient_batch_device(gw_r1cs_t *r1cs, int device, const void *d_witness, size_t n_sets, size_t row_pitch,
+                                  void *d_work, size_t work_pitch, uint32_t *d_first_failed, void *cuda_stream,
+                                  gw_status_t *status);
+
 /* CUDA device used by the single-witness entry points gw_calc_witness / gw_graph_calc_witness (default: the GW_DEVICE
  * environment variable, else device 0 of CUDA_VISIBLE_DEVICES).  Returns 1 if the device does not exist. */
 int gw_set_device(int device);

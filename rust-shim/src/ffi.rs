@@ -67,6 +67,8 @@ pub struct gw_r1cs_info_t {
 
 pub const GW_R1CS_OK: u32 = 0xFFFF_FFFF;
 pub const GW_R1CS_ABC_GROTH16: u32 = 1;
+pub const GW_NTT_INVERSE: u32 = 1;
+pub const GW_NTT_COSET: u32 = 2;
 
 pub type gw_witness_chunk_fn = unsafe extern "C" fn(
     user: *mut c_void, device: c_int, first_set: usize, n_sets: usize, rows: *const u8, row_bytes: usize, flags: *const u32,
@@ -106,4 +108,11 @@ extern "C" {
                                     row_pitch: usize, d_abc: *mut c_void, abc_pitch: usize, options: u32,
                                     d_first_failed: *mut u32, cuda_stream: *mut c_void,
                                     status: *mut gw_status_t) -> c_int;
+    pub fn gw_fr_ntt_batch_device(device: c_int, d_data: *mut c_void, n_vectors: usize, log_n: u32, pitch: usize, flags: u32,
+                                  cuda_stream: *mut c_void, status: *mut gw_status_t) -> c_int;
+    pub fn gw_r1cs_quotient_batch(r1cs: *mut gw_r1cs_t, witness: *const u8, n_sets: usize, row_pitch: usize, h: *mut u8,
+                                  h_pitch: usize, first_failed: *mut u32, n_gpus: c_int, status: *mut gw_status_t) -> c_int;
+    pub fn gw_r1cs_quotient_batch_device(r1cs: *mut gw_r1cs_t, device: c_int, d_witness: *const c_void, n_sets: usize,
+                                         row_pitch: usize, d_work: *mut c_void, work_pitch: usize, d_first_failed: *mut u32,
+                                         cuda_stream: *mut c_void, status: *mut gw_status_t) -> c_int;
 }
