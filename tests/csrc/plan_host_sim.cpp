@@ -22,7 +22,8 @@ static fe to_fe(const U256& v) { fe r; memcpy(r.l, v.l, 32); return r; }
 
 extern "C" {
 
-// flags: bit 0 = fuse linear combinations (OP_DOT), bit 1 = narrow typing OFF, bit 2 = OP_POW5 fusion OFF, bits 8.. = div_batch (0 -> default)
+// flags: bit 0 = fuse linear combinations (OP_DOT), bit 1 = narrow typing OFF, bit 2 = OP_POW5 fusion OFF,
+// bits 8..15 = div_batch, bits 16..23 = max_terms (0 -> default, like GW_DIV_BATCH / GW_MAX_TERMS unset)
 SimGraph* sim_load2(const uint8_t* data, size_t len, uint32_t n_regs, int flags, char* err, size_t errlen);
 SimGraph* sim_load(const uint8_t* data, size_t len, uint32_t n_regs, char* err, size_t errlen) {
   return sim_load2(data, len, n_regs, 1, err, errlen);
@@ -32,12 +33,19 @@ SimGraph* sim_load2(const uint8_t* data, size_t len, uint32_t n_regs, int flags,
     std::unique_ptr<SimGraph> s(new SimGraph());
     s->g = deserialize_witnesscalc_graph(data, len);
     PlanOptions o; o.n_regs = n_regs; o.fuse_dot = (flags & 1) != 0; o.narrow = (flags & 2) == 0; o.fuse_pow5 = (flags & 4) == 0;
-    if (flags >> 8) o.div_batch = (uint32_t)(flags >> 8);
+    if ((flags >> 8) & 0xFF) o.div_batch = (uint32_t)((flags >> 8) & 0xFF);
+    if ((flags >> 16) & 0xFF) o.max_terms = (uint32_t)((flags >> 16) & 0xFF);
     s->plan = compile_plan(s->g, o);
     return s.release();
   } catch (const std::exception& e) { if (err && errlen) { strncpy(err, e.what(), errlen - 1); err[errlen - 1] = 0; } return nullptr; }
 }
 void sim_free(SimGraph* s) { delete s; }
+// the compiled program: copies up to cap slots (4 words each: x, y, z, w) and returns the number of slots
+size_t sim_code(SimGraph* s, uint32_t* out, size_t cap) {
+  const std::vector<Instr>& c = s->plan.code;
+  for (size_t i = 0; i < c.size() && i < cap; i++) { out[4 * i] = c[i].x; out[4 * i + 1] = c[i].y; out[4 * i + 2] = c[i].z; out[4 * i + 3] = c[i].w; }
+  return c.size();
+}
 void sim_info2(SimGraph* s, uint64_t* out) { out[0] = s->plan.stats.narrow_instrs; out[1] = s->plan.stats.op_count[OP_WIDEN]; out[2] = s->plan.n_spill_narrow; out[3] = s->plan.stats.pow5; }
 void sim_info(SimGraph* s, uint64_t* out) {
   const PlanStats& st = s->plan.stats;

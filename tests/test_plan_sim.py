@@ -3,6 +3,7 @@ witness placement) executed by the host simulator with the same alu_exec() the k
 the Python oracle.  No GPU needed."""
 import random
 
+import numpy as np
 import pytest
 
 from tests import util
@@ -297,3 +298,55 @@ def test_poseidon_like_graphs():
         g = _check(nodes, wit, imap, rnd.choice([6, 8, 12, 24]), rnd, n_rows=2)
         fused += g.info["pow5"]
     assert fused > 100
+
+
+def matrix_corpus():
+    """The corpus of the plan-option matrix (here on the simulator, tests/test_gpu_plan_matrix.py on the GPU):
+    [(name, nodes, witness, input map, rows)].  DOT ladder (1..16 terms at every ring offset, worst-case operands),
+    Div groups of 1..16 with their zero patterns, the narrow range limits, a constant-heavy graph, and random, linear-
+    combination, narrow and Poseidon-like graphs."""
+    M = po.M
+    out = []
+    rnd = random.Random(2024)
+    for t in range(1, 17):
+        nodes, wit, imap = util.dot_ladder_graph(t)
+        rows = [[1] + [M - 1] * 6, [1] + [0] * 6, [1] + [(1 << 256) - 1] * 6] + [util.matrix_row(rnd, 6) for _ in range(3)]
+        out.append((f"dot_ladder_{t}", nodes, wit, imap, rows))
+    for k in range(1, 17):
+        nodes, wit, imap = util.div_group_graph(k)
+        out.append((f"div_group_{k}", nodes, wit, imap, util.div_group_rows(k, rnd)))
+    for bits, nodes, wit, imap in util.narrow_limit_graphs():
+        vals = util.narrow_limit_values(bits)
+        out.append((f"narrow_limits_{bits}", nodes, wit, imap, [[1, x, y] for x in vals for y in vals]))
+    nodes, wit, imap = util.const_heavy_graph(rnd)
+    out.append(("const_heavy", nodes, wit, imap, [util.matrix_row(rnd, 6) for _ in range(6)] + [[1] + [M - 1] * 6]))
+    for k in range(2):
+        for name, gen in (("random", lambda: util.random_graph(rnd, n_ops=400)), ("lc", lambda: _lc_graph(rnd)),
+                          ("narrow", lambda: _narrow_graph(rnd)), ("poseidon", lambda: util.poseidon_like_graph(rnd, 3, 8))):
+            nodes, wit, imap = gen()
+            out.append((f"{name}_{k}", nodes, wit, imap, [util.matrix_row(rnd, 6) for _ in range(6)]))
+    return out
+
+
+_PLAN_ONLY = {}
+for _name, _env in util.PLAN_VARIANTS:           # the variants that change the compiled program (the others are launch options)
+    _PLAN_ONLY.setdefault(tuple(sorted(util.sim_options(_env).items())), _name)
+
+
+@pytest.mark.parametrize("variant", sorted(_PLAN_ONLY.values()))
+def test_plan_matrix_corpus(variant):
+    """every corpus graph under every plan option of the matrix, on the simulator, against the C oracle; and the corpus
+    reaches what it is there for (util.assert_plan_coverage)"""
+    from oracle import cref
+    env = dict(util.PLAN_VARIANTS)[variant]
+    opts = util.sim_options(env)
+    cov = None
+    for name, nodes, wit, imap, rows in matrix_corpus():
+        data = po.serialize_graph(nodes, wit, imap)
+        g = util.SimGraph(data, **opts)
+        want = cref.CGraph(data).evaluate_batch(np.frombuffer(b"".join(util.pack_u256(r) for r in rows), dtype=np.uint8).reshape(len(rows), -1, 32), 4)
+        for b, r in enumerate(rows):
+            assert g.eval(r)[0] == util.unpack_u256(want[b].tobytes()), (name, b)
+        c = util.plan_coverage(g.code())
+        cov = c if cov is None else util.merge_coverage(cov, c)
+    util.assert_plan_coverage(cov, util.VARIANT_FEATURES.get(variant, ()))

@@ -238,6 +238,8 @@ def sim_lib():
         L.sim_load2.restype = ctypes.c_void_p
         L.sim_load2.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint32, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]
         L.sim_free.argtypes = [ctypes.c_void_p]
+        L.sim_code.restype = ctypes.c_size_t
+        L.sim_code.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint32), ctypes.c_size_t]
         L.sim_info.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint64)]
         L.sim_info2.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint64)]
         L.sim_eval.restype = ctypes.c_int64
@@ -297,10 +299,12 @@ class BitSimGraph:
 class SimGraph:
     """ctypes wrapper over tests/csrc/plan_host_sim.cpp"""
 
-    def __init__(self, data: bytes, n_regs=24, fuse=True, div_batch=0, narrow=True, pow5=True):
+    def __init__(self, data: bytes, n_regs=24, fuse=True, div_batch=0, narrow=True, pow5=True, max_terms=0):
         self.L = sim_lib()
         err = ctypes.create_string_buffer(512)
-        self.h = self.L.sim_load2(data, len(data), n_regs, int(bool(fuse)) | (0 if narrow else 2) | (0 if pow5 else 4) | (int(div_batch) << 8), err, 512)
+        assert 0 <= div_batch <= 0xFF and 0 <= max_terms <= 0xFF
+        flags = int(bool(fuse)) | (0 if narrow else 2) | (0 if pow5 else 4) | (int(div_batch) << 8) | (int(max_terms) << 16)
+        self.h = self.L.sim_load2(data, len(data), n_regs, flags, err, 512)
         if not self.h:
             raise ValueError(err.value.decode())
         info = (ctypes.c_uint64 * 19)()
@@ -337,6 +341,13 @@ class SimGraph:
             keys[6], keys[8] = "n_rows", "n_waits"
         return unpack_u256(out.raw), dict(zip(keys, [int(x) for x in o8]))
 
+    def code(self) -> np.ndarray:
+        """the compiled program: uint32 [n_slots, 4] (isa.h: x, y, z, w of each 16-byte slot)"""
+        n = self.L.sim_code(self.h, None, 0)
+        out = np.zeros((n, 4), dtype=np.uint32)
+        self.L.sim_code(self.h, out.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), n)
+        return out
+
     def inputs_from_json(self, js: str):
         buf = ctypes.create_string_buffer(32 * self.info["I"])
         err = ctypes.create_string_buffer(512)
@@ -355,3 +366,263 @@ class SimGraph:
         if getattr(self, "h", None):
             self.L.sim_free(self.h)
             self.h = None
+
+
+# ---- plan options, program coverage and corpora of the throughput interpreter ------------------------------------------
+# The options the product reads when a graph is loaded (engine.cu: Engine::init_plan) or launched (GW_HOT_CONSTS,
+# GW_THREADS).  "half" in GW_HOT_CONSTS stands for half of the graph's constant table.
+PLAN_VARIANTS = [
+    ("defaults", {}),
+    ("div_batch_1", {"GW_DIV_BATCH": "1"}), ("div_batch_2", {"GW_DIV_BATCH": "2"}),
+    ("div_batch_3", {"GW_DIV_BATCH": "3"}), ("div_batch_16", {"GW_DIV_BATCH": "16"}),
+    ("no_dot", {"GW_FUSE_DOT": "0"}),
+    ("max_terms_2", {"GW_MAX_TERMS": "2", "GW_REGS": "24"}), ("max_terms_16", {"GW_MAX_TERMS": "16", "GW_REGS": "24"}),
+    ("no_narrow", {"GW_NARROW": "0"}), ("no_pow5", {"GW_FUSE_POW5": "0"}),
+    ("regs_4", {"GW_REGS": "4"}), ("regs_5", {"GW_REGS": "5"}), ("regs_40", {"GW_REGS": "40"}),
+    ("hot_0", {"GW_HOT_CONSTS": "0"}), ("hot_1", {"GW_HOT_CONSTS": "1"}), ("hot_half", {"GW_HOT_CONSTS": "half"}),
+    ("threads_32", {"GW_THREADS": "32"}), ("threads_96", {"GW_THREADS": "96"}),
+]
+
+
+def sim_options(env: dict) -> dict:
+    """SimGraph keyword arguments that compile the program the product compiles under `env` (PlanOptions defaults)"""
+    return dict(n_regs=int(env.get("GW_REGS", 12)), fuse=env.get("GW_FUSE_DOT", "1") != "0", div_batch=int(env.get("GW_DIV_BATCH", 0)),
+                narrow=env.get("GW_NARROW", "1") != "0", pow5=env.get("GW_FUSE_POW5", "1") != "0", max_terms=int(env.get("GW_MAX_TERMS", 0)))
+
+
+# A constant at this table index or above is read with __ldg at every launch shape on a GPU with 227 KB of shared memory
+# per block: the hot prefix is what the smallest CTA (32 threads: one 1 KB instruction ring, 4 registers of 1 KB) leaves.
+COLD_CONST = (227 * 1024 - 1024 - 4 * 1024) // 32
+
+_OP_DOT, _OP_SHRAND, _OP_SPILL_ST, _OP_SPILL_LD, _OP_INV, _OP_NZ1, _OP_POW5 = 53, 54, 49, 50, 36, 37, 55
+_F_A, _F_B, _F_C, _F_NARROW = 1 << 8, 1 << 9, 1 << 10, 1 << 12
+
+
+def plan_coverage(code: np.ndarray) -> dict:
+    """What a compiled program (SimGraph.code()) makes eval_batch_kernel do:
+    dot_cross   {(terms, header offset in its 32-slot block)} of the OP_DOTs whose slots reach the next block
+    narrow_spill_st / narrow_spill_ld   narrow (8-byte) spill moves
+    inv_groups  {number of OP_NZ1 in front of each OP_INV}: the sizes of the batched Div groups
+    pow5        OP_POW5 instructions
+    max_const_wide / max_const_narrow   the highest constant-table index read by a wide / a narrow instruction"""
+    cov = dict(dot_cross=set(), narrow_spill_st=0, narrow_spill_ld=0, inv_groups=set(), pow5=0, max_const_wide=-1, max_const_narrow=-1)
+    pc, nz = 0, 0
+    n = len(code)
+    while pc < n:
+        x, y, z, w = (int(v) for v in code[pc])
+        op, narrow = x & 0xFF, bool(x & _F_NARROW)
+        length = 1 + (((y & 0xFF) + 1) >> 1) if op == _OP_DOT else 1
+        consts = []
+        if op == _OP_DOT:
+            nt = y & 0xFF
+            if pc % 32 + length >= 32:
+                cov["dot_cross"].add((nt, pc % 32))
+            for t in range(nt):
+                sl = code[pc + 1 + (t >> 1)]
+                lo, ci = (int(sl[2]), int(sl[3])) if t & 1 else (int(sl[0]), int(sl[1]))
+                if lo & 0xF in (0, 3):
+                    consts.append(ci)
+        elif op == _OP_SHRAND:
+            consts.append(z >> 8)
+        elif op not in (_OP_POW5, _OP_SPILL_ST, _OP_SPILL_LD):
+            consts += [v for f, v in ((_F_A, y), (_F_B, z), (_F_C, w)) if x & f]
+        if consts:
+            key = "max_const_narrow" if narrow else "max_const_wide"
+            cov[key] = max(cov[key], *consts)
+        if narrow and op == _OP_SPILL_ST:
+            cov["narrow_spill_st"] += 1
+        if narrow and op == _OP_SPILL_LD:
+            cov["narrow_spill_ld"] += 1
+        if op == _OP_NZ1:
+            nz += 1
+        if op == _OP_INV:
+            cov["inv_groups"].add(nz)
+            nz = 0
+        cov["pow5"] += op == _OP_POW5
+        pc += length
+    return cov
+
+
+def merge_coverage(a: dict, b: dict) -> dict:
+    out = {}
+    for k, v in a.items():
+        out[k] = v | b[k] if isinstance(v, set) else max(v, b[k]) if k.startswith("max_") else v + b[k]
+    return out
+
+
+COVERAGE_FEATURES = ("dot_cross", "narrow_spill", "inv_16", "pow5", "cold_consts")
+
+
+def assert_plan_coverage(cov: dict, features=COVERAGE_FEATURES):
+    """the device paths the corpora below exist to reach (tests/test_gpu_plan_matrix.py), by feature:
+    dot_cross    an OP_DOT of every term count 9..16 crossing a ring block from every offset it can cross from
+    narrow_spill narrow spill stores and loads
+    inv_16       a batched inversion of 16 Div nodes (OP_NZ1 x 16, OP_INV)
+    pow5         OP_POW5
+    cold_consts  wide and narrow reads of constants outside every shared-memory prefix"""
+    if "dot_cross" in features:
+        for nt in range(9, 17):
+            length = 1 + ((nt + 1) >> 1)
+            missing = set(range(32 - length, 32)) - {o for t, o in cov["dot_cross"] if t == nt}
+            assert not missing, f"no OP_DOT of {nt} terms crossing a ring block from offsets {sorted(missing)}"
+    if "narrow_spill" in features:
+        assert cov["narrow_spill_st"] > 0 and cov["narrow_spill_ld"] > 0, "no narrow spill moves"
+    if "inv_16" in features:
+        assert 16 in cov["inv_groups"], f"no batched inversion of 16 Div nodes: {sorted(cov['inv_groups'])}"
+    if "pow5" in features:
+        assert cov["pow5"] > 0, "no OP_POW5"
+    if "cold_consts" in features:
+        assert min(cov["max_const_wide"], cov["max_const_narrow"]) >= COLD_CONST, "no constant outside every hot prefix"
+
+
+# what each plan variant of PLAN_VARIANTS must reach on the corpus of test_plan_sim.matrix_corpus
+VARIANT_FEATURES = {"defaults": ("pow5", "cold_consts"), "div_batch_16": ("inv_16",), "max_terms_16": ("dot_cross", "pow5", "cold_consts"),
+                    "regs_4": ("narrow_spill", "cold_consts"), "regs_5": ("narrow_spill",), "hot_0": ("cold_consts",)}
+
+
+def dot_ladder_graph(t: int, n_blocks=34):
+    """Linear combinations of exactly t terms (OP_DOT under GW_MAX_TERMS >= t), each preceded by a run of cheap witness-output
+    instructions.  A block (run + OP_DOT) is 33 slots mod 32, so the OP_DOT headers of consecutive blocks sit at consecutive
+    offsets of the 32-slot ring blocks: every offset, crossing included.  Terms are Mul(x, c) at their worst (x = M - 1 in the
+    worst-case rows, c = M - 1 or the constant whose Montgomery form is M - 1: the largest products), mixed with +-x plain
+    terms and constant terms within the compiler's bound on the reduced sum."""
+    r_inv = pow(1 << 256, -1, M)
+    cmax = (M - 1) * r_inv % M                 # prescale(cmax) = M - 1; prescale(M - cmax, subtracted) = M - 1
+    rnd = random.Random(31337 + t)
+    nodes = [(po.K_INPUT, i) for i in range(7)]
+
+    def add(node):
+        nodes.append(node)
+        return len(nodes) - 1
+    wit = [0]
+    length = 1 + ((t + 1) >> 1)
+    run = (33 - length) % 32
+    for k in range(n_blocks):
+        for i in range(run if k else max(run, 6)):          # the first run reads every input (their loads come first)
+            wit.append(add((po.K_DUO, po.DUO["Add" if i % 2 else "Sub"], 1 + i % 6, 1 + (i + 1) % 6)))
+        q = k % 3 if t >= 3 else 0                          # plain terms, within the bound of plan.cpp: dot_bound
+        while q and 1 + 0.18906 * (t - q) + q > 5.2:
+            q -= 1
+        n_const = 1 if k % 4 == 3 and t - q >= 2 else 0
+        lc = None
+        for j in range(t):
+            sub = j % 2 == 1
+            if j < t - q - n_const:
+                mode = k % 4
+                c = {0: M - 1, 1: (M - cmax) if sub else cmax, 2: cmax if j % 3 else M - 1}.get(mode, random_value(rnd))
+                cn, x = add((po.K_CONST, c)), 1 + j % 3
+                term = add((po.K_DUO, po.DUO["Mul"], x, cn) if j % 2 == 0 else (po.K_DUO, po.DUO["Mul"], cn, x))
+            elif j < t - n_const:
+                term = 4 + j % 3
+            else:
+                term = add((po.K_CONST, random_value(rnd)))
+            lc = term if lc is None else add((po.K_DUO, po.DUO["Sub" if sub else "Add"], lc, term))
+        wit.append(lc)
+    return nodes, wit, {"x": (1, 6)}
+
+
+def div_group_graph(k: int):
+    """k independent Div nodes of one division level: numerators are inputs 1..k, denominators inputs k+1..2k"""
+    nodes = [(po.K_INPUT, i) for i in range(2 * k + 1)]
+    for j in range(k):
+        nodes.append((po.K_DUO, po.DUO["Div"], 1 + j, 1 + k + j))
+    return nodes, list(range(len(nodes))), {"x": (1, 2 * k)}
+
+
+def div_group_rows(k: int, rnd: random.Random) -> list:
+    """every pattern of zero denominators for k <= 4; first only, last only, all and none above.  A zero is 0, M or 2 M
+    in turn (the raw values reduce to 0)"""
+    pats = list(range(1 << k)) if k <= 4 else [1, 1 << (k - 1), (1 << k) - 1, 0]
+    zeros = [0, M, 2 * M]
+    rows = []
+    for p in pats:
+        for rep in range(2):
+            num = [random_value(rnd) if rep else M - 1 for _ in range(k)]
+            den = [zeros[(j + rep) % 3] if (p >> j) & 1 else (random_value(rnd) or 1) if rep else M - 1 - j for j in range(k)]
+            rows.append([1] + num + den)
+    return rows
+
+
+def narrow_limit_graphs():
+    """the shapes of test_plan_sim.test_narrow_range_limits: sums, products and negations at the +-2^62 edge of the narrow
+    domain.  Returns [(bits, nodes, witness, input map)]"""
+    D = po.DUO
+    out = []
+    for bits in (30, 31, 32, 40, 61, 62):
+        mask = (1 << bits) - 1
+        nodes = [(po.K_INPUT, 0), (po.K_INPUT, 1), (po.K_INPUT, 2), (po.K_CONST, mask), (po.K_CONST, 0), (po.K_CONST, 1)]
+        nodes += [(po.K_DUO, D["Band"], 1, 3), (po.K_DUO, D["Band"], 2, 3)]
+        a, b = 6, 7
+        nodes += [(po.K_DUO, D["Mul"], a, b), (po.K_DUO, D["Sub"], 4, a), (po.K_DUO, D["Sub"], b, a), (po.K_DUO, D["Mul"], 9, b),
+                  (po.K_DUO, D["Add"], a, b), (po.K_DUO, D["Add"], 12, 12), (po.K_DUO, D["Mul"], 10, 10), (po.K_UNO, 0, 8),
+                  (po.K_DUO, D["Lt"], 9, 10), (po.K_DUO, D["Geq"], 10, 4), (po.K_TRES, 0, 10, 9, 13), (po.K_DUO, D["Sub"], 18, 5)]
+        out.append((bits, nodes, list(range(len(nodes))), {"x": (1, 2)}))
+    return out
+
+
+def narrow_limit_values(bits: int) -> list:
+    mask = (1 << bits) - 1
+    return [mask, mask + 1, (1 << 62) - 1, 1 << 62, M - (1 << 62), M - 1, (1 << 256) - 1, 0, 1]
+
+
+def const_heavy_graph(rnd: random.Random, n_wide=6400, n_narrow=1600, chain=64):
+    """Several thousand distinct constants, each read once, so that the constant table is longer than any shared-memory
+    prefix (COLD_CONST): long sums of Mul(x, c) (wide OP_DOT terms, or OP_MUL with a constant operand without fusion) and
+    narrow chains over 16-bit slices of the inputs with constant addends, factors and comparisons (8-byte reads)."""
+    D = po.DUO
+    nodes = [(po.K_INPUT, i) for i in range(7)]
+
+    def add(node):
+        nodes.append(node)
+        return len(nodes) - 1
+    mask = add((po.K_CONST, 0xFFFF))
+    seen = set()
+
+    def fresh(lo, hi):
+        while True:
+            v = rnd.randrange(lo, hi)
+            if v not in seen:
+                seen.add(v)
+                return add((po.K_CONST, v))
+    sl = [add((po.K_DUO, D["Band"], 1 + i, mask)) for i in range(6)]
+    wit = [0]
+    lc = acc = None
+    every = max(1, n_wide // n_narrow)
+    for j in range(n_wide):                              # the two kinds interleave over the whole table
+        term = add((po.K_DUO, D["Mul"], 1 + j % 6, fresh(1 << 64, M)))
+        lc = term if lc is None else add((po.K_DUO, D["Add" if j % 5 else "Sub"], lc, term))
+        if (j + 1) % chain == 0:
+            wit.append(lc)
+            lc = None
+        if j % every:
+            continue
+        i = j // every
+        s = sl[i % 6]
+        kind = i % 4
+        if kind == 0:
+            term = add((po.K_DUO, D["Add"], s, fresh(2, 1 << 40)))
+        elif kind == 1:
+            term = add((po.K_DUO, D["Mul"], s, fresh(2, 1 << 20)))
+        elif kind == 2:
+            term = add((po.K_DUO, D["Lt"], s, fresh(2, 1 << 17)))
+        else:
+            term = add((po.K_DUO, D["Sub"], fresh(2, 1 << 40), s))
+        acc = term if acc is None else add((po.K_DUO, D["Add"], acc, term))
+        if (i + 1) % chain == 0:
+            wit.append(acc)
+            acc = None
+    return nodes, wit, {"x": (1, 6)}
+
+
+def matrix_row(rnd: random.Random, n_in: int) -> list:
+    """one input row of the matrix tests: field values, raw 256-bit values >= M, edge values, neighbours of +-2^62"""
+    def one():
+        r = rnd.random()
+        if r < 0.45:
+            return random_value(rnd)
+        if r < 0.6:
+            return rnd.randrange(M, 1 << 256)
+        if r < 0.8:
+            return rnd.choice(EDGE)
+        return rnd.choice([(1 << 62) + d for d in (-2, -1, 0, 1)] + [M - (1 << 62) + d for d in (-1, 0, 1, 2)])
+    return [1] + [one() for _ in range(n_in)]
