@@ -16,7 +16,14 @@
 
 using namespace gw;
 
-struct SimGraph { Graph g; Plan plan; std::string err; };
+static bool lat_is_slow_op(uint32_t op) { return op == OP_DIV || op == OP_INV || op == OP_POW || op == OP_IDIV || op == OP_MOD; }
+static bool op_has_b_host(uint32_t op) { return op < 32 || op == OP_TERN || op == OP_MULADD; }
+
+struct SimGraph {
+  Graph g; Plan plan; std::string err;
+  // the latency plan of the last sim_eval_latency3 call and the options it was compiled under (one compilation per option set)
+  std::vector<uint32_t> lat_key; LatencyPlan lat; bool lat_ok = false;
+};
 
 static fe to_fe(const U256& v) { fe r; memcpy(r.l, v.l, 32); return r; }
 
@@ -191,15 +198,83 @@ void sim_wtns_header(uint32_t n, uint8_t* dst) { wtns_write_header(dst, n); }
 // hazards.  The slow warps are asynchronous on the device; the simulator runs each job at one of the two extremes
 // the protocol allows -- mode 0: as soon as its issue level starts, mode 1: just before the OP_WAIT that guards its
 // readers -- so a slot recycled too early (or a reader scheduled before the wait) shows up as a wrong witness.
-// opts: {n_warps, n_slow_warps, slow_levels, split_dot, fuse, packet_slots} (0 = default except for the two flags)
-// out8: n_levels, n_slots, n_instrs, max level width, status, est_cycles, n_split, slow_levels
-int64_t sim_eval_latency2(SimGraph* s, const uint8_t* inputs, uint8_t* witness, uint64_t* out8, int mode, const uint32_t* opts) {
-  LatencyPlan lp;
-  try {
-    LatencyOptions o;
-    if (opts) { if (opts[0]) o.n_warps = opts[0]; if (opts[1]) o.n_slow_warps = opts[1]; o.slow_levels = opts[2]; o.split_dot = opts[3] != 0; o.fuse = opts[4] != 0; if (opts[5]) o.packet_slots = opts[5]; o.chain = opts[6] != 0; o.dataflow = opts[7] != 0; o.sbox_links = opts[8] != 0; o.force_sbox_links = opts[8] == 2; }
-    lp = compile_latency_plan(s->g, o);
-  } catch (const std::exception& e) { s->err = e.what(); return -2; }
+// opts (11 words): {n_warps, n_slow_warps, slow_levels, split_dot, fuse, packet_slots, chain, dataflow, sbox_links (2 = forced),
+// exclusive_warp0, max_slots} (0 = default for the counts and sizes)
+// out10: n_levels, n_slots, n_instrs, max level width, status, est_cycles, n_split | n_rows, slow_levels, n_chained | n_waits, n_sbox_links
+// cov (LAT_COV_WORDS words or null): what the kernel would execute, accumulated over calls (LatCov below)
+enum LatCov {
+  COV_DOT_SHAPES,     // mask of the straight-line OP_DOT shapes executed (bit = ins.y >> 16)
+  COV_DOT_TERMS,      // largest term count of a generic-loop OP_DOT
+  COV_DOT_KINDS,      // mask of the term kinds of generic-loop OP_DOTs (bit = T_*)
+  COV_SLOW_WIDTHS,    // mask of the lanes of slow-warp jobs (bit = headers of the job, 1..32)
+  COV_SLOW_OPS,       // mask of the opcodes of slow-warp jobs
+  COV_SLOW_CONST,     // slow-warp instructions that read a constant operand
+  COV_POW5, COV_POW4, COV_MULADD, COV_SHRAND, COV_OUT, COV_TERN_CONST, COV_MULADD_CONST,
+  COV_CHAIN,          // largest number of headers per lane in one packet
+  COV_LEVELS_MOD3,    // mask of n_levels mod 3
+  COV_LEVELS_SMALL,   // mask of n_levels below 64
+  COV_EMPTY_PACKET,   // level plan: packets of a main warp without headers
+  COV_CHUNK_FULL,     // dataflow plan: chunks filled to their last slot
+  COV_CHUNK_ZERO,     // dataflow plan: chunks ended by a zero descriptor
+  COV_WAIT_WIDTH,     // dataflow plan: largest number of nonzero entries of a wait vector
+  COV_PHYS_WARPS,     // dataflow plan: n_phys_warps
+  COV_N_SLOTS, COV_MAX_SLOTS,
+  COV_DOT_SHAPES_M1,  // mask of the straight-line OP_DOT shapes executed with a first-product constant of M - 1 (worst case)
+  LAT_COV_WORDS
+};
+int64_t sim_eval_latency3(SimGraph* s, const uint8_t* inputs, uint8_t* witness, uint64_t* out8, int mode, const uint32_t* opts, uint64_t* cov) {
+  const std::vector<uint32_t> key(opts, opts + 11);
+  if (!s->lat_ok || s->lat_key != key) {
+    s->lat_ok = false;
+    try {
+      LatencyOptions o;
+      if (opts[0]) o.n_warps = opts[0]; if (opts[1]) o.n_slow_warps = opts[1]; o.slow_levels = opts[2]; o.split_dot = opts[3] != 0; o.fuse = opts[4] != 0; if (opts[5]) o.packet_slots = opts[5]; o.chain = opts[6] != 0; o.dataflow = opts[7] != 0; o.sbox_links = opts[8] != 0; o.force_sbox_links = opts[8] == 2;
+      o.exclusive_warp0 = opts[9] != 0; if (opts[10]) o.max_slots = opts[10];
+      s->lat = compile_latency_plan(s->g, o);
+      s->lat_key = key; s->lat_ok = true;
+    } catch (const std::exception& e) { s->err = e.what(); return -2; }
+  }
+  const LatencyPlan& lp = s->lat;
+  uint64_t dummy[LAT_COV_WORDS] = {};
+  uint64_t* cv = cov ? cov : dummy;
+  cv[COV_LEVELS_MOD3] |= 1ull << (lp.n_levels % 3);
+  if (lp.n_levels < 64) cv[COV_LEVELS_SMALL] |= 1ull << lp.n_levels;
+  cv[COV_N_SLOTS] = std::max<uint64_t>(cv[COV_N_SLOTS], lp.n_slots);
+  cv[COV_MAX_SLOTS] = opts[10] ? opts[10] : LatencyOptions().max_slots;
+  if (lp.dataflow) cv[COV_PHYS_WARPS] = std::max<uint64_t>(cv[COV_PHYS_WARPS], lp.n_phys_warps);
+  // what one header makes the kernel do (lat_exec; lat_exec_slow for the jobs of the slow warps)
+  auto cover = [&](size_t pk, const Instr& ins, bool slow) {
+    const uint32_t op = ins.x & 0xFF;
+    const bool any_const = (ins.x & F_A_CONST) || ((ins.x & F_B_CONST) && op_has_b_host(op)) || ((ins.x & F_C_CONST) && (op == OP_TERN || op == OP_MULADD));
+    if (op == OP_NOP) return;
+    if (slow) { cv[COV_SLOW_OPS] |= 1ull << op; cv[COV_SLOW_CONST] += any_const; }
+    if (op == OP_DOT) {
+      const uint32_t nt = ins.y & 0xFF, shape = ins.y >> 16;
+      if (shape & 1) {
+        cv[COV_DOT_SHAPES] |= 1ull << shape;
+        const fe m1 = fe_neg(fe_small(1));
+        const size_t ci = pk + ins.z < lp.code.size() ? pk + lp.code[pk + ins.z].y : lp.code.size();
+        if (ci + 1 < lp.code.size()) {
+          const Instr& a = lp.code[ci]; const Instr& b = lp.code[ci + 1];
+          const uint32_t v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+          if (!memcmp(v, m1.l, 32)) cv[COV_DOT_SHAPES_M1] |= 1ull << shape;
+        }
+      } else {
+        cv[COV_DOT_TERMS] = std::max<uint64_t>(cv[COV_DOT_TERMS], nt);
+        for (uint32_t t = 0; t < nt && pk + ins.z + (t >> 1) < lp.code.size(); t++) {
+          const Instr& sl = lp.code[pk + ins.z + (t >> 1)];
+          cv[COV_DOT_KINDS] |= 1ull << (((t & 1) ? sl.z : sl.x) & 0xF);
+        }
+      }
+    }
+    cv[COV_POW5] += op == OP_POW5; cv[COV_POW4] += op == OP_POW4; cv[COV_MULADD] += op == OP_MULADD; cv[COV_SHRAND] += op == OP_SHRAND;
+    cv[COV_OUT] += op == OP_OUT; cv[COV_TERN_CONST] += op == OP_TERN && any_const; cv[COV_MULADD_CONST] += op == OP_MULADD && any_const;
+  };
+  auto cover_packet = [&](size_t pk, uint32_t nh, uint32_t lanes, bool slow) {
+    if (lanes) cv[COV_CHAIN] = std::max<uint64_t>(cv[COV_CHAIN], (nh + lanes - 1) / lanes);
+    if (slow) cv[COV_SLOW_WIDTHS] |= 1ull << nh;
+    for (uint32_t k = 0; k < nh && pk + 1 + k < lp.code.size(); k++) cover(pk, lp.code[pk + 1 + k], slow);
+  };
   std::vector<fe> slots(lp.n_slots, fe_zero());
   uint32_t st = 0;
   struct W { uint32_t dst; fe v; };
@@ -278,6 +353,7 @@ int64_t sim_eval_latency2(SimGraph* s, const uint8_t* inputs, uint8_t* witness, 
       while (chunk[w] < lp.stream_chunks[w]) {
         const size_t base = (size_t)lp.stream_off[w] + (size_t)chunk[w] * C;
         if (off[w] < C && lp.code[base + off[w]].x != 0) { *pk = base + off[w]; return true; }
+        if (off[w] >= C) cv[COV_CHUNK_FULL]++; else cv[COV_CHUNK_ZERO]++;
         chunk[w]++; off[w] = 0;
       }
       return false;
@@ -305,6 +381,12 @@ int64_t sim_eval_latency2(SimGraph* s, const uint8_t* inputs, uint8_t* witness, 
       const Instr d = lp.code[pk];
       const uint32_t nh = d.y & 0xFFFFu, lanes = d.y >> 16;
       if (d.x > C - off[w] || nh + 1 > d.x || lanes > 32 || (nh && !lanes) || d.w != progress[w] + 1) return -1;
+      if (d.z) {
+        uint64_t nz = 0;
+        for (uint32_t x = 0; x < NW; x++) { const Instr& sl = lp.code[pk + d.z + x / 4]; nz += ((x & 3) == 0 ? sl.x : (x & 3) == 1 ? sl.y : (x & 3) == 2 ? sl.z : sl.w) != 0; }
+        cv[COV_WAIT_WIDTH] = std::max(cv[COV_WAIT_WIDTH], nz);
+      }
+      cover_packet(pk, nh, lanes, nh && lat_is_slow_op(lp.code[pk + 1].x & 0xFF));
       std::vector<W> writes;
       for (uint32_t lane = 0; lane < lanes; lane++) {
         overlay.clear();
@@ -322,6 +404,8 @@ int64_t sim_eval_latency2(SimGraph* s, const uint8_t* inputs, uint8_t* witness, 
   std::vector<uint32_t> next_job(lp.n_slow_warps, 0);
   auto run_job = [&](uint32_t w, uint32_t j) {
     const uint32_t* e = &lp.jobs[((size_t)w * lp.max_jobs + j) * 4];
+    if ((size_t)e[1] + e[2] >= lp.code.size()) return false;
+    cover_packet(e[1], e[2], e[2], true);
     std::vector<W> writes;
     for (uint32_t k = 0; k < e[2]; k++) { overlay.clear(); if ((size_t)e[1] + 1 + k >= lp.code.size() || !exec(e[1], lp.code[e[1] + 1 + k], writes)) return false; }
     overlay.clear();
@@ -354,6 +438,8 @@ int64_t sim_eval_latency2(SimGraph* s, const uint8_t* inputs, uint8_t* witness, 
     for (uint32_t w = 0; w < lp.n_warps; w++) {
       const size_t pk = cur[w * 4];
       const uint32_t nh = cur[w * 4 + 2], lanes = cur[w * 4 + 3];
+      if (nh == 0) cv[COV_EMPTY_PACKET]++;
+      cover_packet(pk, nh, lanes, false);
       for (uint32_t lane = 0; lane < lanes; lane++) {
         overlay.clear();
         for (uint32_t k = lane; k < nh; k += lanes) { if (!exec(pk, lp.code[pk + 1 + k], writes)) return -1; n_headers++; }
@@ -372,6 +458,12 @@ int64_t sim_eval_latency2(SimGraph* s, const uint8_t* inputs, uint8_t* witness, 
   out8[5] = lp.est_cycles; out8[6] = lp.n_split; out8[7] = lp.slow_levels; out8[8] = lp.n_chained; out8[9] = lp.n_sbox_links;
   return 0;
 }
+int64_t sim_eval_latency2(SimGraph* s, const uint8_t* inputs, uint8_t* witness, uint64_t* out8, int mode, const uint32_t* opts) {
+  uint32_t o[11] = {0, 0, 0, 1, 1, 0, 1, 0, 1, 0, 0};
+  if (opts) for (int k = 0; k < 9; k++) o[k] = opts[k];
+  return sim_eval_latency3(s, inputs, witness, out8, mode, o, nullptr);
+}
+const char* sim_error(SimGraph* s) { return s->err.c_str(); }
 int64_t sim_eval_latency(SimGraph* s, const uint8_t* inputs, uint8_t* witness, uint64_t* out5) {
   uint64_t o8[10];
   int64_t rc = sim_eval_latency2(s, inputs, witness, o8, 0, nullptr);

@@ -148,3 +148,33 @@ def test_sbox_link_rewrite_on_poseidon_graphs():
     assert got == want and info["n_sbox_links"] > 4000
     got, info = g.eval_latency(buf, mode=2, dataflow=True)
     assert got == want and info["n_sbox_links"] == 0
+
+
+@pytest.mark.parametrize("variant", [name for name, _ in util.LATENCY_VARIANTS])
+def test_latency_matrix_corpus(variant):
+    """every graph of the latency corpus (util.latency_corpus) under one option of the latency matrix, on the simulator:
+    every value against the C oracle, the status against the throughput plan's, the slow-warp jobs or the warp interleaving
+    at both extremes (and one pseudo-random interleaving of the dataflow plan); and the corpus reaches what it is there for
+    (util.assert_latency_coverage).  A graph whose live values do not fit the value file must be refused as too wide."""
+    import numpy as np
+    from oracle import cref
+    opts = util.latency_sim_options(dict(util.LATENCY_VARIANTS)[variant])
+    modes = (0, 1, 17) if opts["dataflow"] else (0, 1)
+    cov = None
+    for name, nodes, wit, imap, rows in util.latency_corpus():
+        data = po.serialize_graph(nodes, wit, imap)
+        g = util.SimGraph(data, **util.sim_options({}))
+        want = cref.CGraph(data).evaluate_batch(np.frombuffer(b"".join(util.pack_u256(r) for r in rows), dtype=np.uint8).reshape(len(rows), -1, 32), 4)
+        util.assert_rows_expose_stores(name, want)
+        for b, r in enumerate(rows):
+            status = g.eval(r)[1]
+            for mode in modes:
+                try:
+                    got, info, c = g.eval_latency(r, mode=mode, coverage=True, **opts)
+                except ValueError as e:
+                    assert "too wide" in str(e) and name == "const_heavy" and not opts["fuse"], (name, str(e))
+                    break
+                assert got == util.unpack_u256(want[b].tobytes()), (name, b, mode)
+                assert info["status"] == status, (name, b, mode)
+                cov = c if cov is None else util.merge_coverage(cov, c)
+    util.assert_latency_coverage(cov, util.LATENCY_VARIANT_FEATURES[variant])

@@ -249,6 +249,11 @@ def sim_lib():
         L.sim_eval_latency2.restype = ctypes.c_int64
         L.sim_eval_latency2.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.POINTER(ctypes.c_uint64), ctypes.c_int,
                                         ctypes.POINTER(ctypes.c_uint32)]
+        L.sim_eval_latency3.restype = ctypes.c_int64
+        L.sim_eval_latency3.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.POINTER(ctypes.c_uint64), ctypes.c_int,
+                                        ctypes.POINTER(ctypes.c_uint32), ctypes.POINTER(ctypes.c_uint64)]
+        L.sim_error.restype = ctypes.c_char_p
+        L.sim_error.argtypes = [ctypes.c_void_p]
         L.sim_inputs.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_size_t]
         L.sim_reserialize.restype = ctypes.c_size_t
         L.sim_reserialize.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_size_t]
@@ -326,20 +331,27 @@ class SimGraph:
         return unpack_u256(out.raw), int(st)
 
     def eval_latency(self, inputs, mode=0, n_warps=0, n_slow_warps=0, slow_levels=0, split_dot=True, fuse=True, packet_slots=0, chain=True,
-                     dataflow=False, sbox_links=True):
+                     dataflow=False, sbox_links=True, exclusive_warp0=False, max_slots=0, coverage=False):
         """latency-mode plan on the host simulator -> (witness list, info dict).  Level plan: mode 0 / 1 = the slow-warp
         jobs run as early / as late as the protocol allows.  dataflow=True: per-warp packet streams with wait vectors;
         mode 0 / 1 / >= 2 = the next runnable warp is the lowest / the highest / a pseudo-random one
-        (tests/csrc/plan_host_sim.cpp)."""
+        (tests/csrc/plan_host_sim.cpp).  max_slots = 0: the LatencyOptions default.  A plan that does not compile raises
+        ValueError with the compiler's message.  coverage=True returns (witness, info, coverage) with the coverage of
+        this call (latency_coverage)."""
         out = ctypes.create_string_buffer(32 * self.info["W"])
         o8 = (ctypes.c_uint64 * 10)()
-        opts = (ctypes.c_uint32 * 9)(n_warps, n_slow_warps, slow_levels, int(split_dot), int(fuse), packet_slots, int(chain), int(dataflow), int(sbox_links))
-        rc = self.L.sim_eval_latency2(self.h, pack_u256(inputs), out, o8, mode, opts)
+        opts = (ctypes.c_uint32 * 11)(n_warps, n_slow_warps, slow_levels, int(split_dot), int(fuse), packet_slots, int(chain), int(dataflow),
+                                      int(sbox_links), int(exclusive_warp0), max_slots)
+        cov = (ctypes.c_uint64 * len(LAT_COV_KEYS))()
+        rc = self.L.sim_eval_latency3(self.h, pack_u256(inputs), out, o8, mode, opts, cov)
+        if rc == -2:
+            raise ValueError(self.L.sim_error(self.h).decode())
         assert rc == 0, f"latency plan failed ({rc})"
         keys = ["n_levels", "n_slots", "n_instrs", "max_width", "status", "est_cycles", "n_split", "slow_levels", "n_chained", "n_sbox_links"]
         if dataflow:
             keys[6], keys[8] = "n_rows", "n_waits"
-        return unpack_u256(out.raw), dict(zip(keys, [int(x) for x in o8]))
+        res = (unpack_u256(out.raw), dict(zip(keys, [int(x) for x in o8])))
+        return res + (latency_coverage(list(cov)),) if coverage else res
 
     def code(self) -> np.ndarray:
         """the compiled program: uint32 [n_slots, 4] (isa.h: x, y, z, w of each 16-byte slot)"""
@@ -626,3 +638,302 @@ def matrix_row(rnd: random.Random, n_in: int) -> list:
             return rnd.choice(EDGE)
         return rnd.choice([(1 << 62) + d for d in (-2, -1, 0, 1)] + [M - (1 << 62) + d for d in (-1, 0, 1, 2)])
     return [1] + [one() for _ in range(n_in)]
+
+
+# ---- latency mode: options, coverage and corpus of eval_latency_kernel / eval_dataflow_kernel ---------------------------
+# The options Engine::calc_latency reads when a graph's latency plan is first built (engine.cu: Engine::run_latency).
+# Every variant runs the generic kernels (GW_LAT_BIT=0) with all other latency options at their defaults.
+LATENCY_ENV_KEYS = ("GW_LAT_MODE", "GW_LAT_WARPS", "GW_LAT_SLOW_WARPS", "GW_LAT_EXCL", "GW_LAT_D", "GW_LAT_SPLIT", "GW_LAT_FUSE", "GW_LAT_LINKS",
+                    "GW_LAT_CHAIN", "GW_LAT_BIT", "GW_LAT_WATCHDOG", "GW_LAT_DBG", "GW_LAT_CLOCKS", "GW_SINGLE_MODE")
+_LAT_BOTH = [("defaults", {}), ("serial", {"GW_LAT_WARPS": "1", "GW_LAT_SLOW_WARPS": "1", "GW_LAT_D": "1"}), ("d_2", {"GW_LAT_D": "2"}),
+             ("no_fuse", {"GW_LAT_FUSE": "0"}), ("links_2", {"GW_LAT_LINKS": "2"})]
+LATENCY_VARIANTS = (
+    [("df_" + n, e) for n, e in _LAT_BOTH] + [("level_" + n, dict(e, GW_LAT_MODE="level")) for n, e in _LAT_BOTH]
+    + [("df_warps_12", {"GW_LAT_WARPS": "8", "GW_LAT_SLOW_WARPS": "4"}), ("df_excl", {"GW_LAT_EXCL": "1"}),
+       ("df_excl_w7s3", {"GW_LAT_EXCL": "1", "GW_LAT_WARPS": "7", "GW_LAT_SLOW_WARPS": "3"}),
+       ("df_excl_w8s4", {"GW_LAT_EXCL": "1", "GW_LAT_WARPS": "8", "GW_LAT_SLOW_WARPS": "4"}),
+       ("df_no_chain", {"GW_LAT_CHAIN": "0"}), ("df_no_split", {"GW_LAT_SPLIT": "0"}), ("df_links_0", {"GW_LAT_LINKS": "0"})]
+    + [("level_warps_12", {"GW_LAT_MODE": "level", "GW_LAT_WARPS": "10", "GW_LAT_SLOW_WARPS": "1"}),
+       ("level_d_200", {"GW_LAT_MODE": "level", "GW_LAT_D": "200"}),
+       ("level_no_split_chain", {"GW_LAT_MODE": "level", "GW_LAT_SPLIT": "0", "GW_LAT_CHAIN": "0"})])
+LATENCY_VARIANTS = [(n, dict(e, GW_LAT_BIT="0")) for n, e in LATENCY_VARIANTS]
+
+B200_SMEM_OPTIN = 232448      # cudaDevAttrMaxSharedMemoryPerBlockOptin of a B200
+LAT_RING_SLOTS = 128          # engine.cu: packet ring stage / dataflow chunk (16 B slots)
+LAT_CTRL_BYTES, DF_CTRL_BYTES = 320, 384
+
+
+def latency_sim_options(env: dict, smem_optin=B200_SMEM_OPTIN) -> dict:
+    """SimGraph.eval_latency keyword arguments that compile the latency plan the product compiles under `env` on a device
+    with `smem_optin` bytes of opt-in shared memory per block (engine.cu: Engine::run_latency)"""
+    geti = lambda k, d: int(env[k]) if env.get(k) else d
+    dataflow = env.get("GW_LAT_MODE") != "level"
+    n_warps, n_slow = geti("GW_LAT_WARPS", 6 if dataflow else 7), geti("GW_LAT_SLOW_WARPS", 3 if dataflow else 4)
+    excl = geti("GW_LAT_EXCL", 0) != 0
+    if dataflow:                      # rings of every physical warp, the empty ones the exclusive warp 0 leaves included
+        rings = min(12, n_warps + n_slow + (2 if excl else 0))
+        max_slots = min((smem_optin // 16 - DF_CTRL_BYTES // 16 - rings * 3 * LAT_RING_SLOTS) // 2, 0xFFFF)
+    else:                             # one ring per main warp
+        max_slots = min((smem_optin // 16 - LAT_CTRL_BYTES // 16 - n_warps * 3 * LAT_RING_SLOTS) // 2, 0xFFFF)
+    links = geti("GW_LAT_LINKS", 1)
+    return dict(dataflow=dataflow, n_warps=n_warps, n_slow_warps=n_slow, slow_levels=geti("GW_LAT_D", 0), split_dot=geti("GW_LAT_SPLIT", 1) != 0,
+                fuse=geti("GW_LAT_FUSE", 1) != 0, packet_slots=LAT_RING_SLOTS, chain=geti("GW_LAT_CHAIN", 1) != 0,
+                sbox_links=2 if links == 2 else int(links != 0), exclusive_warp0=excl, max_slots=max_slots)
+
+
+# tests/csrc/plan_host_sim.cpp: enum LatCov.  Masks become sets, "max_" keys are maxima, the others counts (merge_coverage)
+LAT_COV_KEYS = ("dot_shapes", "max_dot_terms", "dot_kinds", "slow_widths", "slow_ops", "slow_const", "pow5", "pow4", "muladd", "shrand", "out",
+                "tern_const", "muladd_const", "max_chain", "levels_mod3", "n_levels", "empty_packet", "chunk_full", "chunk_zero", "max_wait",
+                "max_phys_warps", "max_n_slots", "max_slots", "dot_shapes_m1")
+_LAT_COV_MASKS = ("dot_shapes", "dot_kinds", "slow_widths", "slow_ops", "levels_mod3", "n_levels", "dot_shapes_m1")
+
+
+def latency_coverage(words) -> dict:
+    """the coverage record of the latency simulator as a dict; at_capacity counts plans whose value file is exactly full"""
+    raw = dict(zip(LAT_COV_KEYS, (int(w) for w in words)))
+    cov = {k: ({b for b in range(64) if (v >> b) & 1} if k in _LAT_COV_MASKS else v) for k, v in raw.items() if k != "max_slots"}
+    cov["at_capacity"] = int(raw["max_n_slots"] == raw["max_slots"])
+    return cov
+
+
+_OP_DIV, _OP_POW, _OP_IDIV, _OP_MOD = 1, 4, 5, 6
+DOT_SHAPES = {1 | (n << 1) | (a << 3) | (c << 4) for n in (1, 2) for a in (0, 1) for c in (0, 1)}
+LATENCY_FEATURES = ("dot_shapes", "dot_generic", "slow_jobs", "slow_const", "ops", "sbox", "chains", "levels", "empty_packet", "chunks", "phys_12",
+                    "warps_12")
+
+
+def assert_latency_coverage(cov: dict, features=LATENCY_FEATURES):
+    """the kernel paths the latency corpus exists to reach (tests/test_gpu_latency_matrix.py), by feature:
+    dot_shapes   every straight-line OP_DOT shape: 1-2 products x an added value or not x a constant or not, each of them
+                 with a first-product constant of M - 1 in the packet (the largest product)
+    dot_generic  generic-loop OP_DOTs with all four term kinds, one of 8 terms (the most a latency plan puts in one)
+    slow_jobs    slow-warp jobs of 32 lanes and of fewer, running Div, Idiv, Mod and Pow
+    slow_const   slow-warp instructions with a constant operand
+    ops          OP_POW5, OP_SHRAND, OP_OUT and an OP_TERN with a constant operand
+    sbox         OP_POW4, OP_MULADD and an OP_MULADD with a constant operand (S-box link rewrite)
+    chains       level plan: a lane running two or more headers of one packet
+    levels       plans of 0, 1 and 2 levels mod 3, and of 1 and of 2 levels
+    empty_packet level plan: a main warp without an instruction at some level
+    chunks       dataflow plan: chunks filled to their last slot and chunks ended by a zero descriptor
+    phys_12      dataflow plan: 12 physical warps (a ring and a progress counter each, the empty ones included)
+    warps_12     dataflow plan: 12 physical warps, and a packet that waits for 11 other warps"""
+    if "dot_shapes" in features:
+        missing = DOT_SHAPES - cov["dot_shapes"]
+        assert not missing, f"straight-line OP_DOT shapes never executed: {sorted(missing)}"
+        missing = DOT_SHAPES - cov["dot_shapes_m1"]
+        assert not missing, f"straight-line OP_DOT shapes never executed with a constant of M - 1: {sorted(missing)}"
+    if "dot_generic" in features:
+        assert cov["dot_kinds"] >= {0, 1, 2, 3}, f"generic OP_DOT term kinds executed: {sorted(cov['dot_kinds'])}"
+        assert cov["max_dot_terms"] >= 8, f"no generic OP_DOT of 8 terms: {cov['max_dot_terms']}"
+    if "slow_jobs" in features:
+        assert 32 in cov["slow_widths"] and min(cov["slow_widths"] or {32}) < 32, f"slow-warp job widths: {sorted(cov['slow_widths'])}"
+        missing = {_OP_DIV, _OP_POW, _OP_IDIV, _OP_MOD} - cov["slow_ops"]
+        assert not missing, f"opcodes never run by a slow warp: {sorted(missing)}"
+    if "slow_const" in features:
+        assert cov["slow_const"] > 0, "no slow-warp instruction reads a constant"
+    if "ops" in features:
+        for k in ("pow5", "shrand", "out", "tern_const"):
+            assert cov[k] > 0, f"no {k}"
+    if "sbox" in features:
+        for k in ("pow4", "muladd", "muladd_const"):
+            assert cov[k] > 0, f"no {k}"
+    if "chains" in features:
+        assert cov["max_chain"] >= 2, "no lane chain"
+    if "levels" in features:
+        assert cov["levels_mod3"] == {0, 1, 2}, f"level counts mod 3: {sorted(cov['levels_mod3'])}"
+        assert {1, 2} <= cov["n_levels"], f"no plan of 1 or of 2 levels: {sorted(b for b in cov['n_levels'] if b < 8)}"
+    if "empty_packet" in features:
+        assert cov["empty_packet"] > 0, "no level at which a main warp is idle"
+    if "chunks" in features:
+        assert cov["chunk_full"] > 0, "no chunk filled to its last slot"
+        assert cov["chunk_zero"] > 0, "no chunk ended by a zero descriptor"
+    if "phys_12" in features or "warps_12" in features:
+        assert cov["max_phys_warps"] == 12, f"physical warps: {cov['max_phys_warps']}"
+    if "warps_12" in features:
+        assert cov["max_phys_warps"] == 12, f"physical warps: {cov['max_phys_warps']}"
+        assert cov["max_wait"] == 11, f"widest wait vector: {cov['max_wait']} warps"
+
+
+_LAT_COMMON = ("slow_jobs", "slow_const", "levels")
+_LAT_FUSED = _LAT_COMMON + ("dot_shapes", "dot_generic", "ops")
+_LAT_DF = _LAT_FUSED + ("chunks",)
+_LAT_LEVEL = _LAT_FUSED + ("chains", "empty_packet")
+# what each variant of LATENCY_VARIANTS must reach on latency_corpus()
+LATENCY_VARIANT_FEATURES = {
+    "df_defaults": _LAT_DF, "df_serial": _LAT_DF, "df_d_2": _LAT_DF, "df_no_fuse": _LAT_COMMON + ("chunks",), "df_links_2": _LAT_DF + ("sbox",),
+    "level_defaults": _LAT_LEVEL, "level_serial": _LAT_LEVEL, "level_d_2": _LAT_LEVEL, "level_no_fuse": _LAT_COMMON + ("chains", "empty_packet"),
+    "level_links_2": _LAT_LEVEL + ("sbox",),
+    "df_warps_12": _LAT_DF + ("warps_12",), "df_excl": _LAT_DF, "df_excl_w7s3": _LAT_DF + ("phys_12",), "df_excl_w8s4": _LAT_DF + ("warps_12",),
+    "df_no_chain": _LAT_DF, "df_no_split": _LAT_DF, "df_links_0": _LAT_DF,
+    "level_warps_12": _LAT_LEVEL, "level_d_200": _LAT_LEVEL, "level_no_split_chain": _LAT_FUSED + ("empty_packet",),
+}
+
+
+def slow_const_graph(k=12):
+    """Idiv, Mod and Pow of the inputs with a constant divisor / exponent on either side, in groups of k per opcode and side
+    (slow-warp jobs that read constants), next to k Div of inputs by inputs.  Constants: 0, 1, small, 2^64 + 1, M - 1."""
+    D = po.DUO
+    nodes = [(po.K_INPUT, i) for i in range(7)]
+    consts = []
+    for v in (0, 1, 3, 255, (1 << 64) + 1, M - 1, 7, M >> 3):
+        nodes.append((po.K_CONST, v))
+        consts.append(len(nodes) - 1)
+    wit = [0]
+    for op in ("Idiv", "Mod", "Pow"):
+        for j in range(k):
+            x, c = 1 + j % 6, consts[j % len(consts)]
+            if op == "Pow":
+                c = consts[2 + j % 2] if j % 3 else consts[j % 2]      # small exponents and a large base stay cheap on the oracle
+            nodes.append((po.K_DUO, D[op], x, c))
+            wit.append(len(nodes) - 1)
+            nodes.append((po.K_DUO, D[op], c if op != "Pow" else consts[5 - j % 2], x if op != "Pow" else 1 + j % 2))
+            wit.append(len(nodes) - 1)
+    for j in range(k):
+        nodes.append((po.K_DUO, D["Div"], 1 + j % 6, 1 + (j + 1) % 6))
+        wit.append(len(nodes) - 1)
+    return nodes, wit, {"x": (1, 6)}
+
+
+def dot_shape_graph(n_copies=4):
+    """Linear combinations of every straight-line OP_DOT shape -- c1 x1 [+ c2 x2] [+ x3] [+ k] -- with worst-case operands
+    (constants M - 1 and the one whose Montgomery form is M - 1, as in dot_ladder_graph), and the same shapes with a
+    subtracted value, which must take the generic loop.  Each combination is a witness value."""
+    r_inv = pow(1 << 256, -1, M)
+    cmax = (M - 1) * r_inv % M
+    D = po.DUO
+    nodes = [(po.K_INPUT, i) for i in range(7)]
+
+    def add(node):
+        nodes.append(node)
+        return len(nodes) - 1
+    wit = [0]
+    for rep in range(n_copies):
+        for n_mac in (1, 2):
+            for plus in (0, 1, 2):                   # 0: no added value, 1: + x3, 2: - x3 (generic loop)
+                for kc in (0, 1):
+                    cs = [(M - 1, cmax), (cmax, M - 1)][rep % 2]
+                    lc = add((po.K_DUO, D["Mul"], 1 + rep % 2, add((po.K_CONST, cs[0]))))
+                    if n_mac == 2:
+                        lc = add((po.K_DUO, D["Add"], lc, add((po.K_DUO, D["Mul"], add((po.K_CONST, cs[1])), 2 + rep % 3))))
+                    if plus:
+                        lc = add((po.K_DUO, D["Add" if plus == 1 else "Sub"], lc, 3 + rep % 4))
+                    if kc:
+                        lc = add((po.K_DUO, D["Add"], lc, add((po.K_CONST, [M - 1, cmax, M - cmax, 1][rep % 4]))))
+                    wit.append(lc)
+    return nodes, wit, {"x": (1, 6)}
+
+
+def tern_muladd_graph():
+    """TernCond with a constant in each operand position (and none), and Poseidon-style S-box links with constants, so that
+    the forced S-box link rewrite emits OP_MULADD with a constant operand; every result is a witness value (OP_TERN and
+    OP_MULADD store through a separate OP_OUT)"""
+    D = po.DUO
+    nodes = [(po.K_INPUT, i) for i in range(7)]
+
+    def add(node):
+        nodes.append(node)
+        return len(nodes) - 1
+    wit = [0]
+    c0, c1, c5 = add((po.K_CONST, 0)), add((po.K_CONST, M - 1)), add((po.K_CONST, 5))
+    for j in range(6):
+        x, y, z = 1 + j % 6, 1 + (j + 1) % 6, 1 + (j + 2) % 6
+        cond = add((po.K_DUO, D["Lt"], x, y)) if j % 2 else x
+        for a, b, c in ((cond, y, z), (c0 if j % 3 else c1, y, z), (cond, c1, z), (cond, y, c5), (cond, c1, c5)):
+            wit.append(add((po.K_TRES, 0, a, b, c)))
+    # S-box links s -> s^5 -> c * s^5 [+ k] -> ^5 ...: a link without other terms leaves OP_MULADD a constant 0 to add
+    s = 1
+    for r in range(8):
+        x2 = add((po.K_DUO, D["Mul"], s, s))
+        x4 = add((po.K_DUO, D["Mul"], x2, x2))
+        x5 = add((po.K_DUO, D["Mul"], x4, s))
+        wit += [x2, x4, x5]
+        s = add((po.K_DUO, D["Mul"], add((po.K_CONST, (r + 2) * 0x1234567 % M)), x5))
+        if r % 2:
+            s = add((po.K_DUO, D["Add"], s, add((po.K_CONST, M - 1 - r))))
+        wit.append(s)
+    return nodes, wit, {"x": (1, 6)}
+
+
+def edge_graphs():
+    """[(name, nodes, witness, input map)]: inputs only, constants only, one operation, and dependent chains of 1 .. 9
+    operations whose every step is also a witness value (level counts of 0, 1 and 2 mod 3, 1 and 2 levels in total)"""
+    D = po.DUO
+    out = [("inputs_only", [(po.K_INPUT, i) for i in range(7)], [0, 3, 1, 6, 2], {"x": (1, 6)}),
+           ("consts_only", [(po.K_INPUT, 0), (po.K_CONST, 7), (po.K_CONST, M - 1), (po.K_CONST, 0)], [0, 1, 2, 3, 1], {}),
+           ("one_op", [(po.K_INPUT, i) for i in range(3)] + [(po.K_DUO, D["Mul"], 1, 2)], [3], {"x": (1, 2)})]
+    for n in range(1, 10):
+        nodes = [(po.K_INPUT, i) for i in range(3)]
+        wit, v = [], 1
+        for j in range(n):
+            nodes.append((po.K_DUO, D["Mul"] if j % 2 else D["Add"], v, 2))
+            v = len(nodes) - 1
+            wit.append(v)
+        out.append((f"chain_{n}", nodes, wit, {"x": (1, 2)}))
+    return out
+
+
+def wide_live_graph(k: int):
+    """k values live at the same time: v_i = x_(i mod 6) + c_i at one level, then w_i = v_i * v_(i+1 mod k) at the next, the
+    products only as witness values.  The latency plan's value file needs k slots plus a constant few."""
+    D = po.DUO
+    nodes = [(po.K_INPUT, i) for i in range(7)]
+    vs = []
+    for i in range(k):
+        nodes.append((po.K_CONST, 1000003 * (i + 1)))
+        nodes.append((po.K_DUO, D["Add"], 1 + i % 6, len(nodes) - 1))
+        vs.append(len(nodes) - 1)
+    wit = [0]
+    for i in range(k):
+        nodes.append((po.K_DUO, D["Mul"], vs[i], vs[(i + 1) % k]))
+        wit.append(len(nodes) - 1)
+    return nodes, wit, {"x": (1, 6)}
+
+
+def latency_rows(rnd: random.Random, n_in: int, extra=()) -> list:
+    """input rows of one latency-corpus graph: an opening row that none of the checked rows repeats, the edge rows (all
+    M - 1, all 0, all 2^256 - 1), `extra` and matrix rows, in an order where consecutive witnesses differ"""
+    edge = [[1] + [M - 1] * n_in, [1] + [0] * n_in, [1] + [(1 << 256) - 1] * n_in]
+    return [matrix_row(rnd, n_in)] + [edge[0], matrix_row(rnd, n_in), edge[1], matrix_row(rnd, n_in), edge[2]] + list(extra) + [matrix_row(rnd, n_in) for _ in range(3)]
+
+
+def latency_corpus():
+    """The corpus of the latency matrix (tests/test_latency_plan.py on the simulator, tests/test_gpu_latency_matrix.py on the
+    GPU): [(name, nodes, witness, input map, rows)].  The plan-option matrix corpus (test_plan_sim.matrix_corpus) with
+    latency rows, slow-warp job widths of 31 .. 65, slow jobs with constants, every straight-line OP_DOT shape,
+    TernCond / S-box links with constants, Boolean and field-bits graphs, and edge graphs."""
+    from tests.test_bitplan import boolean_graph, field_bits_graph
+    from tests.test_plan_sim import matrix_corpus
+    rnd = random.Random(4242)
+    out = []
+    for name, nodes, wit, imap, rows in matrix_corpus():
+        n_in = len(rows[0]) - 1
+        if name.startswith("narrow_limits"):
+            rows = rows[::7]
+        out.append((name, nodes, wit, imap, latency_rows(rnd, n_in, rows[:24])))
+    for k in (31, 32, 33, 64, 65):
+        nodes, wit, imap = div_group_graph(k)
+        out.append((f"div_group_{k}", nodes, wit, imap, [matrix_row(rnd, 2 * k)] + div_group_rows(k, rnd)))
+    for name, (nodes, wit, imap) in (("slow_const", slow_const_graph()), ("dot_shapes", dot_shape_graph()), ("tern_muladd", tern_muladd_graph())):
+        zeros = [[1] + [0, M, 2 * M] * 2, [1, 1, 2, 3, M + 1, 2, 3], [1] + [M, 2 * M, 0] * 2, [1, 3, 1, 2, 3, M + 1, 2]]   # zero and tiny divisors
+        out.append((name, nodes, wit, imap, latency_rows(rnd, 6, zeros)))
+    for j in range(2):
+        nodes, wit, imap = boolean_graph(rnd, n_inputs=24, n_gates=300)
+        out.append((f"boolean_{j}", nodes, wit, imap, [[1] + [rnd.randrange(2) for _ in range(24)] for _ in range(24)]))
+        nodes, wit, imap = field_bits_graph(rnd)
+        n_in = imap["x"][1] if "x" in imap else sum(ln for _, ln in imap.values())
+        out.append((f"field_bits_{j}", nodes, wit, imap, [[1] + [0] * n_in] + [[1] + [random_value(rnd) if i < 3 else rnd.randrange(2) for i in range(n_in)] for _ in range(24)]))
+    for name, nodes, wit, imap in edge_graphs():
+        n_in = sum(ln for _, ln in imap.values())
+        out.append((name, nodes, wit, imap, latency_rows(rnd, n_in)))
+    return out
+
+
+def assert_rows_expose_stores(name, want):
+    """want: the oracle's witness rows [B, W, 32] of one graph, in call order, row 0 the opening row.  The latency entry point
+    copies the witness out of a device buffer that every call of the graph reuses, so a store the kernel skips shows the
+    previous call's value: every position that is not the same in all rows must change between two consecutive checked rows."""
+    w = want.reshape(len(want), -1, 32)
+    varies = (w != w[:1]).any(axis=2).any(axis=0)
+    changes = (w[2:] != w[1:-1]).any(axis=2).any(axis=0) if len(w) > 2 else np.zeros_like(varies)
+    hidden = np.nonzero(varies & ~changes)[0]
+    assert len(hidden) == 0, f"{name}: witness positions {hidden[:8].tolist()} never change between consecutive checked rows"
