@@ -984,7 +984,9 @@ struct Engine::Dev {
   // pinned host ring of the streaming API (three chunks: one in the consumer's hands, one landing, one enqueued)
   uint8_t* h_ring[3] = {nullptr, nullptr, nullptr}; uint32_t* h_flags[3] = {nullptr, nullptr, nullptr};
   size_t h_ring_bytes = 0, h_flags_n = 0;
-  // bit-sliced path (bitplan.hpp): program tables, and per-launch scratch that grows with the largest batch seen
+  // bit-sliced path (bitplan.hpp): program tables, and per-launch scratch that grows with the largest batch seen.
+  // bit_fits: the plan's plane file fits this device's shared memory (otherwise every call takes the generic kernels)
+  bool bit_fits = false;
   uint4* bit_code = nullptr; uint4* bit_inputs = nullptr; uint32_t* bit_field_inputs = nullptr; uint32_t* bit_field_slots = nullptr; uint32_t bit_n_contract = 0, bit_n_field = 0; int32_t* bit_constpos = nullptr; uint4* bit_consts = nullptr; uint4* bit_wide = nullptr;
   uint32_t* bit_planes = nullptr; uint32_t* bit_ok = nullptr; uint32_t* bit_bad = nullptr; uint32_t* bit_nbad = nullptr;
   size_t bit_groups = 0;
@@ -1065,6 +1067,8 @@ void Engine::init_plan() {
 
 // shared memory of a CTA of T threads without the hot-constant area: instruction rings + register file
 static size_t smem_base(const Plan& plan, int T) { return (size_t)(T / 32) * RING * 16 + (size_t)plan.n_regs * 32 * T; }
+// shared memory of one warp's plane file in bit_eval_kernel (the ring variants add mbarriers and header chunks behind it)
+static size_t bit_plane_bytes(const BitPlan& bp) { return ((size_t)bp.n_slots * 4 + 15) & ~(size_t)15; }
 
 // Launch geometry for a batch of B input sets: one persistent CTA per SM; T = the smallest multiple of 32 that
 // covers the batch in the fewest waves of full CTAs.
@@ -1125,7 +1129,8 @@ Engine::Dev* Engine::dev(int device) {
   CUDA_CHECK(cudaMemcpy(d->consts, plan.consts.data(), plan.consts.size() * 32, cudaMemcpyHostToDevice));
   d->spill_threads = (size_t)d->sms * t_max;
   if (plan.n_spill || plan.n_spill_narrow) CUDA_CHECK(cudaMalloc(&d->spill, ((size_t)plan.n_spill * 32 + (size_t)plan.n_spill_narrow * 8) * d->spill_threads));
-  if (use_bit_path()) {
+  d->bit_fits = use_bit_path() && bit_plane_bytes(bit_plan) <= d->smem_max;
+  if (d->bit_fits) {
     const BitPlan& bp = bit_plan;
     CUDA_CHECK(cudaFuncSetAttribute(bit_eval_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));
     CUDA_CHECK(cudaFuncSetAttribute(bit_eval_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));
@@ -1186,6 +1191,9 @@ void Engine::launch_bit(Dev* d, const void* d_inputs, size_t B, void* d_witness,
     CUDA_CHECK(cudaMalloc(&d->bit_bad, n_groups * 32 * 4));
     d->bit_groups = n_groups;
   }
+  // the count of an earlier launch may still be on its way to the host (launch() copies it after recording last_kernel,
+  // on that launch's stream): it has to land before this launch zeroes and recounts it
+  CUDA_CHECK(cudaStreamWaitEvent(s, d->bit_nbad_ev, 0));
   CUDA_CHECK(cudaMemsetAsync(d->bit_nbad, 0, 4, s));
   BParams q;
   q.code = d->bit_code; q.n_steps = bp.n_steps; q.n_slots = bp.n_slots;
@@ -1194,12 +1202,15 @@ void Engine::launch_bit(Dev* d, const void* d_inputs, size_t B, void* d_witness,
   q.inputs = (const uint4*)d_inputs; q.I = bp.n_inputs; q.W = bp.n_witness; q.B = B; q.n_groups = (uint32_t)n_groups;
   q.planes = d->bit_planes; q.plane_stride = bp.plane_stride; q.ok_words = d->bit_ok; q.bad_list = d->bit_bad; q.n_bad = d->bit_nbad; q.status = d_status;
   // shared memory per warp (group): the plane file, and for the ring variants 3 mbarriers + 3 chunks of LUT headers
-  const size_t planes_b = ((size_t)bp.n_slots * 4 + 15) & ~(size_t)15;
+  const size_t planes_b = bit_plane_bytes(bp);
   const size_t single_b = planes_b + 32 + 3 * (size_t)BIT_CHUNK_SINGLE * 512, ring_b = planes_b + 32 + 3 * (size_t)BIT_CHUNK_BATCH * 512;
-  if (planes_b > d->smem_max) throw Error("bit-sliced plan: plane file does not fit shared memory");
+  if (planes_b > d->smem_max) throw Error("bit-sliced plan: plane file does not fit shared memory");     // callers check d->bit_fits
+  // GW_TRACE_HOST=1: which variant of bit_eval_kernel ran, in what shape
+  const bool trace = env_int("GW_TRACE_HOST", 0) != 0;
   if (B == 1 && single_b <= d->smem_max) {
     q.warp_bytes = (uint32_t)single_b;
     bit_eval_kernel<true, true><<<1, 32, single_b, s>>>(q);
+    if (trace) fprintf(stderr, "[gw bit] variant single, warps 1, ctas 1, groups 1\n");
   } else {
     // ring variant unless it would leave an SM with fewer resident groups than the batch can give it (GW_BIT_RING=0/1 forces)
     const int env_ring = env_int("GW_BIT_RING", -1);
@@ -1218,6 +1229,7 @@ void Engine::launch_bit(Dev* d, const void* d_inputs, size_t B, void* d_witness,
     const unsigned grid = (unsigned)((n_groups + wpb - 1) / wpb);
     if (ring) bit_eval_kernel<false, true><<<grid, wpb * 32, (size_t)wpb * wb, s>>>(q);
     else bit_eval_kernel<false, false><<<grid, wpb * 32, (size_t)wpb * wb, s>>>(q);
+    if (trace) fprintf(stderr, "[gw bit] variant %s, warps %d, ctas %u, groups %zu\n", ring ? "ring" : "reg", wpb, grid, n_groups);
   }
   CUDA_CHECK(cudaGetLastError());
   const uint32_t tiles = (bp.n_witness + 31) / 32;
@@ -1245,7 +1257,7 @@ void Engine::launch(Dev* d, const void* d_inputs, size_t B, void* d_witness, uin
     d->bit_nbad_pending = false;
     if (d->bit_nbad_sets >= 64 && (size_t)*d->bit_nbad_host * 2 > d->bit_nbad_sets) bit_disabled.store(true);
   }
-  const bool bit = use_bit_path() && !bit_disabled.load() && B >= (size_t)env_int("GW_BIT_MIN_SETS", 1);
+  const bool bit = d->bit_fits && !bit_disabled.load() && B >= (size_t)env_int("GW_BIT_MIN_SETS", 1);
   if (bit) launch_bit(d, d_inputs, B, d_witness, d_status, stream);
   KParams p;
   p.row_map = bit ? d->bit_bad : nullptr; p.n_dev = bit ? d->bit_nbad : nullptr;
@@ -1500,7 +1512,7 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
   // node per lane, values in a shared-memory plane file, __syncwarp between steps (no CTA barrier, no packets).  One
   // input set occupies bit 0 of every plane word.  SHA-256(512): 8 058 steps against 7 010 levels of 256-bit
   // instructions in the generic latency plan.  An input set that breaks the bit contract takes the generic plan below.
-  if (bit_path_active() && bit_plan.n_luts > 0 && env_int("GW_LAT_BIT", 1) != 0) {     // pure wiring (Num2Bits alone): three launches cost more than the generic kernel
+  if (d->bit_fits && bit_path_active() && bit_plan.n_luts > 0 && env_int("GW_LAT_BIT", 1) != 0) {     // pure wiring (Num2Bits alone): three launches cost more than the generic kernel
     CUDA_CHECK(cudaMemcpyAsync(d->lat_in, inputs, (size_t)plan.n_inputs * 32, cudaMemcpyHostToDevice, 0));
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (kernel_ms) { CUDA_CHECK(cudaEventCreate(&e0)); CUDA_CHECK(cudaEventCreate(&e1)); CUDA_CHECK(cudaEventRecord(e0, 0)); }

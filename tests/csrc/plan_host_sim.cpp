@@ -480,11 +480,16 @@ struct BitSim { Graph g; BitPlan bp; };
 
 extern "C" {
 
+BitSim* sim_bit_load2(const uint8_t* data, size_t len, uint32_t max_support, int merge, uint32_t max_slots, char* err, size_t errlen);
 BitSim* sim_bit_load(const uint8_t* data, size_t len, uint32_t max_support, int merge, char* err, size_t errlen) {
+  return sim_bit_load2(data, len, max_support, merge, 0, err, errlen);
+}
+// max_slots: GW_BIT_MAX_SLOTS (0 = default)
+BitSim* sim_bit_load2(const uint8_t* data, size_t len, uint32_t max_support, int merge, uint32_t max_slots, char* err, size_t errlen) {
   try {
     std::unique_ptr<BitSim> s(new BitSim());
     s->g = deserialize_witnesscalc_graph(data, len);
-    BitPlanOptions o; if (max_support) o.max_support = max_support; o.merge_luts = merge != 0;
+    BitPlanOptions o; if (max_support) o.max_support = max_support; o.merge_luts = merge != 0; if (max_slots) o.max_slots = max_slots;
     s->bp = compile_bit_plan(s->g, o);
     if (!s->bp.eligible && err && errlen) { strncpy(err, s->bp.reason.c_str(), errlen - 1); err[errlen - 1] = 0; }
     return s.release();
@@ -496,6 +501,15 @@ void sim_bit_info(BitSim* s, uint64_t* out) {
   out[0] = b.eligible; out[1] = b.n_steps; out[2] = b.n_slots; out[3] = b.n_luts; out[4] = b.n_levels; out[5] = b.n_nodes_bit;
   out[6] = b.n_nodes_tt; out[7] = b.n_nodes_bv; out[8] = b.n_full_adders; out[9] = b.n_merged; out[10] = b.inputs.size() / 3; out[11] = b.const_vals.size();
   out[12] = b.has_field_inputs; out[13] = b.wide.size() / 3; out[14] = b.plane_stride;
+}
+// the compiled plan: which = 0 code (4 words per LUT), 1 inputs (triples), 2 wide (triples), 3 const_of_pos (int32 as
+// uint32); copies up to cap words and returns the number of words
+size_t sim_bit_plan(BitSim* s, int which, uint32_t* out, size_t cap) {
+  const BitPlan& b = s->bp;
+  const uint32_t* src = which == 0 ? reinterpret_cast<const uint32_t*>(b.code.data()) : which == 1 ? b.inputs.data() : which == 2 ? b.wide.data() : (const uint32_t*)b.const_of_pos.data();
+  const size_t n = which == 0 ? b.code.size() * 4 : which == 1 ? b.inputs.size() : which == 2 ? b.wide.size() : b.const_of_pos.size();
+  if (out && src) memcpy(out, src, std::min(n, cap) * 4);
+  return n;
 }
 // inputs: n x I x 32 B (n <= 32), witness: n x W x 32 B; returns the mask of input sets that satisfy the bit contract
 // (only their rows are written), or -1 on a malformed plan

@@ -240,3 +240,29 @@ def test_field_inputs_taken_apart_into_bits_and_wide_outputs():
         for b, row in enumerate(rows):
             if res[b] is not None:
                 assert res[b] == po.evaluate(nodes, row, wit, "circom"), (t, b)
+
+
+def test_bit_corpus_coverage():
+    """util.bit_corpus, the corpus of the GPU matrix (tests/test_gpu_bit_matrix.py), reaches everything util.bit_plan_coverage
+    records, and its plans are exact on the simulator: every step residue mod 16, header rings of 1 .. 4 and >= 7 chunks,
+    steps of 1, 2 .. 31 and 32 LUTs, copies, slot reuse, wide values of every plane-loop length, constants, unread contract
+    inputs and field-input bits in every limb"""
+    from oracle import cref
+    import numpy as np
+    rnd = random.Random(11)
+    cov = None
+    for name, data in util.bit_corpus():
+        g = util.BitSimGraph(data)
+        assert g.info["eligible"] and (g.info["n_luts"] or g.info["has_field_inputs"]), name
+        c = util.bit_plan_coverage(g.plan())
+        cov = c if cov is None else util.merge_coverage(cov, c)
+        if g.W > 5000:
+            continue                                   # SHA-256: test_sha256_is_all_bits_and_exact
+        rows = [[1] + [rnd.choice([0, 1, 1, M - 1, (1 << 256) - 1]) if rnd.random() < 0.3 else rnd.randrange(2) for _ in range(g.I - 1)]
+                for _ in range(32)]
+        res, ok = g.eval(rows)
+        want = cref.CGraph(data).evaluate_batch(np.frombuffer(b"".join(util.pack_u256(r) for r in rows), dtype=np.uint8).reshape(32, -1, 32), 4)
+        for b in range(32):
+            if (ok >> b) & 1:
+                assert res[b] == util.unpack_u256(want[b].tobytes()), (name, b)
+    util.assert_bit_coverage(cov)

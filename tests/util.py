@@ -259,6 +259,10 @@ def sim_lib():
         L.sim_reserialize.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_size_t]
         L.sim_bit_load.restype = ctypes.c_void_p
         L.sim_bit_load.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint32, ctypes.c_int, ctypes.c_char_p, ctypes.c_size_t]
+        L.sim_bit_load2.restype = ctypes.c_void_p
+        L.sim_bit_load2.argtypes = [ctypes.c_char_p, ctypes.c_size_t, ctypes.c_uint32, ctypes.c_int, ctypes.c_uint32, ctypes.c_char_p, ctypes.c_size_t]
+        L.sim_bit_plan.restype = ctypes.c_size_t
+        L.sim_bit_plan.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_uint32), ctypes.c_size_t]
         L.sim_bit_free.argtypes = [ctypes.c_void_p]
         L.sim_bit_info.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint64)]
         L.sim_bit_eval.restype = ctypes.c_int64
@@ -270,10 +274,10 @@ def sim_lib():
 class BitSimGraph:
     """bit-sliced plan (csrc/bitplan.cpp) on the host simulator: groups of up to 32 input sets"""
 
-    def __init__(self, data: bytes, max_support=0, merge=True):
+    def __init__(self, data: bytes, max_support=0, merge=True, max_slots=0):
         self.L = sim_lib()
         err = ctypes.create_string_buffer(512)
-        self.h = self.L.sim_bit_load(data, len(data), max_support, int(merge), err, 512)
+        self.h = self.L.sim_bit_load2(data, len(data), max_support, int(merge), max_slots, err, 512)
         if not self.h:
             raise ValueError(err.value.decode())
         info = (ctypes.c_uint64 * 15)()
@@ -294,6 +298,17 @@ class BitSimGraph:
         assert ok >= 0, "malformed bit plan"
         res = [unpack_u256(out.raw[32 * self.W * b:32 * self.W * (b + 1)]) if (ok >> b) & 1 else None for b in range(n)]
         return res, int(ok)
+
+    def plan(self) -> dict:
+        """the compiled plan: code [n_steps, 32, 4] (x, y, z, w of every lane), inputs [n, 3] and wide [n, 3] triples,
+        const_of_pos [W] (int32: -1 a plane, -2 a wide value, else a constant index), and W"""
+        def part(which, dtype=np.uint32):
+            n = self.L.sim_bit_plan(self.h, which, None, 0)
+            a = np.zeros(max(n, 1), dtype=np.uint32)
+            self.L.sim_bit_plan(self.h, which, a.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32)), n)
+            return a[:n].view(dtype)
+        return {"code": part(0).reshape(-1, 32, 4), "inputs": part(1).reshape(-1, 3), "wide": part(2).reshape(-1, 3),
+                "const_of_pos": part(3, np.int32), "W": self.W}
 
     def __del__(self):
         if getattr(self, "h", None):
@@ -937,3 +952,168 @@ def assert_rows_expose_stores(name, want):
     changes = (w[2:] != w[1:-1]).any(axis=2).any(axis=0) if len(w) > 2 else np.zeros_like(varies)
     hidden = np.nonzero(varies & ~changes)[0]
     assert len(hidden) == 0, f"{name}: witness positions {hidden[:8].tolist()} never change between consecutive checked rows"
+
+
+# ---- bit-sliced path: coverage and corpus of bit_eval_kernel / bit_expand_kernel / bit_expand_wide_kernel ------------------
+BIT_NO_SLOT, BIT_NO_POS, BIT_CONTRACT = 0xFFFF, 0xFFFFFFFF, 0xFFFFFFFF      # csrc/bitplan.hpp
+BIT_CHUNK_SINGLE, BIT_CHUNK_BATCH = 16, 8                                   # engine.cu: steps per TMA chunk of a header ring
+
+
+def bit_chunks(n_steps: int, ch: int) -> int:
+    """header-ring chunks of a bit program (steps 1 .. n_steps - 1, engine.cu: bit_eval_kernel)"""
+    return -(-(n_steps - 1) // ch)
+
+
+def bit_plan_coverage(plan: dict) -> dict:
+    """what the kernels do with one compiled bit plan (BitSimGraph.plan): sets of step residues and ring chunk counts, the
+    LUTs per step, copies, slot reuse, wide planes and their plane counts, constants, unread contract inputs and the field
+    input bits by limb.  Merge records with merge_coverage."""
+    code, W = plan["code"], plan["W"]
+    n_steps = len(code)
+    cov = {"res4": {(n_steps - 1) % 4}, "res8": {(n_steps - 1) % 8}, "res16": {(n_steps - 1) % 16},
+           "chunks8": {min(bit_chunks(n_steps, BIT_CHUNK_BATCH), 7)}, "chunks16": {min(bit_chunks(n_steps, BIT_CHUNK_SINGLE), 5)},
+           "step_luts": set(), "copy": 0, "multi_pos": 0, "slot_reuse": 0, "wide_writes": 0}
+    written = set(int(s) for s in plan["inputs"][:, 1] if s != BIT_NO_SLOT) | {0, 1}
+    stored = {}                                      # slot -> its current plane is also at a witness position
+    for st in range(1, n_steps):
+        ops = code[st]
+        x, y, z, w = (ops[:, k].astype(np.int64) for k in range(4))
+        dst = z >> 16
+        real = (dst != BIT_NO_SLOT) | (w != BIT_NO_POS)
+        n = int(real.sum())
+        cov["step_luts"].add("1" if n == 1 else "32" if n == 32 else "2-31" if n else "0")
+        copy = real & (x == 0xAA) & (dst == BIT_NO_SLOT)
+        cov["copy"] += int(copy.sum())
+        for a in (y[copy] & 0xFFFF).tolist():
+            cov["multi_pos"] += int(stored.get(a, False))
+            stored[a] = True
+        cov["wide_writes"] += int(((w != BIT_NO_POS) & (w >= W)).sum())
+        for d, pos in zip(dst[dst != BIT_NO_SLOT].tolist(), w[dst != BIT_NO_SLOT].tolist()):
+            cov["slot_reuse"] += int(d in written)
+            written.add(d)
+            stored[d] = pos != BIT_NO_POS and pos < W
+    wide_np = [int(t[2]) for t in plan["wide"]]
+    cov["wide_planes"] = {k for k in (2, 31, 32, 33, 254) if k in wide_np} | ({"225+"} if any(k >= 225 for k in wide_np) else set())
+    cov["wide_m"] = {-(-k // 32) for k in wide_np}
+    cov["consts"] = int((plan["const_of_pos"] >= 0).sum())
+    inp = plan["inputs"]
+    contract = inp[:, 2] == BIT_CONTRACT
+    cov["contract_no_slot"] = int((contract & (inp[:, 1] == BIT_NO_SLOT)).sum())
+    fbits = [int(b) for b in inp[~contract, 2]]
+    cov["field_limbs"] = {b >> 5 for b in fbits}
+    cov["field_bits"] = {b for b in fbits if b in (31, 32, 253)}
+    return cov
+
+
+BIT_COVERAGE = {"res4": set(range(4)), "res8": set(range(8)), "res16": set(range(16)), "chunks8": {1, 2, 3, 4, 7},
+                "chunks16": {1, 2, 3, 4}, "step_luts": {"1", "2-31", "32"}, "wide_planes": {2, 31, 32, 33, 254, "225+"},
+                "wide_m": set(range(1, 9)), "field_limbs": set(range(8)), "field_bits": {31, 32, 253}}
+BIT_COUNTS = ("copy", "multi_pos", "slot_reuse", "wide_writes", "consts", "contract_no_slot")
+
+
+def assert_bit_coverage(cov: dict):
+    for k, want in BIT_COVERAGE.items():
+        assert want <= cov[k], f"bit plan coverage: {k} lacks {sorted(want - cov[k], key=str)}"
+    for k in BIT_COUNTS:
+        assert cov[k] > 0, f"bit plan coverage: no {k}"
+
+
+def wide_counts_graph():
+    """Bits2Num sums of k bits for k = 31, 32, 33 and 64 .. 250 in steps (every iteration count of the wide expansion's plane
+    loop), a Num2Bits input passed through as a witness (254 planes), 2 b (the narrowest wide value: a value of one plane is a
+    plane position), a masked slice, constants and one bit at three witness positions"""
+    D = po.DUO
+    widths = (31, 32, 33, 64, 96, 128, 160, 192, 200, 225, 250)
+    n_bits = 40
+    nodes = [(po.K_INPUT, i) for i in range(n_bits + 2)]
+    cache = {}
+
+    def const(v):
+        if v not in cache:
+            nodes.append((po.K_CONST, v))
+            cache[v] = len(nodes) - 1
+        return cache[v]
+
+    def duo(op, a, b):
+        nodes.append((po.K_DUO, D[op], a, b))
+        return len(nodes) - 1
+    f = n_bits + 1                                      # a field input: taken apart, passed through
+    wit = [0, f]
+    fb = [duo("Band", duo("Shr", f, const(k)), const(1)) for k in range(254)]
+    wit += [fb[31], fb[32], fb[253], fb[0]]
+    for i, k in enumerate(widths):
+        lc = const(0)
+        for j in range(k):
+            b = 1 + (i * 7 + j * 3) % n_bits if j % 2 == 0 else fb[(i * 11 + j) % 254]
+            lc = duo("Add", lc, duo("Mul", b, const(1 << j)))
+        wit.append(lc)
+    x = duo("Mul", 1, 2)
+    wit += [x, const(5), x, const(0), x, const(1), duo("Band", duo("Shr", f, const(100)), const((1 << 37) - 1)), duo("Mul", 3, const(2))]
+    return nodes, wit, {"x": (1, n_bits + 1)}
+
+
+def bit_chain_graph(k: int, n_in=64):
+    """k values alive at once: v_i = x_a ^ x_b (distinct input pairs) at one level, w_i = v_i & v_(i+1 mod k) at the next, the
+    w only as witness values.  The bit plan's plane file needs about k + n_in slots; its program ~2k/32 steps."""
+    D = po.DUO
+    nodes = [(po.K_INPUT, i) for i in range(n_in + 1)]
+    nodes.append((po.K_CONST, 2))
+    two = len(nodes) - 1
+    vs = []
+    pairs = ((a, b) for d in range(1, n_in) for a in range(1, n_in + 1 - d) for b in (a + d,))
+    for _, (a, b) in zip(range(k), pairs):
+        nodes.append((po.K_DUO, D["Mul"], a, b))
+        nodes.append((po.K_DUO, D["Mul"], two, len(nodes) - 1))
+        nodes.append((po.K_DUO, D["Add"], a, b))
+        nodes.append((po.K_DUO, D["Sub"], len(nodes) - 1, len(nodes) - 2))
+        vs.append(len(nodes) - 1)
+    assert len(vs) == k, "not enough input pairs"
+    wit = [0]
+    for i in range(k):
+        nodes.append((po.K_DUO, D["Mul"], vs[i], vs[(i + 1) % k]))
+        wit.append(len(nodes) - 1)
+    return nodes, wit, {"x": (1, n_in)}
+
+
+_bit_corpus = None
+
+
+def bit_corpus():
+    """The corpus of the bit-sliced matrix (tests/test_gpu_bit_matrix.py): random Boolean
+    and field-bits graphs picked by their simulator step counts so that util.bit_plan_coverage of the set is full (every
+    residue of the step count mod 16, header rings of 1 .. 4 and >= 7 chunks), wide_counts_graph, and the golden SHA-256.
+    Entries: (name, graph bytes)."""
+    global _bit_corpus
+    if _bit_corpus is not None:
+        return _bit_corpus
+    from tests.test_bitplan import boolean_graph, field_bits_graph
+    out, cov = [], None
+    rnd = random.Random(5150)
+
+    def take(name, nodes, wit, imap, force=False, data=None):
+        nonlocal cov
+        data = data or po.serialize_graph(nodes, wit, imap)
+        g = BitSimGraph(data)
+        # (not eligible: a random word sum that can reach the modulus; no LUT and no field input: pure wiring, which the
+        # engine leaves to the generic kernel)
+        if not g.info["eligible"] or not (g.info["n_luts"] or g.info["has_field_inputs"]):
+            assert not force, (name, g.reason)
+            return
+        c = bit_plan_coverage(g.plan())
+        new = cov is None or any(not (c[k] <= cov[k]) for k in BIT_COVERAGE)
+        if force or new:
+            cov = c if cov is None else merge_coverage(cov, c)
+            out.append((name, data))
+    take("wide_counts", *wide_counts_graph(), force=True)
+    take("field_bits", *field_bits_graph(rnd, n_field=2, n_bits=6, n_gates=60), force=True)
+    # step counts 2 .. ~70 come from small graphs, long ones from big graphs: keep a graph when it adds a residue or a chunk count
+    for t in range(400):
+        if all(BIT_COVERAGE[k] <= cov[k] for k in ("res16", "chunks8", "chunks16", "step_luts")):
+            break
+        n_gates = (2, 4, 8, 12, 20, 30, 45, 60, 90, 140)[t % 10]
+        take(f"boolean_{t}", *boolean_graph(rnd, n_inputs=rnd.choice([3, 5, 24, 70]), n_gates=n_gates))
+    take("boolean_long", *boolean_graph(rnd, n_inputs=40, n_gates=700), force=True)
+    take("sha256_512", None, None, None, force=True, data=golden_graph("circuit8_sha256_512"))
+    assert_bit_coverage(cov)
+    _bit_corpus = out
+    return out
