@@ -28,6 +28,8 @@ BIN_EXAMPLE = os.path.join(HERE, "bin", "example-calc-witness")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 SOURCES = ["engine.cu", "r1cs.cu", "ntt.cu", "graph.cpp", "plan.cpp", "bitplan.cpp", "inputs.cpp", "wtns.cpp", "r1cs.cpp", "capi.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
+# the optimisation flags of every device build (the test-only device harness of tests/csrc is built with them too)
+OPT = ["-std=c++17", "-O3", "-lineinfo"]
 
 
 def _newer(target, deps):
@@ -42,14 +44,14 @@ def build(force=False, verbose=False):
     os.makedirs(os.path.dirname(BIN), exist_ok=True)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, "..", "include", "graph_witness.h")]
     if force or _newer(LIB, deps):
-        cmd = [NVCC, "-shared", "-Xcompiler", "-fPIC,-O3,-Wall,-Wno-unknown-pragmas,-Wno-misleading-indentation", "-std=c++17", "-O3", "-lineinfo", *ARCH,
+        cmd = [NVCC, "-shared", "-Xcompiler", "-fPIC,-O3,-Wall,-Wno-unknown-pragmas,-Wno-misleading-indentation", *OPT, *ARCH,
                "-Xptxas", "-v" if verbose else "-O3", "-o", LIB] + [os.path.join(CSRC, s) for s in SOURCES]
         if verbose:
             print(" ".join(cmd))
         subprocess.check_call(cmd)
     if force or _newer(LIB_PROF, deps):
         os.makedirs(os.path.dirname(LIB_PROF), exist_ok=True)
-        cmd = [NVCC, "-shared", "-Xcompiler", "-fPIC,-O3", "-std=c++17", "-O3", "-lineinfo", *ARCH, "-DGW_PROFILING",
+        cmd = [NVCC, "-shared", "-Xcompiler", "-fPIC,-O3", *OPT, *ARCH, "-DGW_PROFILING",
                "-o", LIB_PROF] + [os.path.join(CSRC, s) for s in SOURCES]
         subprocess.check_call(cmd)
     if force or _newer(BIN, [LIB, os.path.join(CSRC, "calc_witness_main.cpp")]):

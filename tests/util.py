@@ -204,14 +204,26 @@ def poseidon_like_graph(rnd: random.Random, t=3, rounds=8, n_inputs=6):
 
 
 # ---- test-only host libraries -------------------------------------------------------------------------
-def _build(name, sources, extra=()):
+GXX = ("g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-Wno-unknown-pragmas")
+
+
+def _build(name, sources, extra=(), compiler=GXX):
+    """tests/_build/<name> from `sources` with the compiler command `compiler`, rebuilt when a source or csrc/ is newer"""
     os.makedirs(BUILD, exist_ok=True)
     out = os.path.join(BUILD, name)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [s for s in sources]
     if not os.path.exists(out) or any(os.path.getmtime(d) > os.path.getmtime(out) for d in deps):
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-Wno-unknown-pragmas", "-o", out,
-                               *sources, *extra])
+        subprocess.check_call([*compiler, "-o", out, *sources, *extra])
     return out
+
+
+def _product_build():
+    """circom-witnesscalc_b200/build.py as a module: its compiler, architecture and optimisation flags"""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("_cwc_build", os.path.join(ROOT, "circom-witnesscalc_b200", "build.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
 
 
 _libs = {}
@@ -226,6 +238,20 @@ def field_host_lib(emulate_ptx=False):
                                         [os.path.join(ROOT, "tests/csrc/field_host_api.cpp")],
                                         extra=("-DGW_EMULATE_PTX",) if emulate_ptx else ()))
     return _libs[key]
+
+
+def field_device_lib():
+    """tests/csrc/field_device_api.cu: the primitives of csrc/field.cuh, inv_safegcd.cuh, alu.cuh and ntt.cuh as device
+    kernels (fd_launch), compiled for sm_100a with the library's compiler and flags"""
+    if "field_device" not in _libs:
+        b = _product_build()
+        L = ctypes.CDLL(_build("libfielddevice.so", [os.path.join(ROOT, "tests/csrc/field_device_api.cu")],
+                               compiler=(b.NVCC, "-shared", "-Xcompiler", "-fPIC", *b.OPT, *b.ARCH)))
+        u32p = ctypes.POINTER(ctypes.c_uint32)
+        L.fd_shape.argtypes = [ctypes.c_int, ctypes.POINTER(ctypes.c_int)]
+        L.fd_launch.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int] + [u32p] * 6
+        _libs["field_device"] = L
+    return _libs["field_device"]
 
 
 def sim_lib():
