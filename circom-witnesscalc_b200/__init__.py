@@ -74,6 +74,8 @@ _L.gw_calc_witness_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _vp, _v
 _L.gw_calc_witness_latency.argtypes = [_vp, ctypes.c_int, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(gw_status_t)]
 _L.gw_wtns_header.argtypes = [ctypes.c_uint32, _vp]
 _L.gw_inputs_parse_batch.argtypes = [_vp, ctypes.c_char_p, _sz, ctypes.c_int, ctypes.POINTER(_vp), ctypes.POINTER(_sz), ctypes.POINTER(gw_status_t)]
+_L.gw_inputs_parse_batch_device.argtypes = [_vp, ctypes.c_int, ctypes.c_char_p, _sz, _vp, _sz, ctypes.POINTER(_sz), _vp,
+                                             ctypes.POINTER(gw_status_t)]
 _L.gw_wtns_file_size.restype = _sz
 _L.gw_wtns_file_size.argtypes = [_vp]
 _L.gw_calc_witness_batch_wtns.argtypes = [_vp, _vp, _sz, _vp, _sz, _vp, ctypes.c_int, ctypes.POINTER(gw_status_t)]
@@ -105,7 +107,7 @@ EXPORTS = ["gw_calc_witness", "gw_graph_load", "gw_graph_free", "gw_graph_info",
            "gw_graph_select", "gw_calc_witness_batch_stream", "gw_set_device", "gw_r1cs_load", "gw_r1cs_free", "gw_r1cs_info",
            "gw_r1cs_check_batch", "gw_r1cs_check_batch_device", "gw_calc_witness_batch_check", "gw_r1cs_abc_len",
            "gw_r1cs_abc_batch", "gw_r1cs_abc_batch_device", "gw_fr_ntt_batch_device", "gw_r1cs_quotient_batch",
-           "gw_r1cs_quotient_batch_device"]
+           "gw_r1cs_quotient_batch_device", "gw_inputs_parse_batch_device"]
 
 
 class WitnessCalcError(RuntimeError):
@@ -251,6 +253,19 @@ class Graph:
         arr = arr.reshape(n.value, self.n_inputs, 32).copy()           # one copy out of the malloc'ed buffer
         _libc.free(out)
         return arr
+
+    def parse_inputs_batch_device(self, text, device, d_inputs_ptr, max_sets, stream=None) -> int:
+        """JSON Lines (or a JSON array of objects) -> DEVICE rows: row r (n_inputs x 32 B) at d_inputs_ptr + r * n_inputs * 32,
+        the same bytes as parse_inputs_batch.  Returns the number of input sets; more than max_sets is an error whose
+        message names the count (max_sets=0 with d_inputs_ptr=None only counts).  Ordered on `stream` (a cudaStream_t
+        as int, None = default stream); returns when the rows are complete (gw_inputs_parse_batch_device)."""
+        if isinstance(text, str):
+            text = text.encode("utf-8")
+        n, st = _sz(), gw_status_t()
+        rc = _L.gw_inputs_parse_batch_device(self._h, device, text, len(text), d_inputs_ptr, max_sets, ctypes.byref(n), stream,
+                                             ctypes.byref(st))
+        _check(rc, st)
+        return n.value
 
     def wtns_file_size(self) -> int:
         return int(_L.gw_wtns_file_size(self._h))

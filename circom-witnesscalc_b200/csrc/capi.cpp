@@ -20,6 +20,9 @@ using namespace gw;
 struct gw_graph {
   std::unique_ptr<Engine> engine;
   std::vector<std::string> input_names;
+  // device input parser (key tables and scratch per device), made by the first gw_inputs_parse_batch_device
+  mutable std::unique_ptr<DeviceInputs> dev_inputs;
+  mutable std::mutex dev_inputs_mu;
 };
 
 struct gw_r1cs {
@@ -205,6 +208,22 @@ int gw_inputs_parse_batch(const gw_graph_t* graph, const char* text, size_t text
     U256* rows = nullptr;
     size_t n = parse_inputs_batch(graph->engine->graph, text, text_len, n_threads, &rows);
     *inputs = (uint8_t*)rows; *n_sets = n;
+  });
+}
+
+int gw_inputs_parse_batch_device(const gw_graph_t* graph, int device, const char* text, size_t text_len, void* d_inputs,
+                                 size_t max_sets, size_t* n_sets, void* cuda_stream, gw_status_t* status) {
+  if (!graph || !n_sets || (text_len && !text) || (max_sets && !d_inputs)) { set_status(status, ERROR, "null argument"); return 1; }
+  *n_sets = 0;
+  return guarded(status, [&]() {
+    if (cuda_device_count() == 0) throw Error("no CUDA device available: this library has no CPU fallback");
+    DeviceInputs* p;
+    {
+      std::lock_guard<std::mutex> lk(graph->dev_inputs_mu);
+      if (!graph->dev_inputs) graph->dev_inputs.reset(new DeviceInputs(graph->engine->graph));
+      p = graph->dev_inputs.get();
+    }
+    p->parse(device, text, text_len, d_inputs, max_sets, cuda_stream, n_sets);
   });
 }
 

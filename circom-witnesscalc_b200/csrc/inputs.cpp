@@ -160,7 +160,7 @@ std::vector<U256> build_inputs_buffer(const Graph& g, const InputList& inputs) {
 
 
 // record boundaries: JSON Lines, or the elements of one top-level array (split at depth-1 commas, strings skipped)
-static void split_records(const char* text, size_t len, std::vector<std::pair<size_t, size_t>>& rec) {
+void split_records(const char* text, size_t len, std::vector<std::pair<size_t, size_t>>& rec) {
   size_t i = 0;
   while (i < len && (text[i] == ' ' || text[i] == '\t' || text[i] == '\n' || text[i] == '\r')) i++;
   if (i < len && text[i] == '[') {

@@ -139,6 +139,17 @@ int gw_calc_witness_latency(gw_graph_t *graph, int device, const uint8_t *inputs
 int gw_inputs_parse_batch(const gw_graph_t *graph, const char *text, size_t text_len, int n_threads,
                           uint8_t **inputs, size_t *n_sets, gw_status_t *status);
 
+/* the same parse on CUDA device `device`: `text` (host memory, pageable or pinned; pinned copies faster) is copied
+ * up once and split and parsed there; row r (n_inputs x 32 B) goes to d_inputs + r * n_inputs * 32, the layout
+ * gw_calc_witness_batch_device reads.  *n_sets and the rows are byte-identical to gw_inputs_parse_batch, and so is
+ * the error text.  Records outside the plain grammar (string escapes, '_' in numbers, repeated keys, "", errors) are
+ * parsed by the host from the same text.  More than max_sets records is an error that leaves *n_sets = the count and
+ * writes no row; max_sets = 0 with d_inputs = NULL only counts.  The work is ordered on `cuda_stream` (a cudaStream_t,
+ * NULL = default stream); the call returns when the rows are complete, and later work on that stream sees them. */
+int gw_inputs_parse_batch_device(const gw_graph_t *graph, int device, const char *text, size_t text_len,
+                                 void *d_inputs, size_t max_sets, size_t *n_sets, void *cuda_stream,
+                                 gw_status_t *status);
+
 /* ---- batch output path (SURVEY 8f-2) ----
  * .wtns framing: like gw_calc_witness_batch, but set i is delivered as a complete .wtns file image
  * (wtns_from_witness, src/lib.rs:114-123: 76-byte header + n_witness x 32 B) at files + i * file_pitch;

@@ -115,4 +115,7 @@ extern "C" {
     pub fn gw_r1cs_quotient_batch_device(r1cs: *mut gw_r1cs_t, device: c_int, d_witness: *const c_void, n_sets: usize,
                                          row_pitch: usize, d_work: *mut c_void, work_pitch: usize, d_first_failed: *mut u32,
                                          cuda_stream: *mut c_void, status: *mut gw_status_t) -> c_int;
+    pub fn gw_inputs_parse_batch_device(graph: *const gw_graph_t, device: c_int, text: *const c_char, text_len: usize,
+                                        d_inputs: *mut c_void, max_sets: usize, n_sets: *mut usize, cuda_stream: *mut c_void,
+                                        status: *mut gw_status_t) -> c_int;
 }
