@@ -1249,7 +1249,11 @@ void Engine::launch_bit(Dev* d, const void* d_inputs, size_t B, void* d_witness,
 }
 
 void Engine::launch(Dev* d, const void* d_inputs, size_t B, void* d_witness, uint32_t* d_status, void* stream) {
-  if (B == 0 || plan.code.empty()) return;
+  if (B == 0) return;
+  if (plan.code.empty()) {            // an empty witness (gw_graph_select of no position): nothing to run, no set is flagged
+    if (d_status) CUDA_CHECK(cudaMemsetAsync(d_status, 0, B * 4, (cudaStream_t)stream));
+    return;
+  }
   // The bit-sliced plan speculates that the inputs under its contract are bits.  When most input sets of a launch were
   // not (somebody feeds field elements to a graph that would also work on bits), the speculation is dropped for this
   // graph: such batches would pay for both paths.  The count arrives asynchronously; it is looked at on the next launch.
@@ -1501,6 +1505,11 @@ void Engine::run_stream(const uint8_t* inputs, size_t B, int n_gpus, int first_d
 // one witness, host buffers: inputs I x 32 B, witness W x 32 B; returns the kernel time in ms if asked
 void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, uint32_t* status, float* kernel_ms) {
   Dev* d = dev(device);
+  if (plan.code.empty()) {            // an empty witness: no kernel, no set flagged
+    if (status) *status = 0;
+    if (kernel_ms) *kernel_ms = 0;
+    return;
+  }
   DeviceGuard on(device);
   std::lock_guard<std::mutex> lk(d->mu);
   if (!d->lat_in) {
