@@ -72,6 +72,8 @@ _L.gw_calc_witness_batch.argtypes = [_vp, _vp, _sz, _vp, _vp, ctypes.c_int, ctyp
 _L.gw_calc_witness_batch_on.argtypes = [_vp, ctypes.c_int, _vp, _sz, _vp, _vp, ctypes.c_int, ctypes.POINTER(gw_status_t)]
 _L.gw_calc_witness_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _vp, _vp, _vp, ctypes.POINTER(gw_status_t)]
 _L.gw_calc_witness_latency.argtypes = [_vp, ctypes.c_int, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(gw_status_t)]
+_L.gw_calc_witness_latency_batch.argtypes = [_vp, ctypes.c_int, ctypes.c_int, _vp, _sz, _vp, _vp, ctypes.POINTER(gw_status_t)]
+_L.gw_calc_witness_latency_batch_device.argtypes = [_vp, ctypes.c_int, _vp, _sz, _vp, _vp, _vp, ctypes.POINTER(gw_status_t)]
 _L.gw_wtns_header.argtypes = [ctypes.c_uint32, _vp]
 _L.gw_inputs_parse_batch.argtypes = [_vp, ctypes.c_char_p, _sz, ctypes.c_int, ctypes.POINTER(_vp), ctypes.POINTER(_sz), ctypes.POINTER(gw_status_t)]
 _L.gw_inputs_parse_batch_device.argtypes = [_vp, ctypes.c_int, ctypes.c_char_p, _sz, _vp, _sz, ctypes.POINTER(_sz), _vp,
@@ -107,7 +109,8 @@ EXPORTS = ["gw_calc_witness", "gw_graph_load", "gw_graph_free", "gw_graph_info",
            "gw_graph_select", "gw_calc_witness_batch_stream", "gw_set_device", "gw_r1cs_load", "gw_r1cs_free", "gw_r1cs_info",
            "gw_r1cs_check_batch", "gw_r1cs_check_batch_device", "gw_calc_witness_batch_check", "gw_r1cs_abc_len",
            "gw_r1cs_abc_batch", "gw_r1cs_abc_batch_device", "gw_fr_ntt_batch_device", "gw_r1cs_quotient_batch",
-           "gw_r1cs_quotient_batch_device", "gw_inputs_parse_batch_device"]
+           "gw_r1cs_quotient_batch_device", "gw_inputs_parse_batch_device", "gw_calc_witness_latency_batch",
+           "gw_calc_witness_latency_batch_device"]
 
 
 class WitnessCalcError(RuntimeError):
@@ -303,6 +306,28 @@ class Graph:
                                         ctypes.addressof(fl) if want_flags else None, ctypes.byref(ms), ctypes.byref(st))
         _check(rc, st)
         return (out, int(fl.value)) if want_flags else (out, float(ms.value))
+
+    def calc_witness_latency_batch(self, inputs: np.ndarray, n_gpus=1, first_device=0, want_flags=False):
+        """HOST buffers: inputs uint8 [B, I, 32] -> witness uint8 [B, W, 32], one latency-mode CTA per set; row r equals
+        calc_witness_latency(inputs[r]) (gw_calc_witness_latency_batch).  want_flags=True returns (witness, flags)."""
+        inputs = np.ascontiguousarray(inputs, dtype=np.uint8)
+        B = inputs.shape[0]
+        assert inputs.shape[1:] == (self.n_inputs, 32), inputs.shape
+        out = np.empty((B, self.n_witness, 32), dtype=np.uint8)
+        flags = np.zeros(B, dtype=np.uint32) if want_flags else None
+        st = gw_status_t()
+        rc = _L.gw_calc_witness_latency_batch(self._h, first_device, n_gpus, inputs.ctypes.data, B, out.ctypes.data,
+                                              flags.ctypes.data if want_flags else None, ctypes.byref(st))
+        _check(rc, st)
+        return (out, flags) if want_flags else out
+
+    def calc_witness_latency_batch_device(self, device, d_inputs_ptr, n_sets, d_witness_ptr, d_flags_ptr=None, stream=None):
+        """DEVICE pointers, one latency-mode CTA per set; ordered on `stream` (a cudaStream_t as int, None = default
+        stream); returns when the rows are complete (gw_calc_witness_latency_batch_device)."""
+        st = gw_status_t()
+        rc = _L.gw_calc_witness_latency_batch_device(self._h, device, d_inputs_ptr, n_sets, d_witness_ptr, d_flags_ptr,
+                                                     stream, ctypes.byref(st))
+        _check(rc, st)
 
     def calc_witness_batch_ptr(self, inputs_ptr, n_sets, witness_ptr, flags_ptr=None, n_gpus=1, first_device=0):
         """HOST pointers (e.g. pinned torch tensors): no allocation, no copies besides the DMA.  The sets are sharded

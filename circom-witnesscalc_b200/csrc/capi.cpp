@@ -201,6 +201,25 @@ int gw_calc_witness_latency(gw_graph_t* graph, int device, const uint8_t* inputs
   return guarded(status, [&]() { graph->engine->run_latency(device, inputs, witness, flags, kernel_ms); });
 }
 
+int gw_calc_witness_latency_batch(gw_graph_t* graph, int first_device, int n_gpus, const uint8_t* inputs, size_t n_sets,
+                                  uint8_t* witness, uint32_t* flags, gw_status_t* status) {
+  if (!graph || (n_sets && (!inputs || !witness))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() {
+    if (!n_sets) return;
+    int ndev = cuda_device_count();
+    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
+    if (n_gpus < 1) n_gpus = 1;
+    if (first_device < 0 || first_device + n_gpus > ndev) throw Error("device range exceeds the visible CUDA devices");
+    graph->engine->run_host(inputs, n_sets, witness, flags, n_gpus, first_device, 0, nullptr, nullptr, true);
+  });
+}
+
+int gw_calc_witness_latency_batch_device(gw_graph_t* graph, int device, const void* d_inputs, size_t n_sets, void* d_witness,
+                                         uint32_t* d_flags, void* cuda_stream, gw_status_t* status) {
+  if (!graph || (n_sets && (!d_inputs || !d_witness))) { set_status(status, ERROR, "null argument"); return 1; }
+  return guarded(status, [&]() { graph->engine->run_latency_device(device, d_inputs, n_sets, d_witness, d_flags, cuda_stream); });
+}
+
 int gw_inputs_parse_batch(const gw_graph_t* graph, const char* text, size_t text_len, int n_threads, uint8_t** inputs,
                           size_t* n_sets, gw_status_t* status) {
   if (!graph || !text || !inputs || !n_sets) { set_status(status, ERROR, "null argument"); return 1; }

@@ -529,6 +529,8 @@ struct LParams {
   uint32_t n_slots;
   uint32_t dbg;            // GW_LAT_DBG, timing experiments only: 1 = no witness stores, 16 = no instructions (level skeleton alone)
   unsigned long long* level_clock;   // profiling aid (GW_LAT_CLOCKS): clock64 at the end of every level, or null
+  // batch form (BATCH = true): CTA b evaluates input set row_map ? row_map[b] : b; inputs [.][I][2], out [.][W][2], status [.]
+  const uint32_t* row_map; uint32_t I, W;
 };
 
 static const int LAT_MAX_THREADS = 384;     // main + control + slow warps <= 12: 170 registers per thread
@@ -681,19 +683,31 @@ __device__ __forceinline__ void lat_exec_slow(const LatCtx& cx, const uint4* pk,
   if ((ins.x & F_OUT) && op != OP_TERN) { cx.out[2 * (size_t)ins.w] = fe_lo(R); cx.out[2 * (size_t)ins.w + 1] = fe_hi(R); }
 }
 
+// the input set of a latency CTA: 0 for the single-set kernels, row_map[b] or b for CTA b of a batch launch (CTAs of
+// different sets share nothing but the read-only plan)
+template <bool BATCH, typename P> __device__ __forceinline__ unsigned long long lat_set(const P& p) {
+  if (!BATCH) return 0ull;
+  return p.row_map ? (unsigned long long)__ldg(p.row_map + blockIdx.x) : (unsigned long long)blockIdx.x;
+}
+
 // Dynamic shared memory: [LAT_CTRL_BYTES: control words + mbarriers][n_slots][2] value file | [n_warps][3][LAT_RING_SLOTS] packet rings
+template <bool BATCH>
 __global__ void __launch_bounds__(LAT_MAX_THREADS) eval_latency_kernel(const LParams p) {
   extern __shared__ uint4 lat_smem[];
   volatile uint32_t* ctrl = reinterpret_cast<volatile uint32_t*>(lat_smem);   // [0] = completed levels, [1 + w] = jobs done by slow warp w
   const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
   const uint32_t smem_s = (uint32_t)__cvta_generic_to_shared(lat_smem);
+  const unsigned long long set = lat_set<BATCH>(p);
+  uint32_t* const status = (BATCH && p.status) ? p.status + set : p.status;
+  if (BATCH && tid == 0 && status) *status = 0;                  // this set's flag word (the single call clears it on the host)
   if (tid < 8) ctrl[tid] = 0;
   if (tid < 3u * p.n_warps) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_s + 32u + 8u * tid) : "memory");
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   __syncthreads();
   uint32_t st = 0;
   LatCtx cx;
-  cx.inputs = p.inputs; cx.out = p.out; cx.slots_s = smem_s + LAT_CTRL_BYTES; cx.dbg = p.dbg;
+  cx.inputs = BATCH ? p.inputs + set * p.I * 2 : p.inputs; cx.out = BATCH ? p.out + set * p.W * 2 : p.out;
+  cx.slots_s = smem_s + LAT_CTRL_BYTES; cx.dbg = p.dbg;
 
   // Packets reach the rings by TMA: ONE bulk copy (cp.async.bulk) per packet, issued by the CONTROL warp (lane w serves
   // main warp w), completing on the mbarrier of the ring stage; the main warps only wait for their barrier, so neither
@@ -774,7 +788,7 @@ __global__ void __launch_bounds__(LAT_MAX_THREADS) eval_latency_kernel(const LPa
       if (lane == 0) flag_publish(smem_s + 4u * (1u + ws), j + 1);
     }
   }
-  if (p.status != nullptr && st) atomicOr(p.status, st);
+  if (status != nullptr && st) atomicOr(status, st);
 }
 
 // ---- single-witness latency mode, dataflow plan (plan.hpp: LatencyPlan::dataflow) -----------------------------------
@@ -791,16 +805,25 @@ struct DParams {
   uint32_t dbg;            // GW_LAT_DBG, -DGW_PROFILING experiments: 1 = no witness stores, 2 = publish without fence / atomic, 4 = poll with plain
                            // volatile loads, 8 = fault injection: warp 1's first wait can never be satisfied (watchdog test)
   unsigned long long* clocks; uint32_t clock_rows;   // profiling aid (GW_LAT_CLOCKS, -DGW_PROFILING): [warp][row]{start, after wait, end, first opcode}
+  // batch form (BATCH = true): CTA b evaluates input set row_map ? row_map[b] : b; inputs [.][I][2], out [.][W][2], status [.];
+  // a CTA whose watchdog fired also sets `aborted` (one word for the launch: the caller's flags are optional)
+  const uint32_t* row_map; uint32_t I, W; uint32_t* aborted;
 };
 static const uint32_t DF_ABORT_WORD = 15;              // control word 15: set by a warp whose wait ran into the watchdog; everybody leaves
 static const uint32_t DF_WATCHDOG_SPINS = 1u << 28;    // polls of one wait (tens of seconds: the longest real wait is a Pow, < 1 ms)
 static const uint32_t DF_CTRL_BYTES = 384;  // 16 progress words (64 B) + 3 mbarriers x up to 12 warps (288 B), 16 B aligned
+// (the "latency plan:" prefix makes gw_calc_witness fall back to the throughput kernel, capi.cpp)
+static const char* const LAT_WATCHDOG_ERROR = "latency plan: a packet waited for progress that never came (watchdog); please report the graph";
 
+template <bool BATCH>
 __global__ void __launch_bounds__(LAT_MAX_THREADS) eval_dataflow_kernel(const DParams p) {
   extern __shared__ uint4 lat_smem[];
   const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = __shfl_sync(0xFFFFFFFFu, tid >> 5, 0);   // warp-uniform for the compiler too
   const uint32_t smem_s = (uint32_t)__cvta_generic_to_shared(lat_smem);
   const uint32_t bar0_s = smem_s + 64u;
+  const unsigned long long set = lat_set<BATCH>(p);
+  uint32_t* const status = (BATCH && p.status) ? p.status + set : p.status;
+  if (BATCH && tid == 0 && status) *status = 0;                  // this set's flag word (the single call clears it on the host)
   if (tid < 16) reinterpret_cast<volatile uint32_t*>(lat_smem)[tid] = 0;
   if (tid < 3u * p.n_warps) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0_s + 8u * tid) : "memory");
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -808,7 +831,8 @@ __global__ void __launch_bounds__(LAT_MAX_THREADS) eval_dataflow_kernel(const DP
   if (warp >= p.n_warps) return;
   uint32_t st = 0;
   LatCtx cx;
-  cx.inputs = p.inputs; cx.out = p.out; cx.slots_s = smem_s + DF_CTRL_BYTES; cx.dbg = p.dbg;
+  cx.inputs = BATCH ? p.inputs + set * p.I * 2 : p.inputs; cx.out = BATCH ? p.out + set * p.W * 2 : p.out;
+  cx.slots_s = smem_s + DF_CTRL_BYTES; cx.dbg = p.dbg;
   const uint32_t chunk_bytes = p.chunk_slots * 16u;
   const uint32_t ring_s = cx.slots_s + 32u * p.n_slots + warp * 3u * chunk_bytes;
   const uint32_t n_chunks = __ldg(p.stream_chunks + warp);
@@ -864,7 +888,8 @@ __global__ void __launch_bounds__(LAT_MAX_THREADS) eval_dataflow_kernel(const DP
         __threadfence_block();                    // acquire: the value-file loads below come after the counters were seen
         __syncwarp();
         if (flag_read(smem_s + 4u * DF_ABORT_WORD) != 0u) {       // warp-uniform: read after the __syncwarp
-          if (lane == 0 && p.status != nullptr) atomicOr(p.status, 0x80000000u);
+          if (lane == 0 && status != nullptr) atomicOr(status, 0x80000000u);
+          if (BATCH && lane == 0) atomicOr(p.aborted, 1u);
           return;
         }
       }
@@ -890,7 +915,7 @@ __global__ void __launch_bounds__(LAT_MAX_THREADS) eval_dataflow_kernel(const DP
       pk_s += 16u * desc.x;
     }
   }
-  if (p.status != nullptr && st) atomicOr(p.status, st);
+  if (status != nullptr && st) atomicOr(status, st);
 }
 
 // ---- integer-pipe microbenchmark (roofline denominator for multiplication-heavy graphs) ---------
@@ -997,6 +1022,7 @@ struct Engine::Dev {
   uint4* lat_code = nullptr; uint4* lat_first = nullptr; uint4* lat_jobs = nullptr; uint32_t* lat_njobs = nullptr; uint4* lat_waits = nullptr;
   unsigned long long* lat_clock = nullptr;
   uint4* lat_in = nullptr; uint4* lat_out = nullptr; uint32_t* lat_status = nullptr;
+  uint32_t* lat_aborted = nullptr;       // latency batch calls: set by a CTA whose watchdog fired (DParams::aborted)
   std::mutex mu;
 };
 
@@ -1091,7 +1117,7 @@ Engine::~Engine() {
     cudaFree(d->bit_planes); cudaFree(d->bit_ok); cudaFree(d->bit_bad); cudaFree(d->bit_nbad);
     cudaFreeHost(d->bit_nbad_host); if (d->bit_nbad_ev) cudaEventDestroy(d->bit_nbad_ev);
     cudaFree(d->lat_soff); cudaFree(d->lat_schunks);
-    cudaFree(d->lat_code); cudaFree(d->lat_first); cudaFree(d->lat_jobs); cudaFree(d->lat_njobs); cudaFree(d->lat_waits); cudaFree(d->lat_clock); cudaFree(d->lat_in); cudaFree(d->lat_out); cudaFree(d->lat_status);
+    cudaFree(d->lat_code); cudaFree(d->lat_first); cudaFree(d->lat_jobs); cudaFree(d->lat_njobs); cudaFree(d->lat_waits); cudaFree(d->lat_clock); cudaFree(d->lat_in); cudaFree(d->lat_out); cudaFree(d->lat_status); cudaFree(d->lat_aborted);
     for (int i = 0; i < 2; i++) { cudaFree(d->d_in[i]); cudaFree(d->d_out[i]); cudaFree(d->d_status[i]); cudaFree(d->d_ff[i]); if (d->stream[i]) cudaStreamDestroy(d->stream[i]); }
     for (int i = 0; i < 3; i++) { cudaFreeHost(d->h_ring[i]); cudaFreeHost(d->h_flags[i]); }
     if (d->last_kernel) cudaEventDestroy(d->last_kernel);
@@ -1120,8 +1146,13 @@ Engine::Dev* Engine::dev(int device) {
   if (t_max < 32) throw Error("register file does not fit shared memory: lower GW_REGS");
   d->max_threads = t_max;
   CUDA_CHECK(cudaFuncSetAttribute(eval_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));
-  CUDA_CHECK(cudaFuncSetAttribute(eval_dataflow_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));
-  CUDA_CHECK(cudaFuncSetAttribute(eval_latency_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));   // per device, not per graph
+  CUDA_CHECK(cudaFuncSetAttribute(eval_dataflow_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));
+  CUDA_CHECK(cudaFuncSetAttribute(eval_latency_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));   // per device, not per graph
+  // batch forms: as many CTAs per SM as shared memory holds (two of a small graph), so the carveout goes to shared memory
+  CUDA_CHECK(cudaFuncSetAttribute(eval_dataflow_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));
+  CUDA_CHECK(cudaFuncSetAttribute(eval_latency_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)d->smem_max));
+  CUDA_CHECK(cudaFuncSetAttribute(eval_dataflow_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+  CUDA_CHECK(cudaFuncSetAttribute(eval_latency_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
   CUDA_CHECK(cudaEventCreateWithFlags(&d->last_kernel, cudaEventDisableTiming));
   CUDA_CHECK(cudaMalloc(&d->code, plan.code.size() * sizeof(Instr)));
   CUDA_CHECK(cudaMemcpy(d->code, plan.code.data(), plan.code.size() * sizeof(Instr), cudaMemcpyHostToDevice));
@@ -1344,9 +1375,9 @@ struct StreamDrain {
 };
 }  // namespace
 
-// host buffers: chunked, double-buffered H2D -> kernel -> D2H on two streams
+// host buffers: chunked, double-buffered H2D -> kernel -> D2H on two streams (latency: the latency kernels, one CTA per set)
 void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, size_t out_pitch,
-                         R1cs* check, uint32_t* first_failed) {
+                         R1cs* check, uint32_t* first_failed, bool latency) {
   Dev* d = dev(device);
   DeviceGuard on(device);
   std::lock_guard<std::mutex> lk(d->mu);
@@ -1360,8 +1391,16 @@ void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* w
   CUDA_CHECK(cudaMemGetInfo(&free_b, &total_b));
   size_t budget = (size_t)env_int("GW_CHUNK_MB", 24576) << 20;
   budget = std::min(budget, (free_b + 2 * d->chunk * (in_b + out_b)) / 5);
-  size_t chunk = std::min<size_t>(budget / std::max<size_t>(out_b + in_b, 1), 2 * d->spill_threads);
-  if (B >= 4 * 2048) chunk = std::min(chunk, (B + 3) / 4);
+  size_t chunk = budget / std::max<size_t>(out_b + in_b, 1);
+  if (latency) {
+    // latency kernels: whole waves of resident CTAs (what the budget holds if that is less than one wave)
+    const size_t wave = latency_wave(d);
+    if (chunk >= wave) chunk = chunk / wave * wave;
+    if (B >= 4 * wave) chunk = std::min(chunk, ((B + 3) / 4 + wave - 1) / wave * wave);
+  } else {
+    chunk = std::min<size_t>(chunk, 2 * d->spill_threads);
+    if (B >= 4 * 2048) chunk = std::min(chunk, (B + 3) / 4);
+  }
   chunk = std::max<size_t>(std::min(chunk, B), 1);
   ensure_staging(d, chunk);
   if (check)                                   // verdict buffers of the staging chunk size, allocated on the first check
@@ -1370,6 +1409,7 @@ void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* w
   // of the two streams overlap with them.
   HostTrace tr;
   StreamDrain drain{d->stream[0], d->stream[1]};
+  if (latency) { latency_arm(d, d->stream[0]); CUDA_CHECK(cudaStreamSynchronize(d->stream[0])); }
   int k = 0;
   for (size_t off = 0; off < B; off += chunk, k ^= 1) {
     size_t nb = std::min(chunk, B - off);
@@ -1377,7 +1417,8 @@ void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* w
     tr.mark(s);
     CUDA_CHECK(cudaMemcpyAsync(d->d_in[k], inputs + off * in_b, nb * in_b, cudaMemcpyHostToDevice, s));
     tr.mark(s);
-    launch(d, d->d_in[k], nb, d->d_out[k], status ? d->d_status[k] : nullptr, s);
+    if (latency) latency_launch(d, d->d_in[k], nb, d->d_out[k], status ? d->d_status[k] : nullptr, s);
+    else launch(d, d->d_in[k], nb, d->d_out[k], status ? d->d_status[k] : nullptr, s);
     if (check) {
       // the chunk's witness rows are checked where they are; only the verdicts have to cross PCIe
       check->check_device(device, d->d_out[k], nb, out_b, d->d_ff[k], s);
@@ -1392,14 +1433,15 @@ void Engine::run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* w
   }
   CUDA_CHECK(cudaStreamSynchronize(d->stream[0]));
   CUDA_CHECK(cudaStreamSynchronize(d->stream[1]));
+  if (latency) latency_check(d);
   tr.print(device, B, chunk);
 }
 
 void Engine::run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, int n_gpus, int first_device, size_t out_pitch,
-                      R1cs* check, uint32_t* first_failed) {
+                      R1cs* check, uint32_t* first_failed, bool latency) {
   if (B == 0) return;
   if (out_pitch == 0) out_pitch = (size_t)plan.n_witness * 32;
-  if (n_gpus <= 1) { run_host_on(first_device, inputs, B, witness, status, out_pitch, check, first_failed); return; }
+  if (n_gpus <= 1) { run_host_on(first_device, inputs, B, witness, status, out_pitch, check, first_failed, latency); return; }
   // independent input sets: contiguous shards, one host thread per GPU (pinned to the GPU's NUMA node), no collective
   const size_t in_b = (size_t)plan.n_inputs * 32;
   std::vector<std::thread> th;
@@ -1411,7 +1453,7 @@ void Engine::run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_
       try {
         bind_thread_near_device(first_device + g);
         run_host_on(first_device + g, inputs + lo * in_b, hi - lo, witness ? witness + lo * out_pitch : nullptr, status ? status + lo : nullptr,
-                    out_pitch, check, check ? first_failed + lo : nullptr);
+                    out_pitch, check, check ? first_failed + lo : nullptr, latency);
       } catch (const std::exception& e) { errs[g] = e.what(); }
     });
   }
@@ -1502,6 +1544,74 @@ void Engine::run_stream(const uint8_t* inputs, size_t B, int n_gpus, int first_d
   for (auto& e : errs) if (!e.empty()) throw Error(e);
 }
 
+// shared memory of one latency CTA of plan lp (engine.cu: eval_dataflow_kernel, eval_latency_kernel)
+static size_t latency_smem(const LatencyPlan& lp) {
+  if (lp.dataflow) return DF_CTRL_BYTES + (size_t)lp.n_slots * 32 + (size_t)lp.n_phys_warps * 3 * lp.chunk_slots * 16;
+  return ((size_t)lp.n_slots * 2 + LAT_CTRL_BYTES / 16 + (size_t)lp.n_warps * 3 * LAT_RING_SLOTS) * 16;
+}
+static int latency_threads(const LatencyPlan& lp) { return (int)(lp.dataflow ? lp.n_phys_warps : lp.n_warps + 1 + lp.n_slow_warps) * 32; }
+
+// The latency plan of the graph and its tables on d's device, for the single call and the batch alike: compiled once, under
+// the GW_LAT_* options of that moment (a compile error -- "graph is too wide" -- is remembered and given to every later
+// call), uploaded once per device.  Callers hold d->mu.
+const LatencyPlan& Engine::latency_plan(Dev* d) {
+  {
+    std::lock_guard<std::mutex> lk2(mu);
+    if (!lat_error.empty()) throw Error(lat_error);
+    if (!lat_ready) {
+      LatencyOptions lo;
+      // GW_LAT_MODE=level: the level-synchronous plan (control warp, CTA barrier per level); default: the dataflow plan
+      const char* lat_mode = getenv("GW_LAT_MODE");
+      lo.dataflow = !(lat_mode && strcmp(lat_mode, "level") == 0);
+      // dataflow: no control warp
+      // (measured on authV2, profiles/r02o: 6 + 3 warps 16.3 ms, 7 + 3: 16.9, 8 + 4: 17.6, 7 + 3 with warp 0 alone on its
+      // sub-partition: 18.1 -- every extra warp of dependent carry chains slows its sub-partition's other warps down)
+      lo.n_warps = (uint32_t)env_int("GW_LAT_WARPS", lo.dataflow ? 6 : (int)lo.n_warps);
+      lo.n_slow_warps = (uint32_t)env_int("GW_LAT_SLOW_WARPS", lo.dataflow ? 3 : (int)lo.n_slow_warps);
+      lo.exclusive_warp0 = env_int("GW_LAT_EXCL", 0) != 0;
+      lo.packet_slots = LAT_RING_SLOTS;
+      const size_t df_rings = std::min<size_t>(12, lo.n_warps + lo.n_slow_warps + (lo.exclusive_warp0 ? 2 : 0));     // physical warps, empty ones included
+      if (lo.dataflow) lo.max_slots = (uint32_t)std::min<size_t>((d->smem_max / 16 - DF_CTRL_BYTES / 16 - df_rings * 3 * LAT_RING_SLOTS) / 2, 0xFFFF);
+      else
+      lo.max_slots = (uint32_t)std::min<size_t>((d->smem_max / 16 - LAT_CTRL_BYTES / 16 - (size_t)lo.n_warps * 3 * LAT_RING_SLOTS) / 2, 0xFFFF);
+      lo.slow_levels = (uint32_t)env_int("GW_LAT_D", 0);
+      lo.split_dot = env_int("GW_LAT_SPLIT", 1) != 0;
+      lo.fuse = env_int("GW_LAT_FUSE", 1) != 0;
+      lo.sbox_links = env_int("GW_LAT_LINKS", 1) != 0;           // 0: never, 1: where the timing model prefers it, 2: always
+      lo.force_sbox_links = env_int("GW_LAT_LINKS", 1) == 2;
+      lo.chain = env_int("GW_LAT_CHAIN", 1) != 0;
+      if (!lo.dataflow && (lo.n_warps + 1 + lo.n_slow_warps) * 32 > (uint32_t)LAT_MAX_THREADS) throw Error("GW_LAT_WARPS + GW_LAT_SLOW_WARPS must not exceed 11");
+      try { lat_plan = compile_latency_plan(graph, lo); }
+      catch (const Error& e) { lat_error = e.what(); throw; }
+      lat_ready = true;
+    }
+  }
+  const LatencyPlan& lp = lat_plan;
+  if (!d->lat_code) {
+    CUDA_CHECK(cudaMalloc(&d->lat_code, std::max<size_t>(lp.code.size(), 1) * sizeof(Instr)));
+    CUDA_CHECK(cudaMemcpy(d->lat_code, lp.code.data(), lp.code.size() * sizeof(Instr), cudaMemcpyHostToDevice));
+    if (lp.dataflow) {
+      const uint32_t NW = lp.n_phys_warps;
+      CUDA_CHECK(cudaMalloc(&d->lat_soff, NW * 4)); CUDA_CHECK(cudaMalloc(&d->lat_schunks, NW * 4));
+      CUDA_CHECK(cudaMemcpy(d->lat_soff, lp.stream_off.data(), NW * 4, cudaMemcpyHostToDevice));
+      CUDA_CHECK(cudaMemcpy(d->lat_schunks, lp.stream_chunks.data(), NW * 4, cudaMemcpyHostToDevice));
+    } else {
+      CUDA_CHECK(cudaMalloc(&d->lat_first, std::max<size_t>(lp.first.size(), 4) * 4));
+      CUDA_CHECK(cudaMemcpy(d->lat_first, lp.first.data(), lp.first.size() * 4, cudaMemcpyHostToDevice));
+      CUDA_CHECK(cudaMalloc(&d->lat_jobs, std::max<size_t>(lp.jobs.size(), 4) * 4));
+      CUDA_CHECK(cudaMemcpy(d->lat_jobs, lp.jobs.data(), lp.jobs.size() * 4, cudaMemcpyHostToDevice));
+      CUDA_CHECK(cudaMalloc(&d->lat_njobs, std::max<size_t>(lp.n_jobs.size(), 1) * 4));
+      CUDA_CHECK(cudaMemcpy(d->lat_njobs, lp.n_jobs.data(), lp.n_jobs.size() * 4, cudaMemcpyHostToDevice));
+      CUDA_CHECK(cudaMalloc(&d->lat_waits, std::max<size_t>(lp.waits.size(), 4) * 4));
+      CUDA_CHECK(cudaMemcpy(d->lat_waits, lp.waits.data(), lp.waits.size() * 4, cudaMemcpyHostToDevice));
+#ifdef GW_PROFILING
+      if (env_int("GW_LAT_CLOCKS", 0) != 0) CUDA_CHECK(cudaMalloc(&d->lat_clock, ((size_t)lp.n_levels + 1) * 8));
+#endif
+    }
+  }
+  return lp;
+}
+
 // one witness, host buffers: inputs I x 32 B, witness W x 32 B; returns the kernel time in ms if asked
 void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, uint32_t* status, float* kernel_ms) {
   Dev* d = dev(device);
@@ -1537,53 +1647,15 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
       return;
     }
   }
-  {
-    std::lock_guard<std::mutex> lk2(mu);
-    if (!lat_error.empty()) throw Error(lat_error);
-    if (!lat_ready) {
-      cudaDeviceProp prop; CUDA_CHECK(cudaGetDeviceProperties(&prop, device));
-      LatencyOptions lo;
-      // GW_LAT_MODE=level: the level-synchronous plan (control warp, CTA barrier per level); default: the dataflow plan
-      const char* lat_mode = getenv("GW_LAT_MODE");
-      lo.dataflow = !(lat_mode && strcmp(lat_mode, "level") == 0);
-      // dataflow: no control warp
-      // (measured on authV2, profiles/r02o: 6 + 3 warps 16.3 ms, 7 + 3: 16.9, 8 + 4: 17.6, 7 + 3 with warp 0 alone on its
-      // sub-partition: 18.1 -- every extra warp of dependent carry chains slows its sub-partition's other warps down)
-      lo.n_warps = (uint32_t)env_int("GW_LAT_WARPS", lo.dataflow ? 6 : (int)lo.n_warps);
-      lo.n_slow_warps = (uint32_t)env_int("GW_LAT_SLOW_WARPS", lo.dataflow ? 3 : (int)lo.n_slow_warps);
-      lo.exclusive_warp0 = env_int("GW_LAT_EXCL", 0) != 0;
-      lo.packet_slots = LAT_RING_SLOTS;
-      const size_t df_rings = std::min<size_t>(12, lo.n_warps + lo.n_slow_warps + (lo.exclusive_warp0 ? 2 : 0));     // physical warps, empty ones included
-      if (lo.dataflow) lo.max_slots = (uint32_t)std::min<size_t>((prop.sharedMemPerBlockOptin / 16 - DF_CTRL_BYTES / 16 - df_rings * 3 * LAT_RING_SLOTS) / 2, 0xFFFF);
-      else
-      lo.max_slots = (uint32_t)std::min<size_t>((prop.sharedMemPerBlockOptin / 16 - LAT_CTRL_BYTES / 16 - (size_t)lo.n_warps * 3 * LAT_RING_SLOTS) / 2, 0xFFFF);
-      lo.slow_levels = (uint32_t)env_int("GW_LAT_D", 0);
-      lo.split_dot = env_int("GW_LAT_SPLIT", 1) != 0;
-      lo.fuse = env_int("GW_LAT_FUSE", 1) != 0;
-      lo.sbox_links = env_int("GW_LAT_LINKS", 1) != 0;           // 0: never, 1: where the timing model prefers it, 2: always
-      lo.force_sbox_links = env_int("GW_LAT_LINKS", 1) == 2;
-      lo.chain = env_int("GW_LAT_CHAIN", 1) != 0;
-      if (!lo.dataflow && (lo.n_warps + 1 + lo.n_slow_warps) * 32 > (uint32_t)LAT_MAX_THREADS) throw Error("GW_LAT_WARPS + GW_LAT_SLOW_WARPS must not exceed 11");
-      try { lat_plan = compile_latency_plan(graph, lo); }
-      catch (const Error& e) { lat_error = e.what(); throw; }
-      lat_ready = true;
-    }
-  }
-  const LatencyPlan& lp = lat_plan;
+  const LatencyPlan& lp = latency_plan(d);
   const size_t in_b = (size_t)lp.n_inputs * 32;
   if (lp.dataflow) {
     const uint32_t NW = lp.n_phys_warps;
-    if (!d->lat_code) {
-      CUDA_CHECK(cudaMalloc(&d->lat_code, std::max<size_t>(lp.code.size(), 1) * sizeof(Instr)));
-      CUDA_CHECK(cudaMemcpy(d->lat_code, lp.code.data(), lp.code.size() * sizeof(Instr), cudaMemcpyHostToDevice));
-      CUDA_CHECK(cudaMalloc(&d->lat_soff, NW * 4)); CUDA_CHECK(cudaMalloc(&d->lat_schunks, NW * 4));
-      CUDA_CHECK(cudaMemcpy(d->lat_soff, lp.stream_off.data(), NW * 4, cudaMemcpyHostToDevice));
-      CUDA_CHECK(cudaMemcpy(d->lat_schunks, lp.stream_chunks.data(), NW * 4, cudaMemcpyHostToDevice));
-    }
     DParams q;
     q.code = d->lat_code; q.stream_off = d->lat_soff; q.stream_chunks = d->lat_schunks; q.n_warps = NW; q.chunk_slots = lp.chunk_slots;
     q.inputs = d->lat_in; q.out = d->lat_out; q.status = d->lat_status; q.n_slots = lp.n_slots;
-    const size_t smem_df = DF_CTRL_BYTES + (size_t)lp.n_slots * 32 + (size_t)NW * 3 * lp.chunk_slots * 16;
+    q.row_map = nullptr; q.I = q.W = 0; q.aborted = nullptr;
+    const size_t smem_df = latency_smem(lp);
     q.clocks = nullptr; q.clock_rows = 0; q.dbg = 0;
     q.watchdog = (uint32_t)env_int("GW_LAT_WATCHDOG", (int)DF_WATCHDOG_SPINS);
 #ifdef GW_PROFILING
@@ -1604,7 +1676,7 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
     CUDA_CHECK(cudaMemsetAsync(d->lat_status, 0, 4, 0));
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (kernel_ms) { CUDA_CHECK(cudaEventCreate(&e0)); CUDA_CHECK(cudaEventCreate(&e1)); CUDA_CHECK(cudaEventRecord(e0, 0)); }
-    eval_dataflow_kernel<<<1, NW * 32, smem_df, 0>>>(q);
+    eval_dataflow_kernel<false><<<1, NW * 32, smem_df, 0>>>(q);
     CUDA_CHECK(cudaGetLastError());
     if (kernel_ms) CUDA_CHECK(cudaEventRecord(e1, 0));
     uint32_t h_status = 0;
@@ -1613,7 +1685,7 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
     CUDA_CHECK(cudaStreamSynchronize(0));
     if (kernel_ms) { CUDA_CHECK(cudaEventElapsedTime(kernel_ms, e0, e1)); cudaEventDestroy(e0); cudaEventDestroy(e1); }
     // (the "latency plan:" prefix makes gw_calc_witness fall back to the throughput kernel, capi.cpp)
-    if (h_status & 0x80000000u) throw Error("latency plan: a packet waited for progress that never came (watchdog); please report the graph");
+    if (h_status & 0x80000000u) throw Error(LAT_WATCHDOG_ERROR);
     if (status) *status = h_status;
 #ifdef GW_PROFILING
     if (d_clk) {
@@ -1638,25 +1710,12 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
 #endif
     return;
   }
-  const size_t smem = ((size_t)lp.n_slots * 2 + LAT_CTRL_BYTES / 16 + (size_t)lp.n_warps * 3 * LAT_RING_SLOTS) * 16;
+  const size_t smem = latency_smem(lp);
 #ifdef GW_PROFILING
   const bool clocks = env_int("GW_LAT_CLOCKS", 0) != 0;
 #else
   const bool clocks = false;
 #endif
-  if (!d->lat_code) {
-    CUDA_CHECK(cudaMalloc(&d->lat_code, std::max<size_t>(lp.code.size(), 1) * sizeof(Instr)));
-    CUDA_CHECK(cudaMemcpy(d->lat_code, lp.code.data(), lp.code.size() * sizeof(Instr), cudaMemcpyHostToDevice));
-    CUDA_CHECK(cudaMalloc(&d->lat_first, std::max<size_t>(lp.first.size(), 4) * 4));
-    CUDA_CHECK(cudaMemcpy(d->lat_first, lp.first.data(), lp.first.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_CHECK(cudaMalloc(&d->lat_jobs, std::max<size_t>(lp.jobs.size(), 4) * 4));
-    CUDA_CHECK(cudaMemcpy(d->lat_jobs, lp.jobs.data(), lp.jobs.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_CHECK(cudaMalloc(&d->lat_njobs, std::max<size_t>(lp.n_jobs.size(), 1) * 4));
-    CUDA_CHECK(cudaMemcpy(d->lat_njobs, lp.n_jobs.data(), lp.n_jobs.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_CHECK(cudaMalloc(&d->lat_waits, std::max<size_t>(lp.waits.size(), 4) * 4));
-    CUDA_CHECK(cudaMemcpy(d->lat_waits, lp.waits.data(), lp.waits.size() * 4, cudaMemcpyHostToDevice));
-    if (clocks) CUDA_CHECK(cudaMalloc(&d->lat_clock, ((size_t)lp.n_levels + 1) * 8));
-  }
   if (lp.n_levels == 0) return;
   LParams p;
   p.code = d->lat_code; p.first = d->lat_first; p.n_levels = lp.n_levels; p.n_warps = lp.n_warps; p.n_slots = lp.n_slots;
@@ -1664,6 +1723,7 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
   p.waits = d->lat_waits; p.n_waits = (uint32_t)(lp.waits.size() / 4);
   p.inputs = d->lat_in; p.out = d->lat_out; p.status = status ? d->lat_status : nullptr;
   p.level_clock = d->lat_clock;
+  p.row_map = nullptr; p.I = p.W = 0;
   p.dbg = 0;
 #ifdef GW_PROFILING
   p.dbg = (uint32_t)env_int("GW_LAT_DBG", 0);      // timing experiments: -DGW_PROFILING builds only
@@ -1672,7 +1732,7 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
   if (status) CUDA_CHECK(cudaMemsetAsync(d->lat_status, 0, 4, 0));
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (kernel_ms) { CUDA_CHECK(cudaEventCreate(&e0)); CUDA_CHECK(cudaEventCreate(&e1)); CUDA_CHECK(cudaEventRecord(e0, 0)); }
-  eval_latency_kernel<<<1, (lp.n_warps + 1 + lp.n_slow_warps) * 32, smem, 0>>>(p);
+  eval_latency_kernel<false><<<1, (lp.n_warps + 1 + lp.n_slow_warps) * 32, smem, 0>>>(p);
   CUDA_CHECK(cudaGetLastError());
   if (kernel_ms) CUDA_CHECK(cudaEventRecord(e1, 0));
   CUDA_CHECK(cudaMemcpyAsync(witness, d->lat_out, (size_t)lp.n_witness * 32, cudaMemcpyDeviceToHost, 0));
@@ -1690,6 +1750,95 @@ void Engine::run_latency(int device, const uint8_t* inputs, uint8_t* witness, ui
       fclose(f);
     }
   }
+}
+
+// Boolean graphs take the bit-sliced plan in latency mode, as the single call decides (Engine::run_latency)
+bool Engine::latency_bit(Dev* d) const { return d->bit_fits && bit_path_active() && bit_plan.n_luts > 0 && env_int("GW_LAT_BIT", 1) != 0; }
+
+// input sets one wave of latency_launch holds on d's device: one CTA per set, as many per SM as registers and shared
+// memory allow (the bit-sliced plan: 32 sets per warp, a warp per SM and wave at least)
+size_t Engine::latency_wave(Dev* d) {
+  if (latency_bit(d)) return (size_t)d->sms * 32;
+  const LatencyPlan& lp = latency_plan(d);
+  int per_sm = 0;
+  if (lp.dataflow) CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eval_dataflow_kernel<true>, latency_threads(lp), latency_smem(lp)));
+  else CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, eval_latency_kernel<true>, latency_threads(lp), latency_smem(lp)));
+  return (size_t)d->sms * (size_t)std::max(per_sm, 1);
+}
+
+// n input sets, one latency CTA each: CTA b evaluates set row_map ? row_map[b] : b of d_inputs / d_witness / d_status.
+// Chained behind every earlier launch of this engine on the device, as launch() is.  Callers hold d->mu.
+void Engine::latency_kernels(Dev* d, const void* d_inputs, size_t n, const uint32_t* row_map, void* d_witness, uint32_t* d_status, void* stream) {
+  const LatencyPlan& lp = latency_plan(d);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (n > 0x7FFFFFFFull) throw Error("batch too large");
+  CUDA_CHECK(cudaStreamWaitEvent(s, d->last_kernel, 0));
+  if (lp.dataflow) {
+    DParams q;
+    q.code = d->lat_code; q.stream_off = d->lat_soff; q.stream_chunks = d->lat_schunks; q.n_warps = lp.n_phys_warps; q.chunk_slots = lp.chunk_slots;
+    q.inputs = (const uint4*)d_inputs; q.out = (uint4*)d_witness; q.status = d_status; q.n_slots = lp.n_slots;
+    q.watchdog = (uint32_t)env_int("GW_LAT_WATCHDOG", (int)DF_WATCHDOG_SPINS);
+    q.dbg = 0; q.clocks = nullptr; q.clock_rows = 0;
+    q.row_map = row_map; q.I = lp.n_inputs; q.W = lp.n_witness; q.aborted = d->lat_aborted;
+    eval_dataflow_kernel<true><<<(unsigned)n, latency_threads(lp), latency_smem(lp), s>>>(q);
+  } else {
+    LParams p;
+    p.code = d->lat_code; p.first = d->lat_first; p.n_levels = lp.n_levels; p.n_warps = lp.n_warps; p.n_slots = lp.n_slots;
+    p.jobs = d->lat_jobs; p.n_jobs = d->lat_njobs; p.max_jobs = lp.max_jobs; p.n_slow = lp.n_slow_warps;
+    p.waits = d->lat_waits; p.n_waits = (uint32_t)(lp.waits.size() / 4);
+    p.inputs = (const uint4*)d_inputs; p.out = (uint4*)d_witness; p.status = d_status;
+    p.level_clock = nullptr; p.dbg = 0;
+    p.row_map = row_map; p.I = lp.n_inputs; p.W = lp.n_witness;
+    eval_latency_kernel<true><<<(unsigned)n, latency_threads(lp), latency_smem(lp), s>>>(p);
+  }
+  CUDA_CHECK(cudaGetLastError());
+  CUDA_CHECK(cudaEventRecord(d->last_kernel, s));
+}
+
+// gw_calc_witness_latency for n input sets on `stream` (d_status optional): what the single call does for one set, for
+// every set of the batch.  A Boolean graph runs all n sets bit-sliced, then the sets that broke the bit contract through
+// the latency kernels (a 4-byte readback decides).  Callers hold d->mu; the watchdog is checked by latency_check.
+void Engine::latency_launch(Dev* d, const void* d_inputs, size_t n, void* d_witness, uint32_t* d_status, void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+  if (n == 0) return;
+  if (plan.code.empty()) {            // an empty witness: no kernel, no set flagged
+    if (d_status) CUDA_CHECK(cudaMemsetAsync(d_status, 0, n * 4, s));
+    return;
+  }
+  if (latency_bit(d)) {
+    launch_bit(d, d_inputs, n, d_witness, d_status, s);
+    CUDA_CHECK(cudaEventRecord(d->last_kernel, s));
+    uint32_t n_bad = 0;
+    CUDA_CHECK(cudaMemcpyAsync(&n_bad, d->bit_nbad, 4, cudaMemcpyDeviceToHost, s));
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    if (n_bad != 0) latency_kernels(d, d_inputs, n_bad, d->bit_bad, d_witness, d_status, s);
+    return;
+  }
+  latency_kernels(d, d_inputs, n, nullptr, d_witness, d_status, s);
+}
+
+// clears the watchdog word of d's device before a latency batch call (ordered before its kernels on `s`)
+void Engine::latency_arm(Dev* d, void* stream) {
+  if (!d->lat_aborted) CUDA_CHECK(cudaMalloc(&d->lat_aborted, 4));
+  CUDA_CHECK(cudaMemsetAsync(d->lat_aborted, 0, 4, (cudaStream_t)stream));
+}
+// after the call's work is complete: fails the call when a CTA's watchdog fired
+void Engine::latency_check(Dev* d) {
+  uint32_t aborted = 0;
+  CUDA_CHECK(cudaMemcpy(&aborted, d->lat_aborted, 4, cudaMemcpyDeviceToHost));
+  if (aborted) throw Error(LAT_WATCHDOG_ERROR);
+}
+
+void Engine::run_latency_device(int device, const void* d_inputs, size_t n, void* d_witness, uint32_t* d_status, void* stream) {
+  if (n == 0) return;
+  Dev* d = dev(device);
+  DeviceGuard on(device);
+  std::lock_guard<std::mutex> lk(d->mu);
+  cudaStream_t s = (cudaStream_t)stream;
+  latency_arm(d, s);
+  latency_launch(d, d_inputs, n, d_witness, d_status, s);
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  latency_check(d);
 }
 
 int cuda_device_count() {

@@ -38,8 +38,9 @@ class Engine {
   // .wtns file image once the caller has written the 76-byte headers (the DMA engine does the framing).
   // With `check`, every chunk's rows are also checked against that R1CS on the device (first_failed[r] = lowest violated
   // constraint of set r, or R1CS_OK), and witness may be null: then no witness row is copied to the host.
+  // With `latency`, the chunks run on the latency kernels (run_latency_device) instead of the throughput kernel.
   void run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, int n_gpus, int first_device, size_t out_pitch = 0,
-                R1cs* check = nullptr, uint32_t* first_failed = nullptr);
+                R1cs* check = nullptr, uint32_t* first_failed = nullptr, bool latency = false);
   // Streaming output path: chunks of witness rows are handed to `fn` from a pinned ring as they land (one worker
   // thread per GPU; fn(device, first_set, n_sets, rows, row_bytes, flags) returns nonzero to stop).  The memory
   // is only valid during the call.  chunk_sets = 0 picks the chunk size.
@@ -47,6 +48,9 @@ class Engine {
   void run_stream(const uint8_t* inputs, size_t B, int n_gpus, int first_device, size_t chunk_sets, const ChunkFn& fn);
   // single witness, latency mode (one CTA, intra-level node parallelism); host buffers
   void run_latency(int device, const uint8_t* inputs, uint8_t* witness, uint32_t* status, float* kernel_ms);
+  // run_latency for B input sets resident on `device`, one latency CTA per set (as many at once as the device holds);
+  // ordered on `stream`, returns when the rows are complete
+  void run_latency_device(int device, const void* d_inputs, size_t B, void* d_witness, uint32_t* d_status, void* stream);
   // a plan without LUTs is pure wiring: worth it only when field inputs are taken apart into bits (Num2Bits of a field element)
   bool use_bit_path() const { return bit_plan.eligible && (bit_plan.n_luts > 0 || bit_plan.has_field_inputs); }
   bool bit_path_active() const { return use_bit_path() && !bit_disabled.load(); }
@@ -59,10 +63,17 @@ class Engine {
   Dev* dev(int device);
   void launch(Dev* d, const void* d_inputs, size_t B, void* d_witness, uint32_t* d_status, void* stream);
   void launch_bit(Dev* d, const void* d_inputs, size_t B, void* d_witness, uint32_t* d_status, void* stream);
+  const LatencyPlan& latency_plan(Dev* d);
+  bool latency_bit(Dev* d) const;
+  size_t latency_wave(Dev* d);
+  void latency_kernels(Dev* d, const void* d_inputs, size_t n, const uint32_t* row_map, void* d_witness, uint32_t* d_status, void* stream);
+  void latency_launch(Dev* d, const void* d_inputs, size_t B, void* d_witness, uint32_t* d_status, void* stream);
+  void latency_arm(Dev* d, void* stream);
+  void latency_check(Dev* d);
   void ensure_staging(Dev* d, size_t chunk);
   void stream_on(int device, const uint8_t* inputs, size_t B, size_t first_set, size_t chunk_req, const ChunkFn& fn);
   void run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, size_t out_pitch, R1cs* check,
-                   uint32_t* first_failed);
+                   uint32_t* first_failed, bool latency);
   void init_plan();
   std::map<int, Dev*> devs;
   std::mutex mu;

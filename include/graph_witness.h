@@ -131,6 +131,24 @@ int gw_calc_witness_batch_device(gw_graph_t *graph, int device, const void *d_in
 int gw_calc_witness_latency(gw_graph_t *graph, int device, const uint8_t *inputs, uint8_t *witness, uint32_t *flags,
                             float *kernel_ms, gw_status_t *status);
 
+/* gw_calc_witness_latency for n_sets input sets: one latency-mode CTA per set, as many at once as the device holds.
+ * Row r of witness / flags is byte-identical to gw_calc_witness_latency on input row r.  Host buffers as
+ * gw_calc_witness_batch (inputs n_sets x n_inputs x 32 B, witness n_sets x n_witness x 32 B, flags optional),
+ * sharded over devices first_device .. first_device + n_gpus - 1.
+ * When to use it rather than gw_calc_witness_batch: for batches too small to fill the throughput kernel, where each
+ * of its lanes walks the whole graph alone (a server answering a few to a few hundred concurrent requests).  Every
+ * wave of one set per SM (148 on a B200) takes about one single-witness time.  Measured on a B200 at 1000 W (DESIGN.md
+ * section 5g), device buffers: authV2 17.2 ms for 1 .. 148 sets against 85 ms on gw_calc_witness_batch, faster up to
+ * about 740 sets; authV2_32_32 up to about 590; Poseidon(4) up to about 400.  Above that gw_calc_witness_batch is
+ * faster.  Fails like gw_calc_witness_latency ("latency plan: graph is too wide ...") when the graph does not fit the
+ * latency kernels; there is no fallback. */
+int gw_calc_witness_latency_batch(gw_graph_t *graph, int first_device, int n_gpus, const uint8_t *inputs, size_t n_sets,
+                                  uint8_t *witness, uint32_t *flags, gw_status_t *status);
+/* the same on device buffers on `device`; ordered on cuda_stream (NULL = default stream); returns when the rows are
+ * complete (the Boolean-graph fallback and the watchdog need a readback, as in gw_inputs_parse_batch_device) */
+int gw_calc_witness_latency_batch_device(gw_graph_t *graph, int device, const void *d_inputs, size_t n_sets,
+                                         void *d_witness, uint32_t *d_flags, void *cuda_stream, gw_status_t *status);
+
 /* ---- batch input path (SURVEY 8f-1: replaces deserialize_inputs + populate_inputs, src/lib.rs:154-247, for many
  * input sets).  `text` is JSON Lines (one inputs object per non-empty line) or one top-level JSON array of such
  * objects; it is parsed by n_threads host threads (0 = all) into *inputs = a malloc'ed n_sets x n_inputs x 32 B

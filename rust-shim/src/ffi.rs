@@ -118,4 +118,9 @@ extern "C" {
     pub fn gw_inputs_parse_batch_device(graph: *const gw_graph_t, device: c_int, text: *const c_char, text_len: usize,
                                         d_inputs: *mut c_void, max_sets: usize, n_sets: *mut usize, cuda_stream: *mut c_void,
                                         status: *mut gw_status_t) -> c_int;
+    pub fn gw_calc_witness_latency_batch(graph: *mut gw_graph_t, first_device: c_int, n_gpus: c_int, inputs: *const u8,
+                                         n_sets: usize, witness: *mut u8, flags: *mut u32, status: *mut gw_status_t) -> c_int;
+    pub fn gw_calc_witness_latency_batch_device(graph: *mut gw_graph_t, device: c_int, d_inputs: *const c_void, n_sets: usize,
+                                                d_witness: *mut c_void, d_flags: *mut u32, cuda_stream: *mut c_void,
+                                                status: *mut gw_status_t) -> c_int;
 }
