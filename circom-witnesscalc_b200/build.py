@@ -26,7 +26,7 @@ BIN_WTNS_CHECK = os.path.join(HERE, "bin", "wtns-check")
 EXAMPLE_SRC = os.path.join(HERE, "..", "examples", "calc_witness.c")
 BIN_EXAMPLE = os.path.join(HERE, "bin", "example-calc-witness")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-SOURCES = ["engine.cu", "r1cs.cu", "ntt.cu", "inputs.cu", "graph.cpp", "plan.cpp", "bitplan.cpp", "inputs.cpp", "wtns.cpp", "r1cs.cpp", "capi.cpp"]
+SOURCES = ["engine.cu", "r1cs.cu", "ntt.cu", "inputs.cu", "cuda_util.cpp", "graph.cpp", "plan.cpp", "bitplan.cpp", "inputs.cpp", "wtns.cpp", "r1cs.cpp", "capi.cpp"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 # the optimisation flags of every device build (the test-only device harness of tests/csrc is built with them too)
 OPT = ["-std=c++17", "-O3", "-lineinfo"]

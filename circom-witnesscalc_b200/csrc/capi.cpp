@@ -10,6 +10,7 @@
 #include <memory>
 #include <mutex>
 
+#include "cuda_util.hpp"
 #include "engine.hpp"
 #include "inputs.hpp"
 #include "ntt.hpp"
@@ -45,6 +46,19 @@ template <typename F> static int guarded(const gw_status_t* status, F&& f) {
   try { f(); set_status(status, OK, nullptr); return 0; }
   catch (const std::exception& e) { set_status(status, ERROR, e.what()); return 1; }
   catch (...) { set_status(status, ERROR, "unknown error"); return 1; }
+}
+
+static const char* const RANGE_ERROR = "device range exceeds the visible CUDA devices";   // host entry points with a first_device
+static const char* const N_GPUS_ERROR = "n_gpus exceeds the number of visible CUDA devices";   // host entry points that start at device 0
+
+// The devices [first_device, first_device + n_gpus) of a host entry point (n_gpus < 1: one device); range_error is the
+// message of the entry point's family.  Returns n_gpus.
+static int check_devices(int first_device, int n_gpus, const char* range_error) {
+  const int ndev = cuda_device_count();
+  if (ndev == 0) throw Error(NO_DEVICE_ERROR);
+  if (n_gpus < 1) n_gpus = 1;
+  if (first_device < 0 || first_device + n_gpus > ndev) throw Error(range_error);
+  return n_gpus;
 }
 
 static int single_device();
@@ -175,17 +189,14 @@ int gw_calc_witness_batch_on(gw_graph_t* graph, int first_device, const uint8_t*
                              uint32_t* flags, int n_gpus, gw_status_t* status) {
   if (!graph || (n_sets && (!inputs || !witness))) { set_status(status, ERROR, "null argument"); return 1; }
   return guarded(status, [&]() {
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (first_device < 0 || first_device + n_gpus > ndev) throw Error("device range exceeds the visible CUDA devices");
+    n_gpus = check_devices(first_device, n_gpus, RANGE_ERROR);
     graph->engine->run_host(inputs, n_sets, witness, flags, n_gpus, first_device);
   });
 }
 
 int gw_calc_witness_batch(gw_graph_t* graph, const uint8_t* inputs, size_t n_sets, uint8_t* witness, uint32_t* flags,
                           int n_gpus, gw_status_t* status) {
-  if (graph && n_gpus > cuda_device_count() && cuda_device_count() > 0) { set_status(status, ERROR, "n_gpus exceeds the number of visible CUDA devices"); return 1; }
+  if (graph && n_gpus > cuda_device_count() && cuda_device_count() > 0) { set_status(status, ERROR, N_GPUS_ERROR); return 1; }
   return gw_calc_witness_batch_on(graph, 0, inputs, n_sets, witness, flags, n_gpus, status);
 }
 
@@ -206,10 +217,7 @@ int gw_calc_witness_latency_batch(gw_graph_t* graph, int first_device, int n_gpu
   if (!graph || (n_sets && (!inputs || !witness))) { set_status(status, ERROR, "null argument"); return 1; }
   return guarded(status, [&]() {
     if (!n_sets) return;
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (first_device < 0 || first_device + n_gpus > ndev) throw Error("device range exceeds the visible CUDA devices");
+    n_gpus = check_devices(first_device, n_gpus, RANGE_ERROR);
     graph->engine->run_host(inputs, n_sets, witness, flags, n_gpus, first_device, 0, nullptr, nullptr, true);
   });
 }
@@ -235,7 +243,6 @@ int gw_inputs_parse_batch_device(const gw_graph_t* graph, int device, const char
   if (!graph || !n_sets || (text_len && !text) || (max_sets && !d_inputs)) { set_status(status, ERROR, "null argument"); return 1; }
   *n_sets = 0;
   return guarded(status, [&]() {
-    if (cuda_device_count() == 0) throw Error("no CUDA device available: this library has no CPU fallback");
     DeviceInputs* p;
     {
       std::lock_guard<std::mutex> lk(graph->dev_inputs_mu);
@@ -254,10 +261,7 @@ int gw_calc_witness_batch_wtns(gw_graph_t* graph, const uint8_t* inputs, size_t 
   return guarded(status, [&]() {
     const uint32_t W = graph->engine->plan.n_witness;
     if (file_pitch < wtns_size(W)) throw Error("file_pitch is smaller than a .wtns file of this graph");
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (n_gpus > ndev) throw Error("n_gpus exceeds the number of visible CUDA devices");
+    n_gpus = check_devices(0, n_gpus, N_GPUS_ERROR);
     for (size_t i = 0; i < n_sets; i++) wtns_write_header(files + i * file_pitch, W);
     graph->engine->run_host(inputs, n_sets, files + WTNS_HEADER_BYTES, flags, n_gpus, 0, file_pitch);
   });
@@ -285,10 +289,7 @@ int gw_calc_witness_batch_stream(gw_graph_t* graph, int first_device, int n_gpus
                                  size_t chunk_sets, gw_witness_chunk_fn fn, void* user, gw_status_t* status) {
   if (!graph || !fn || (n_sets && !inputs)) { set_status(status, ERROR, "null argument"); return 1; }
   return guarded(status, [&]() {
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (first_device < 0 || first_device + n_gpus > ndev) throw Error("device range exceeds the visible CUDA devices");
+    n_gpus = check_devices(first_device, n_gpus, RANGE_ERROR);
     graph->engine->run_stream(inputs, n_sets, n_gpus, first_device, chunk_sets,
                               [&](int device, size_t first, size_t n, const uint8_t* rows, size_t row_bytes, const uint32_t* flags) {
                                 return fn(user, device, first, n, rows, row_bytes, flags);
@@ -321,10 +322,7 @@ int gw_r1cs_check_batch(gw_r1cs_t* r1cs, const uint8_t* witness, size_t n_sets, 
                         int n_gpus, gw_status_t* status) {
   if (!r1cs || (n_sets && (!witness || !first_failed))) { set_status(status, ERROR, "null argument"); return 1; }
   return guarded(status, [&]() {
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (n_gpus > ndev) throw Error("n_gpus exceeds the number of visible CUDA devices");
+    n_gpus = check_devices(0, n_gpus, N_GPUS_ERROR);
     r1cs->r1cs->check_host(witness, n_sets, row_pitch ? row_pitch : (size_t)r1cs->r1cs->hdr.n_wires * 32, first_failed, n_gpus, 0);
   });
 }
@@ -352,10 +350,7 @@ int gw_r1cs_abc_batch(gw_r1cs_t* r1cs, const uint8_t* witness, size_t n_sets, si
     if (!abc_pitch) abc_pitch = 3 * 32 * (size_t)r.abc_len(options);
     r.abc_row_bytes(row_pitch, abc_pitch, options, false);          // the arguments first: no device is touched
     if (!n_sets) return;
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (n_gpus > ndev) throw Error("n_gpus exceeds the number of visible CUDA devices");
+    n_gpus = check_devices(0, n_gpus, N_GPUS_ERROR);
     r.abc_host(witness, n_sets, row_pitch, abc, abc_pitch, options, first_failed, n_gpus, 0);
   });
 }
@@ -386,10 +381,7 @@ int gw_r1cs_quotient_batch(gw_r1cs_t* r1cs, const uint8_t* witness, size_t n_set
     if (!h_pitch) h_pitch = 32 * (size_t)r.abc_len(GW_R1CS_ABC_GROTH16);
     r.quotient_log_n(row_pitch, h_pitch, false);                    // the arguments first: no device is touched
     if (!n_sets) return;
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (n_gpus > ndev) throw Error("n_gpus exceeds the number of visible CUDA devices");
+    n_gpus = check_devices(0, n_gpus, N_GPUS_ERROR);
     r.quotient_host(witness, n_sets, row_pitch, h, h_pitch, first_failed, n_gpus, 0);
   });
 }
@@ -412,10 +404,7 @@ int gw_calc_witness_batch_check(gw_graph_t* graph, gw_r1cs_t* r1cs, int first_de
     const uint32_t W = graph->engine->plan.n_witness, n_wires = r1cs->r1cs->hdr.n_wires;
     if (W != n_wires)
       throw Error("the graph's witness has " + std::to_string(W) + " values but the R1CS has " + std::to_string(n_wires) + " wires");
-    int ndev = cuda_device_count();
-    if (ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-    if (n_gpus < 1) n_gpus = 1;
-    if (first_device < 0 || first_device + n_gpus > ndev) throw Error("device range exceeds the visible CUDA devices");
+    n_gpus = check_devices(first_device, n_gpus, RANGE_ERROR);
     graph->engine->run_host(inputs, n_sets, witness, flags, n_gpus, first_device, 0, r1cs->r1cs.get(), first_failed);
   });
 }

@@ -14,12 +14,9 @@
 #include <stdio.h>
 #include <string.h>
 
-#include <sched.h>
-
 #include <algorithm>
 #include <memory>
 #include <mutex>
-#include <thread>
 #include <vector>
 
 #include "engine.hpp"
@@ -1024,47 +1021,25 @@ struct Engine::Dev {
   uint4* lat_in = nullptr; uint4* lat_out = nullptr; uint32_t* lat_status = nullptr;
   uint32_t* lat_aborted = nullptr;       // latency batch calls: set by a CTA whose watchdog fired (DParams::aborted)
   std::mutex mu;
+  ~Dev() {
+    int prev = -1;
+    cudaGetDevice(&prev);
+    cudaSetDevice(device);
+    cudaFree(code); cudaFree(consts); cudaFree(spill);
+    cudaFree(bit_code); cudaFree(bit_inputs); cudaFree(bit_constpos); cudaFree(bit_consts); cudaFree(bit_wide); cudaFree(bit_field_inputs); cudaFree(bit_field_slots);
+    cudaFree(bit_planes); cudaFree(bit_ok); cudaFree(bit_bad); cudaFree(bit_nbad);
+    cudaFreeHost(bit_nbad_host); if (bit_nbad_ev) cudaEventDestroy(bit_nbad_ev);
+    cudaFree(lat_soff); cudaFree(lat_schunks);
+    cudaFree(lat_code); cudaFree(lat_first); cudaFree(lat_jobs); cudaFree(lat_njobs); cudaFree(lat_waits); cudaFree(lat_clock); cudaFree(lat_in); cudaFree(lat_out); cudaFree(lat_status); cudaFree(lat_aborted);
+    for (int i = 0; i < 2; i++) { cudaFree(d_in[i]); cudaFree(d_out[i]); cudaFree(d_status[i]); cudaFree(d_ff[i]); if (stream[i]) cudaStreamDestroy(stream[i]); }
+    for (int i = 0; i < 3; i++) { cudaFreeHost(h_ring[i]); cudaFreeHost(h_flags[i]); }
+    if (last_kernel) cudaEventDestroy(last_kernel);
+    if (prev >= 0) cudaSetDevice(prev);
+  }
 };
 
 static int env_int(const char* name, int dflt) { const char* s = getenv(name); return (s && *s) ? atoi(s) : dflt; }
 
-
-// Pins the CALLING thread to the CPUs of the NUMA node the GPU hangs off (sysfs: numa_node of its PCI function,
-// cpulist of that node), so that the thread's pinned allocations are node-local and its copies do not cross the
-// socket interconnect.  Only ever called on threads this library created.  GW_NUMA=0 turns it off.
-void bind_thread_near_device(int device) {
-  if (env_int("GW_NUMA", 1) == 0) return;
-  char bus[32] = {0};
-  if (cudaDeviceGetPCIBusId(bus, (int)sizeof bus, device) != cudaSuccess) return;
-  for (char* c = bus; *c; c++) if (*c >= 'A' && *c <= 'Z') *c = (char)(*c - 'A' + 'a');
-  char path[160];
-  snprintf(path, sizeof path, "/sys/bus/pci/devices/%s/numa_node", bus);
-  FILE* f = fopen(path, "r");
-  if (!f) return;
-  int node = -1;
-  if (fscanf(f, "%d", &node) != 1) node = -1;
-  fclose(f);
-  if (node < 0) return;
-  snprintf(path, sizeof path, "/sys/devices/system/node/node%d/cpulist", node);
-  f = fopen(path, "r");
-  if (!f) return;
-  char list[4096] = {0};
-  const bool got = fgets(list, (int)sizeof list, f) != nullptr;
-  fclose(f);
-  if (!got) return;
-  cpu_set_t allowed, want;
-  CPU_ZERO(&allowed); CPU_ZERO(&want);
-  if (sched_getaffinity(0, sizeof allowed, &allowed) != 0) return;
-  int n_want = 0;
-  for (const char* c = list; *c;) {
-    while (*c == ',' || *c == ' ' || *c == '\n') c++;
-    if (*c < '0' || *c > '9') break;
-    long lo = strtol(c, const_cast<char**>(&c), 10), hi = lo;
-    if (*c == '-') hi = strtol(c + 1, const_cast<char**>(&c), 10);
-    for (long k = lo; k <= hi && k < CPU_SETSIZE; k++) if (CPU_ISSET((int)k, &allowed)) { CPU_SET((int)k, &want); n_want++; }
-  }
-  if (n_want > 0) sched_setaffinity(0, sizeof want, &want);
-}
 
 Engine::Engine(const uint8_t* graph_data, size_t len) {
   graph = deserialize_witnesscalc_graph(graph_data, len);
@@ -1106,34 +1081,13 @@ int Engine::threads_for(size_t B, int sms, int t_max) const {
   return (int)std::min<size_t>(std::max<size_t>(t, 32), (size_t)t_max);
 }
 
-Engine::~Engine() {
-  for (auto& kv : devs) {
-    Dev* d = kv.second;
-    int prev = -1;
-    cudaGetDevice(&prev);
-    cudaSetDevice(d->device);
-    cudaFree(d->code); cudaFree(d->consts); cudaFree(d->spill);
-    cudaFree(d->bit_code); cudaFree(d->bit_inputs); cudaFree(d->bit_constpos); cudaFree(d->bit_consts); cudaFree(d->bit_wide); cudaFree(d->bit_field_inputs); cudaFree(d->bit_field_slots);
-    cudaFree(d->bit_planes); cudaFree(d->bit_ok); cudaFree(d->bit_bad); cudaFree(d->bit_nbad);
-    cudaFreeHost(d->bit_nbad_host); if (d->bit_nbad_ev) cudaEventDestroy(d->bit_nbad_ev);
-    cudaFree(d->lat_soff); cudaFree(d->lat_schunks);
-    cudaFree(d->lat_code); cudaFree(d->lat_first); cudaFree(d->lat_jobs); cudaFree(d->lat_njobs); cudaFree(d->lat_waits); cudaFree(d->lat_clock); cudaFree(d->lat_in); cudaFree(d->lat_out); cudaFree(d->lat_status); cudaFree(d->lat_aborted);
-    for (int i = 0; i < 2; i++) { cudaFree(d->d_in[i]); cudaFree(d->d_out[i]); cudaFree(d->d_status[i]); cudaFree(d->d_ff[i]); if (d->stream[i]) cudaStreamDestroy(d->stream[i]); }
-    for (int i = 0; i < 3; i++) { cudaFreeHost(d->h_ring[i]); cudaFreeHost(d->h_flags[i]); }
-    if (d->last_kernel) cudaEventDestroy(d->last_kernel);
-    delete d;
-    if (prev >= 0) cudaSetDevice(prev);
-  }
-}
+Engine::~Engine() = default;
 
 Engine::Dev* Engine::dev(int device) {
   std::lock_guard<std::mutex> lk(mu);
   auto it = devs.find(device);
-  if (it != devs.end()) return it->second;
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-  if (device < 0 || device >= ndev) throw Error("CUDA device index out of range");
+  if (it != devs.end()) return it->second.get();
+  check_device(device);
   DeviceGuard on(device);
   std::unique_ptr<Dev> d(new Dev());
   d->device = device;
@@ -1199,8 +1153,7 @@ Engine::Dev* Engine::dev(int device) {
     CUDA_CHECK(cudaHostAlloc(&d->bit_nbad_host, 4, cudaHostAllocDefault));
     CUDA_CHECK(cudaEventCreateWithFlags(&d->bit_nbad_ev, cudaEventDisableTiming));
   }
-  devs[device] = d.get();
-  return d.release();
+  return (devs[device] = std::move(d)).get();
 }
 
 // Enqueues one eval_batch_kernel on `stream`, behind every earlier launch of this engine on the device (the spill
@@ -1368,11 +1321,6 @@ struct HostTrace {
   }
   ~HostTrace() { for (cudaEvent_t e : ev) cudaEventDestroy(e); }
 };
-// no copy may still target the caller's (or the ring's) memory when a host-buffer call returns, also on errors
-struct StreamDrain {
-  cudaStream_t a, b;
-  ~StreamDrain() { cudaStreamSynchronize(a); cudaStreamSynchronize(b); }
-};
 }  // namespace
 
 // host buffers: chunked, double-buffered H2D -> kernel -> D2H on two streams (latency: the latency kernels, one CTA per set)
@@ -1442,23 +1390,11 @@ void Engine::run_host(const uint8_t* inputs, size_t B, uint8_t* witness, uint32_
   if (B == 0) return;
   if (out_pitch == 0) out_pitch = (size_t)plan.n_witness * 32;
   if (n_gpus <= 1) { run_host_on(first_device, inputs, B, witness, status, out_pitch, check, first_failed, latency); return; }
-  // independent input sets: contiguous shards, one host thread per GPU (pinned to the GPU's NUMA node), no collective
   const size_t in_b = (size_t)plan.n_inputs * 32;
-  std::vector<std::thread> th;
-  std::vector<std::string> errs(n_gpus);
-  for (int g = 0; g < n_gpus; g++) {
-    size_t lo = B * g / n_gpus, hi = B * (g + 1) / n_gpus;
-    if (hi == lo) continue;
-    th.emplace_back([=, &errs]() {
-      try {
-        bind_thread_near_device(first_device + g);
-        run_host_on(first_device + g, inputs + lo * in_b, hi - lo, witness ? witness + lo * out_pitch : nullptr, status ? status + lo : nullptr,
-                    out_pitch, check, check ? first_failed + lo : nullptr, latency);
-      } catch (const std::exception& e) { errs[g] = e.what(); }
-    });
-  }
-  for (auto& t : th) t.join();
-  for (auto& e : errs) if (!e.empty()) throw Error(e);
+  run_shards(B, n_gpus, first_device, [&](int device, size_t lo, size_t hi) {
+    run_host_on(device, inputs + lo * in_b, hi - lo, witness ? witness + lo * out_pitch : nullptr, status ? status + lo : nullptr,
+                out_pitch, check, check ? first_failed + lo : nullptr, latency);
+  });
 }
 
 // Streaming output path: the witnesses of the batch never exist in host memory all at once.  Per GPU, chunk k's rows
@@ -1528,20 +1464,7 @@ void Engine::run_stream(const uint8_t* inputs, size_t B, int n_gpus, int first_d
   if (n_gpus < 1) n_gpus = 1;
   // always on worker threads: they are pinned near their GPU before the ring is allocated, the caller's affinity is left alone
   const size_t in_b = (size_t)plan.n_inputs * 32;
-  std::vector<std::thread> th;
-  std::vector<std::string> errs(n_gpus);
-  for (int g = 0; g < n_gpus; g++) {
-    size_t lo = B * g / n_gpus, hi = B * (g + 1) / n_gpus;
-    if (hi == lo) continue;
-    th.emplace_back([=, &errs, &fn]() {
-      try {
-        bind_thread_near_device(first_device + g);
-        stream_on(first_device + g, inputs + lo * in_b, hi - lo, lo, chunk_sets, fn);
-      } catch (const std::exception& e) { errs[g] = e.what(); }
-    });
-  }
-  for (auto& t : th) t.join();
-  for (auto& e : errs) if (!e.empty()) throw Error(e);
+  run_shards(B, n_gpus, first_device, [&](int device, size_t lo, size_t hi) { stream_on(device, inputs + lo * in_b, hi - lo, lo, chunk_sets, fn); });
 }
 
 // shared memory of one latency CTA of plan lp (engine.cu: eval_dataflow_kernel, eval_latency_kernel)
@@ -1839,12 +1762,6 @@ void Engine::run_latency_device(int device, const void* d_inputs, size_t n, void
   latency_launch(d, d_inputs, n, d_witness, d_status, s);
   CUDA_CHECK(cudaStreamSynchronize(s));
   latency_check(d);
-}
-
-int cuda_device_count() {
-  int n = 0;
-  if (cudaGetDeviceCount(&n) != cudaSuccess) return 0;
-  return n;
 }
 
 }  // namespace gw

@@ -5,6 +5,7 @@
 #include <atomic>
 #include <functional>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 
@@ -75,11 +76,10 @@ class Engine {
   void run_host_on(int device, const uint8_t* inputs, size_t B, uint8_t* witness, uint32_t* status, size_t out_pitch, R1cs* check,
                    uint32_t* first_failed, bool latency);
   void init_plan();
-  std::map<int, Dev*> devs;
+  std::map<int, std::unique_ptr<Dev>> devs;
   std::mutex mu;
 };
 
-int cuda_device_count();
 double imad_microbench(int device, int which);
 
 }  // namespace gw

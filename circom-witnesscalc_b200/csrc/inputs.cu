@@ -421,30 +421,26 @@ struct DeviceInputs::Dev {
   unsigned long long* marks = nullptr; size_t marks_cap = 0;
   unsigned long long* sum = nullptr;
   unsigned long long* h_sum = nullptr;         // pinned
-};
-
-DeviceInputs::~DeviceInputs() {
-  for (auto& kv : devs) {
-    Dev* d = kv.second;
+  ~Dev() {
     int prev = -1;
     cudaGetDevice(&prev);
-    cudaSetDevice(d->device);
-    cudaFree(d->slots); cudaFree(d->keys); cudaFree(d->names); cudaFree(d->text);
-    cudaFree(d->tile_fn); cudaFree(d->tile_state); cudaFree(d->tile_dd); cudaFree(d->tile_depth); cudaFree(d->tile_cnt); cudaFree(d->tile_off);
-    cudaFree(d->starts); cudaFree(d->ends); cudaFree(d->seen); cudaFree(d->marks); cudaFree(d->sum);
-    cudaFreeHost(d->h_sum);
-    delete d;
+    cudaSetDevice(device);
+    cudaFree(slots); cudaFree(keys); cudaFree(names); cudaFree(text);
+    cudaFree(tile_fn); cudaFree(tile_state); cudaFree(tile_dd); cudaFree(tile_depth); cudaFree(tile_cnt); cudaFree(tile_off);
+    cudaFree(starts); cudaFree(ends); cudaFree(seen); cudaFree(marks); cudaFree(sum);
+    cudaFreeHost(h_sum);
     if (prev >= 0) cudaSetDevice(prev);
   }
-}
+};
+
+DeviceInputs::DeviceInputs(const Graph& g) : g(g) {}
+DeviceInputs::~DeviceInputs() = default;
 
 DeviceInputs::Dev* DeviceInputs::dev(int device) {
   std::lock_guard<std::mutex> lk(mu);
   auto it = devs.find(device);
-  if (it != devs.end()) return it->second;
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-  if (device < 0 || device >= ndev) throw Error("CUDA device index out of range");
+  if (it != devs.end()) return it->second.get();
+  check_device(device);
   DeviceGuard on(device);
   std::unique_ptr<Dev> d(new Dev());
   d->device = device;
@@ -480,8 +476,7 @@ DeviceInputs::Dev* DeviceInputs::dev(int device) {
   CUDA_CHECK(cudaMemcpy(d->names, names.data(), names.size(), cudaMemcpyHostToDevice));
   CUDA_CHECK(cudaMalloc(&d->sum, SUM_WORDS * 8));
   CUDA_CHECK(cudaHostAlloc(&d->h_sum, SUM_WORDS * 8, cudaHostAllocDefault));
-  devs[device] = d.get();
-  return d.release();
+  return (devs[device] = std::move(d)).get();
 }
 
 void DeviceInputs::parse(int device, const char* text, size_t len, void* d_rows, size_t max_sets, void* stream, size_t* n_sets) {

@@ -4,6 +4,7 @@
 // InputFieldNumberParseError keep their wording; cases where the reference panics (invalid JSON,
 // unknown key, wrong length) are reported as gw::Error instead.
 #pragma once
+#include <memory>
 #include <mutex>
 
 #include "graph.hpp"
@@ -34,7 +35,7 @@ void split_records(const char* text, size_t len, std::vector<std::pair<size_t, s
 // the record count, also when there are more than max_sets records (an error: nothing is written then).
 class DeviceInputs {
  public:
-  explicit DeviceInputs(const Graph& g) : g(g) {}
+  explicit DeviceInputs(const Graph& g);
   ~DeviceInputs();
   DeviceInputs(const DeviceInputs&) = delete;
   void parse(int device, const char* text, size_t len, void* d_rows, size_t max_sets, void* stream, size_t* n_sets);
@@ -43,7 +44,7 @@ class DeviceInputs {
  private:
   Dev* dev(int device);
   const Graph& g;
-  std::map<int, Dev*> devs;
+  std::map<int, std::unique_ptr<Dev>> devs;
   std::mutex mu;
 };
 

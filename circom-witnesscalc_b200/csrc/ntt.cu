@@ -262,10 +262,7 @@ const uint4* ntt_tables(int device, uint32_t lg) {
   std::lock_guard<std::mutex> lk(g_mu);
   auto it = g_tabs.find({device, lg});
   if (it != g_tabs.end()) return it->second;
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-  if (device < 0 || device >= ndev) throw Error("CUDA device index out of range");
+  check_device(device);
   DeviceGuard on(device);
   if (!g_ready[device]) {
     cudaDeviceProp prop; CUDA_CHECK(cudaGetDeviceProperties(&prop, device));
@@ -281,7 +278,7 @@ const uint4* ntt_tables(int device, uint32_t lg) {
   const std::vector<fe> tab = ntt_build_tables(lg);
   uint4* d = nullptr;
   CUDA_CHECK(cudaMalloc(&d, tab.size() * 32));
-  e = cudaMemcpy(d, tab.data(), tab.size() * 32, cudaMemcpyHostToDevice);
+  const cudaError_t e = cudaMemcpy(d, tab.data(), tab.size() * 32, cudaMemcpyHostToDevice);
   if (e != cudaSuccess) { cudaFree(d); CUDA_CHECK(e); }
   g_tabs[{device, lg}] = d;
   return d;

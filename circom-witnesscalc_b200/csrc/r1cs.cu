@@ -13,7 +13,6 @@
 #include <algorithm>
 #include <memory>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "cuda_util.hpp"
@@ -203,33 +202,28 @@ struct R1cs::Dev {
   uint8_t* d_rows[2] = {nullptr, nullptr}; uint32_t* d_ff[2] = {nullptr, nullptr}; uint8_t* d_out[2] = {nullptr, nullptr};
   size_t chunk = 0, out_b = 0;             // rows per chunk; bytes of each d_out
   std::mutex mu;
-};
-
-R1cs::~R1cs() {
-  for (auto& kv : devs) {
-    Dev* d = kv.second;
+  ~Dev() {
     int prev = -1;
     cudaGetDevice(&prev);
-    cudaSetDevice(d->device);
-    cudaFree(d->code); cudaFree(d->consts);
+    cudaSetDevice(device);
+    cudaFree(code); cudaFree(consts);
     for (int i = 0; i < 2; i++) {
-      cudaFree(d->d_rows[i]); cudaFree(d->d_ff[i]); cudaFree(d->d_out[i]);
-      if (d->stream[i]) cudaStreamDestroy(d->stream[i]);
+      cudaFree(d_rows[i]); cudaFree(d_ff[i]); cudaFree(d_out[i]);
+      if (stream[i]) cudaStreamDestroy(stream[i]);
     }
-    delete d;
     if (prev >= 0) cudaSetDevice(prev);
   }
-}
+};
+
+R1cs::R1cs(const uint8_t* data, size_t len) { parse_r1cs(data, len, hdr, prog); }
+R1cs::~R1cs() = default;
 
 // program and constant table, uploaded on first use of a device
 R1cs::Dev* R1cs::dev(int device) {
   std::lock_guard<std::mutex> lk(mu);
   auto it = devs.find(device);
-  if (it != devs.end()) return it->second;
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess || ndev == 0) throw Error("no CUDA device available: this library has no CPU fallback");
-  if (device < 0 || device >= ndev) throw Error("CUDA device index out of range");
+  if (it != devs.end()) return it->second.get();
+  gw::check_device(device);   // the free function, not R1cs::check_device
   if (prog.code.size() / 2 > 0xFFFFFFFFull) throw Error("r1cs: program too large (more than 2^32 items)");
   DeviceGuard on(device);
   std::unique_ptr<Dev> d(new Dev());
@@ -244,8 +238,7 @@ R1cs::Dev* R1cs::dev(int device) {
   CUDA_CHECK(cudaMemcpy(d->code, prog.code.data(), prog.code.size() * 4, cudaMemcpyHostToDevice));
   CUDA_CHECK(cudaMalloc(&d->consts, std::max<size_t>(prog.consts.size(), 1) * 32));
   CUDA_CHECK(cudaMemcpy(d->consts, prog.consts.data(), prog.consts.size() * 32, cudaMemcpyHostToDevice));
-  devs[device] = d.get();
-  return d.release();
+  return (devs[device] = std::move(d)).get();
 }
 
 struct R1cs::Launch {
@@ -331,14 +324,6 @@ void R1cs::abc_device(int device, const void* d_witness, size_t B, size_t row_pi
   CUDA_CHECK(cudaGetLastError());
 }
 
-namespace {
-// no copy may still target the caller's memory when a host-buffer call returns, also on errors
-struct Drain {
-  cudaStream_t a, b;
-  ~Drain() { if (a) cudaStreamSynchronize(a); if (b) cudaStreamSynchronize(b); }
-};
-}  // namespace
-
 // host rows: chunked, double-buffered H2D (pitched) -> check, ABC or quotient -> D2H of the results on two streams.
 // out == NULL: the check; else the ABC vectors or h (and the verdicts when first_failed is not NULL).  The chunk size
 // counts the 3 x n x 32 device bytes of a row in both output modes; only h (n x 32 bytes) of a quotient row is copied.
@@ -370,7 +355,7 @@ void R1cs::host_rows_on(int device, const uint8_t* witness, size_t B, size_t row
     }
     d->chunk = chunk; d->out_b = chunk * out_row;
   }
-  Drain drain{d->stream[0], d->stream[1]};
+  StreamDrain drain{d->stream[0], d->stream[1]};
   int k = 0;
   for (size_t off = 0; off < B; off += chunk, k ^= 1) {
     const size_t nb = std::min(chunk, B - off);
@@ -396,24 +381,11 @@ void R1cs::host_rows(const uint8_t* witness, size_t B, size_t row_pitch, uint32_
                      int first_device) {
   if (B == 0) return;
   if (n_gpus <= 1) { host_rows_on(first_device, witness, B, row_pitch, first_failed, out); return; }
-  // independent rows: contiguous shards, one host thread per GPU, no collective
-  std::vector<std::thread> th;
-  std::vector<std::string> errs(n_gpus);
-  for (int g = 0; g < n_gpus; g++) {
-    const size_t lo = B * g / n_gpus, hi = B * (g + 1) / n_gpus;
-    if (hi == lo) continue;
-    th.emplace_back([=, &errs]() {
-      try {
-        bind_thread_near_device(first_device + g);
-        AbcOut shard;
-        if (out) shard = AbcOut{out->abc + lo * out->pitch, out->pitch, out->options, out->quotient};
-        host_rows_on(first_device + g, witness + lo * row_pitch, hi - lo, row_pitch, first_failed ? first_failed + lo : nullptr,
-                     out ? &shard : nullptr);
-      } catch (const std::exception& e) { errs[g] = e.what(); }
-    });
-  }
-  for (auto& t : th) t.join();
-  for (auto& e : errs) if (!e.empty()) throw Error(e);
+  run_shards(B, n_gpus, first_device, [&](int device, size_t lo, size_t hi) {
+    AbcOut shard;
+    if (out) shard = AbcOut{out->abc + lo * out->pitch, out->pitch, out->options, out->quotient};
+    host_rows_on(device, witness + lo * row_pitch, hi - lo, row_pitch, first_failed ? first_failed + lo : nullptr, out ? &shard : nullptr);
+  });
 }
 
 void R1cs::check_host(const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, int n_gpus, int first_device) {

@@ -44,7 +44,7 @@ void parse_r1cs(const uint8_t* data, size_t len, R1csHeader& hdr, R1csProgram& p
 
 class R1cs {
  public:
-  R1cs(const uint8_t* data, size_t len) { parse_r1cs(data, len, hdr, prog); }
+  R1cs(const uint8_t* data, size_t len);
   ~R1cs();
   R1cs(const R1cs&) = delete;
 
@@ -88,7 +88,7 @@ class R1cs {
   void host_rows_on(int device, const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, const AbcOut* out);
   void host_rows(const uint8_t* witness, size_t B, size_t row_pitch, uint32_t* first_failed, const AbcOut* out, int n_gpus,
                  int first_device);
-  std::map<int, Dev*> devs;
+  std::map<int, std::unique_ptr<Dev>> devs;
   std::mutex mu;
 };
 
